@@ -1,8 +1,11 @@
 #!/usr/bin/env python
 """bench.py -- throughput of the render() hot path on N B200s (one process per GPU).
 
-    python bench.py --gpus N --steps K --warmup W [--workload c1|c2|c3|c4|c5] [--scale F]
+    python bench.py --gpus N --steps K --warmup W [--workload c1|c2|c3|c4|c5] [--scale F] [--dump-outputs DIR]
     python bench.py --impl reference ...        # the reference's CPU algorithm on host cores
+
+--dump-outputs DIR writes what the last timed step computed (see dump_outputs) so that two builds can be
+compared output for output: the inputs are seeded, identical from run to run for the same arguments.
 
 A "step" is one pass of the hot path over one frame of synthetic input: the workload's frame at its
 named samples per pixel.  With N GPUs the job is FIXED (--scaling strong, the default: C3 is "1080p,
@@ -93,6 +96,27 @@ def algorithmic_cost(name, n_prims, S, P):
         return 38 * 20 + 60, 38 * 16
     L = max(1, math.ceil(math.log2(max(n_prims, 8) / 4.0)))
     return 2 * L * 22 + 4 * P + 60, L * 64 + 4 * S
+
+
+DUMP_LIMIT_BYTES = 60 * 10 ** 6  # under 64 MB in all, .npy headers included
+
+
+def dump_outputs(out_dir, frames):
+    """frames: {name: (H, W, 3) host array}, written as out_dir/<name>.npy in float32.  When the whole frames
+    would exceed DUMP_LIMIT_BYTES, every frame is cut to the same fixed, seeded sample of pixels (rows of
+    (n, 3)), and pixel_index.npy (float64) holds their flat indices y * W + x."""
+    os.makedirs(out_dir, exist_ok=True)
+    frames = {k: np.ascontiguousarray(v, dtype=np.float32) for k, v in frames.items()}
+    h, w, c = next(iter(frames.values())).shape
+    n_pix = h * w
+    per_pixel = len(frames) * c * 4
+    if n_pix * per_pixel > DUMP_LIMIT_BYTES:
+        keep = DUMP_LIMIT_BYTES // (per_pixel + 8)
+        idx = np.sort(np.random.default_rng(SEED).choice(n_pix, keep, replace=False))
+        frames = {k: v.reshape(n_pix, c)[idx] for k, v in frames.items()}
+        frames["pixel_index"] = idx.astype(np.float64)
+    for k, v in frames.items():
+        np.save(os.path.join(out_dir, k + ".npy"), v)
 
 
 class ClockSampler:
@@ -377,6 +401,13 @@ def main_gpu(args):
         ev[i][1].record(stream)
     sync_all()
     clocks = sampler.stop() if sampler else None
+    if args.dump_outputs and rank == 0:
+        # the last timed step's results, before the e2e and kernel-timing passes below reuse the buffers;
+        # a group keeps the per-rank sums inside the library and hands rank 0 the framebuffer only
+        frames = {"framebuffer": fb.cpu().numpy()}
+        if comm is None:
+            frames["accum"] = accum.cpu().numpy()
+        dump_outputs(args.dump_outputs, frames)
     ms_local = sum(a.elapsed_time(b) for a, b in ev)
     t = torch.tensor([ms_local], dtype=torch.float64, device=dev)
     if world > 1:
@@ -555,8 +586,14 @@ def main():
                     help="strong (default): the named job, samples split over the GPUs; weak: the named spp per GPU")
     ap.add_argument("--integrator", default="path", choices=["path", "whitted"],
                     help="path = trace_path (raytracer.c:482-554, the upstream default); whitted = cast_ray (raytracer.c:556-641)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the last timed step's framebuffer and per-pixel sums as DIR/<name>.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
+        if args.dump_outputs:
+            ap.error("--dump-outputs applies to the GPU arm (--impl b200)")
         return main_reference(args)
     return main_gpu(args)
 

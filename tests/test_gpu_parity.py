@@ -8,12 +8,15 @@ The three-way check BASELINE.json asks for:
   3. converged image PSNR against the reference's own high-spp render (test_gpu_image.py).
 Tolerances are written next to each assert.  Integer/index results are exact.
 """
+import os
+
 import numpy as np
 import pytest
 
 from conftest import random_rays_in_room
 
 pytestmark = pytest.mark.gpu
+GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 
 REL_1E4 = 1e-4  # north_star: "1-bounce normals and depth must match within 1e-4 relative"
 
@@ -87,6 +90,20 @@ def test_nearest_hit_vs_reference_binary(gpu_api, ref_or_skip):
     np.testing.assert_allclose(got["points"], want["points"], rtol=1e-9, atol=1e-9)
     np.testing.assert_allclose(got["normals"], want["normals"], rtol=1e-9, atol=1e-9)
     np.testing.assert_allclose(got["uvs"], want["uvs"], rtol=1e-9, atol=1e-9)
+
+
+def test_nearest_hit_vs_reference_golden(gpu_api):
+    """the same check against the unmodified reference's intersect() outputs stored in
+    tests/golden/c1_hits.npz (make_golden.py): runs without the reference build"""
+    g = np.load(os.path.join(GOLD, "c1_hits.npz"))
+    rays = random_rays_in_room(np.random.default_rng(105), 3000)
+    with gpu_api.Scene(gpu_api.scene_default(320, 180)) as sc:
+        got = sc.trace_rays(rays)
+    assert np.array_equal(got["ids"], g["ids"])
+    hit = g["ids"] >= 0
+    assert hit.sum() > 1000
+    for k in ("points", "normals", "uvs"):
+        np.testing.assert_allclose(got[k][hit], g[k][hit], rtol=1e-9, atol=1e-9, err_msg=k)
 
 
 def test_bvh_equals_bruteforce_10k_spheres(gpu_api, ol):

@@ -42,9 +42,9 @@ def test_init_camera_bit_exact(R, api, wh):
     assert np.array_equal(api.init_camera(W, H, pos, tgt).as_array(), want)
 
 
-def test_default_camera_values(R):
+def test_default_camera_values(ol):
     """SURVEY.md 8(a) a3: C1 camera numbers measured on the reference"""
-    cam = R.init_camera(320, 180).as_array()
+    cam = ol.init_camera(320, 180).as_array()
     np.testing.assert_allclose(cam[3:6], (-2.0528, 0, 0), atol=1e-4)
     np.testing.assert_allclose(cam[6:9], (0, 1.1547, 0), atol=1e-4)
     np.testing.assert_allclose(cam[9:12], (1.0264, -0.57735, 51), atol=1e-4)
@@ -229,15 +229,15 @@ def test_reference_counters_default_run(R, api):
     assert tests % 38 == 0
 
 
-def test_stochastic_dielectric_has_the_split_expectation(R, api):
+def test_stochastic_dielectric_has_the_split_expectation(ol, api):
     """the GPU's estimator (one child per dielectric vertex) against the reference's split:
     same mean within Monte Carlo error on a dielectric-heavy scene"""
     W, H = 24, 14
     objs = api.scene_sphere_field(40, W, H, mix=(0.3, 0.6, 0.0))
-    cam = R.init_camera(W, H)
+    cam = ol.init_camera(W, H)
     S = 600
-    a, _ = R.render_sum(objs, cam, W, H, S, rng="philox", dielectric="split", max_depth=5, seed=11)
-    b, _ = R.render_sum(objs, cam, W, H, S, rng="philox", dielectric="stochastic", max_depth=5, seed=12)
+    a, _ = ol.render_sum(objs, cam, W, H, S, rng="philox", dielectric="split", max_depth=5, seed=11)
+    b, _ = ol.render_sum(objs, cam, W, H, S, rng="philox", dielectric="stochastic", max_depth=5, seed=12)
     a, b = a / S, b / S
     # frame-average radiance: 336 pixels x 600 samples each -> ~1% statistical error
     assert abs(a.mean() - b.mean()) / a.mean() < 0.03
