@@ -6,7 +6,7 @@
  *   rtb_scene_create*      the implicit "scene" = the Object[] the caller hands to
  *                          render() (raytracer.h:156, main.c:256-397, main.c:429); here it
  *                          is uploaded once (a pageable Vertex array is narrowed to floats on the way up when
- *                          every position is float-representable), converted AoS-double -> SoA on the device and
+ *                          every coordinate is float-representable), converted AoS-double -> SoA on the device and
  *                          a BVH is built over it (replaces the O(n) loop of intersect(),
  *                          raytracer.c:393-464)
  *   rtb_render_accum       the loop nest of render() up to the per-pixel sum
@@ -113,6 +113,8 @@ typedef struct
   int device;
   int double_triangles; /* 1: some mesh coordinate is not float-representable, the scene keeps the caller's doubles
                            (72 B per triangle) for the exact triangle test; 0: the float records are exact */
+  int double_texcoords; /* 1: some texture coordinate is not float-representable, the scene keeps the caller's doubles
+                           (48 B per triangle) for the checker pattern; 0: the float texture coordinates are exact */
 } rtb_scene_info;
 
 const char *rtb_last_error(void);

@@ -795,12 +795,25 @@ __device__ __forceinline__ Surface surface_at(const SceneView &sv, const d3 &o, 
       double t, bu, bv;
       if (triangle_exact(o, d, v0, v1, v2, t, bu, bv))
       {
-        float2 t0 = __ldg(sv.tex + 3 * best.slot + 0);
-        float2 t1 = __ldg(sv.tex + 3 * best.slot + 1);
-        float2 t2 = __ldg(sv.tex + 3 * best.slot + 2);
+        double t0x, t0y, t1x, t1y, t2x, t2y;
+        if (sv.tex64 != nullptr)
+        {
+          const double *q = sv.tex64 + 6 * (size_t)best.slot; /* 48-byte records: 16-byte aligned */
+          const double2 a = __ldg(reinterpret_cast<const double2 *>(q) + 0);
+          const double2 b = __ldg(reinterpret_cast<const double2 *>(q) + 1);
+          const double2 c = __ldg(reinterpret_cast<const double2 *>(q) + 2);
+          t0x = a.x; t0y = a.y; t1x = b.x; t1y = b.y; t2x = c.x; t2y = c.y;
+        }
+        else
+        {
+          const float2 a = __ldg(sv.tex + 3 * best.slot + 0);
+          const float2 b = __ldg(sv.tex + 3 * best.slot + 1);
+          const float2 c = __ldg(sv.tex + 3 * best.slot + 2);
+          t0x = a.x; t0y = a.y; t1x = b.x; t1y = b.y; t2x = c.x; t2y = c.y;
+        }
         double w0 = __dsub_rn(__dsub_rn(1.0, bu), bv); /* 1 - u - v, raytracer.c:160 */
-        s.u = __dadd_rn(__dadd_rn(__dmul_rn((double)t0.x, w0), __dmul_rn((double)t1.x, bu)), __dmul_rn((double)t2.x, bv));
-        s.v = __dadd_rn(__dadd_rn(__dmul_rn((double)t0.y, w0), __dmul_rn((double)t1.y, bu)), __dmul_rn((double)t2.y, bv));
+        s.u = __dadd_rn(__dadd_rn(__dmul_rn(t0x, w0), __dmul_rn(t1x, bu)), __dmul_rn(t2x, bv));
+        s.v = __dadd_rn(__dadd_rn(__dmul_rn(t0y, w0), __dmul_rn(t1y, bu)), __dmul_rn(t2y, bv));
       }
     }
   }

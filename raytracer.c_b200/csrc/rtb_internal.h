@@ -32,7 +32,7 @@ static_assert(sizeof(RefMesh) == 16, "TriangleMesh");
 static_assert(sizeof(RefSceneObject) == 96, "SceneObject");
 
 /* rtb_narrow.cpp: n_vertices Vertex records (five doubles) -> five floats each, on the host (AVX2 where the CPU has
- * it); true when every position is float-representable */
+ * it); true when every double -- positions and texture coordinates -- is float-representable */
 extern "C" bool rtb_narrow_vertices(const double *src, float *dst, size_t n_vertices);
 extern "C" bool rtb_narrow_vertices_scalar(const double *src, float *dst, size_t n_vertices);
 
@@ -97,6 +97,9 @@ struct SceneView
                            NULL when every mesh coordinate is float-representable (the floats of PrimRec are exact) */
   int n_prims, n_big, root_ref, n_objects;
   float guard_lo[3], guard_hi[3]; /* box rays are re-based into before FP32 traversal */
+  /* last, so that the fields the trace kernels read keep their parameter offsets */
+  const double *tex64;  /* 6 doubles per BVH primitive slot: texture coordinates exactly as the caller gave them, or
+                           NULL when every texture coordinate is float-representable (the floats of `tex` are exact) */
 };
 
 struct rtb_scene
@@ -109,6 +112,7 @@ struct rtb_scene
   float2 *d_tex = nullptr;
   double *d_colors = nullptr;
   double *d_tri64 = nullptr;
+  double *d_tex64 = nullptr;
   float *d_scratch = nullptr; /* split planes */
   size_t scratch_bytes = 0;
   void *d_wf = nullptr;       /* wavefront kernels: ray queues + accumulation planes (rtb_wavefront.cu) */
@@ -138,9 +142,10 @@ struct rtb_scene_shard
   void *nccl;
 };
 /* in-place all-gather (chunk `rank` of each array is this rank's) of the marshalled triangle records,
- * their boxes and (optionally) texture coordinates, on the legacy default stream of the current device */
+ * their boxes and (optionally) texture coordinates, on the legacy default stream of the current device;
+ * d_flags_max_or_null: int[2] max-reduced over the ranks ("needs double positions", "needs double texcoords") */
 int rtb_shard_allgather(const rtb_scene_shard *shard, void *prims, size_t prim_chunk_bytes, void *box_lo, void *box_hi,
-                        size_t box_chunk_bytes, void *tex_or_null, size_t tex_chunk_bytes, int *d_flag_max_or_null);
+                        size_t box_chunk_bytes, void *tex_or_null, size_t tex_chunk_bytes, int *d_flags_max_or_null);
 int rtb_shard_allgather_bytes(const rtb_scene_shard *shard, void *base, size_t chunk_bytes);
 int rtb_scene_create_sharded(const void *objects, size_t n_objects, int kind, int device, unsigned flags,
                              const rtb_scene_shard *shard, rtb_scene **out);

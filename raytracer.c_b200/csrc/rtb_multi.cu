@@ -235,7 +235,7 @@ extern "C" void rtb_comm_destroy(rtb_comm *comm)
 
 /* rtb_scene.cu calls this in the middle of a sharded build */
 int rtb_shard_allgather(const rtb_scene_shard *shard, void *prims, size_t prim_chunk_bytes, void *box_lo, void *box_hi,
-                        size_t box_chunk_bytes, void *tex_or_null, size_t tex_chunk_bytes, int *d_flag_max_or_null)
+                        size_t box_chunk_bytes, void *tex_or_null, size_t tex_chunk_bytes, int *d_flags_max_or_null)
 {
   ncclComm_t comm = static_cast<ncclComm_t>(shard->nccl);
   const size_t r = (size_t)shard->rank;
@@ -246,8 +246,8 @@ int rtb_shard_allgather(const rtb_scene_shard *shard, void *prims, size_t prim_c
   RTB_NCCL(nccl_api().AllGather(mine(box_hi, box_chunk_bytes), box_hi, box_chunk_bytes, ncclChar, comm, 0));
   if (tex_or_null)
     RTB_NCCL(nccl_api().AllGather(mine(tex_or_null, tex_chunk_bytes), tex_or_null, tex_chunk_bytes, ncclChar, comm, 0));
-  if (d_flag_max_or_null)
-    RTB_NCCL(nccl_api().AllReduce(d_flag_max_or_null, d_flag_max_or_null, 1, ncclInt32, ncclMax, comm, 0));
+  if (d_flags_max_or_null)
+    RTB_NCCL(nccl_api().AllReduce(d_flags_max_or_null, d_flags_max_or_null, 2, ncclInt32, ncclMax, comm, 0));
   RTB_NCCL(nccl_api().GroupEnd());
   return RTB_OK;
 }

@@ -64,7 +64,8 @@ def path_cases(seed=103, n=200):
 
 def whitted_golden():
     """cast_ray (raytracer.c:556-641) of the unmodified reference on fixed rays: the default scene
-    (checkered + mirror + dielectric spheres) and a packed sphere field with mixed materials"""
+    (diffuse and mirror spheres; no checkered object) and a packed sphere field with mixed materials
+    (tests/test_gpu_texture.py checks checkered spheres against the reference's cast_ray)"""
     out = {}
     rays = random_rays_in_room(np.random.default_rng(106), 3000)
     objs = api.scene_default(320, 180)

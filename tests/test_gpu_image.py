@@ -75,28 +75,52 @@ def test_golden_hits_on_device(gpu_api):
             np.testing.assert_allclose(got["uvs"], g["uvs"], rtol=0, atol=1e-15)  # atan2: libm vs CUDA
 
 
-@pytest.mark.parametrize("kernel", [1, 2, 3, 4, 5, 6])
-def test_kernel_variants_agree(gpu_api, kernel):
+def _checkered_scene(gpu_api, abi, W, H):
+    """scene_mesh_room with checkered surfaces of every material (mesh, walls, mirror and glass balls) and a mesh
+    whose texture coordinates are genuine doubles, unrelated to position: the scene keeps them as doubles, and a
+    texture coordinate read from the wrong triangle or rounded to float changes the checker at M = 100 000"""
+    verts = gpu_api.heightfield_mesh(40, 20 * W / H * 0.98)
+    verts["tex"] = np.random.default_rng(8).uniform(0.0, 1.0, (len(verts), 2))
+    holder = gpu_api.mesh_room(verts, W, H)
+    for k in (1, 2, 6, 11, 12):
+        holder.objects[k].material.flags |= abi.M_CHECKERED
+    return holder
+
+
+@pytest.mark.parametrize("kernel,scene", [(k, "field") for k in range(1, 7)] + [(k, "checkered") for k in range(1, 7)],
+                         ids=[str(k) for k in range(1, 7)] + [f"{k}-checkered" for k in range(1, 7)])
+def test_kernel_variants_agree(gpu_api, abi, kernel, scene):
     """megakernel, warp-scheduled state machine, the FP32 pre-test variants and the wavefront
     kernels compute the same per-pixel sums (same Philox streams, same exact tests, same
-    order of additions)"""
+    order of additions) -- on a sphere field and on a scene with checkered surfaces"""
     W, H, SPP = 96, 54, 8
-    objs = gpu_api.scene_sphere_field(400, W, H, mix=(0.3, 0.3, 0.3))
+    if scene == "field":
+        objs = gpu_api.scene_sphere_field(400, W, H, mix=(0.3, 0.3, 0.3))
+    else:
+        objs = _checkered_scene(gpu_api, abi, W, H)
     cam = gpu_api.init_camera(W, H)
     with gpu_api.Scene(objs, all_trees=True) as sc:
+        info = sc.info
         _, base, c0 = sc.render(cam, gpu_api.make_desc(W, H, 0, SPP, max_depth=8, kernel=0), want_accum=True)
         _, acc, c1 = sc.render(cam, gpu_api.make_desc(W, H, 0, SPP, max_depth=8, kernel=kernel), want_accum=True)
     assert np.array_equal(acc, base)
     assert c0.rays == c1.rays and c0.paths == c1.paths
+    assert info.double_texcoords == (scene == "checkered")
 
 
-@pytest.mark.parametrize("spp,planes", [(7, 3), (6, 1), (5, 5), (9, 2)])
-def test_wavefront_equals_megakernel_on_a_mesh(gpu_api, spp, planes):
+@pytest.mark.parametrize("spp,planes,checkered", [(7, 3, False), (6, 1, False), (5, 5, False), (9, 2, False),
+                                                  (7, 3, True), (5, 5, True)],
+                         ids=["7-3", "6-1", "5-5", "9-2", "7-3-checkered", "5-5-checkered"])
+def test_wavefront_equals_megakernel_on_a_mesh(gpu_api, abi, spp, planes, checkered):
     """wavefront (ray queues + persistent trace kernel) vs megakernel on a mesh + spheres scene,
-    including ragged plane/wave combinations: bit-identical sums and equal counters"""
+    including ragged plane/wave combinations: bit-identical sums and equal counters; also with
+    checkered surfaces and double texture coordinates"""
     W, H = 80, 46  # not a multiple of the 8x4 tile
-    verts = gpu_api.heightfield_mesh(40, 20 * W / H * 0.98)
-    holder = gpu_api.mesh_room(verts, W, H)
+    if checkered:
+        holder = _checkered_scene(gpu_api, abi, W, H)
+    else:
+        verts = gpu_api.heightfield_mesh(40, 20 * W / H * 0.98)
+        holder = gpu_api.mesh_room(verts, W, H)
     cam = gpu_api.init_camera(W, H)
     with gpu_api.Scene(holder, all_trees=True) as sc:
         _, base, c0 = sc.render(cam, gpu_api.make_desc(W, H, 3, 3 + spp, max_depth=6, kernel=4, planes=planes), want_accum=True)

@@ -321,9 +321,7 @@ def test_render_params_carry_num_gpus(pkg):
 
 # ---- narrowed mesh upload: the host-side conversion (csrc/rtb_narrow.cpp) --------------------------------
 
-def test_narrow_vertices_equals_numpy_and_flags_inexact_positions(api):
-    """15 doubles -> 15 floats per triangle: round-to-nearest like numpy, vector form == scalar form, and the
-    `exact` result is false exactly when a POSITION (not a texture coordinate) loses bits, overflows or is NaN"""
+def _narrow_fns(api):
     import ctypes as C
     cu, _ = api.load()
     fns = []
@@ -332,10 +330,18 @@ def test_narrow_vertices_equals_numpy_and_flags_inexact_positions(api):
         f.restype = C.c_bool
         f.argtypes = [C.c_void_p, C.c_void_p, C.c_size_t]
         fns.append(f)
+    return fns
+
+
+def test_narrow_vertices_equals_numpy_and_flags_every_inexact_lane(api):
+    """15 doubles -> 15 floats per triangle: round-to-nearest like numpy, vector form == scalar form, and the
+    `exact` result is false exactly when some lane -- a position or a texture coordinate -- loses bits, overflows
+    or is NaN"""
+    fns = _narrow_fns(api)
     rng = np.random.default_rng(5)
     for n in (0, 1, 3, 4, 5, 12, 13, 1000, 4099):
         src = rng.uniform(-50, 50, (n, 5)).astype(np.float32).astype(np.float64)
-        src[:, 3:] = rng.uniform(0, 1, (n, 2))  # texture coordinates: genuine doubles, rounded, never "inexact"
+        src[:, 3:] = rng.uniform(0, 1, (n, 2)).astype(np.float32)  # texture coordinates: floats, like an OBJ file's
         for f in fns:
             dst = np.full((n, 5), -1.0, np.float32)
             assert f(src.ctypes.data, dst.ctypes.data, n) is True
@@ -350,9 +356,37 @@ def test_narrow_vertices_equals_numpy_and_flags_inexact_positions(api):
                     for f in fns:
                         dst = np.zeros((n, 5), np.float32)
                         exact = f(s2.ctypes.data, dst.ctypes.data, n)
-                        assert exact is (a >= 3), (n, v, a, bad)
+                        assert exact is False, (n, v, a, bad)
                         with np.errstate(over="ignore"):
                             assert np.array_equal(dst, s2.astype(np.float32), equal_nan=True)
+
+
+def test_narrow_vertices_flags_an_inexact_texcoord_in_every_lane(api):
+    """only a texture coordinate is not float-representable (a caller's double texcoords): both forms report
+    "inexact" wherever it sits -- every texcoord slot of a four-vertex group, i.e. each of the five 256-bit vectors
+    of the AVX2 form and every lane position a texcoord takes there, and the scalar tail -- and still convert like
+    numpy; positions alone that are floats stay exact"""
+    fns = _narrow_fns(api)
+    rng = np.random.default_rng(6)
+    for n in (4, 8, 11):
+        src = rng.uniform(-50, 50, (n, 5)).astype(np.float32).astype(np.float64)
+        src[:, 3:] = rng.uniform(0, 1, (n, 2)).astype(np.float32)
+        slots = set()
+        for v in range(n):
+            for a in (3, 4):
+                k = 5 * (v % 4) + a  # double index inside the vertex's group of four
+                if v < 4 * (n // 4):
+                    slots.add((k // 4, k % 4))  # (vector, lane) of the AVX2 form
+                for bad in (src[v, a] + 2.0 ** -40, -700.123456789, 1e300, float("nan")):
+                    s2 = src.copy()
+                    s2[v, a] = bad
+                    for f in fns:
+                        dst = np.zeros((n, 5), np.float32)
+                        assert f(s2.ctypes.data, dst.ctypes.data, n) is False, (n, v, a, bad)
+                        with np.errstate(over="ignore"):
+                            assert np.array_equal(dst, s2.astype(np.float32), equal_nan=True)
+        assert {vec for vec, _ in slots} == {0, 1, 2, 3, 4}
+        assert len(slots) == 8  # texcoords are doubles 3, 4, 8, 9, 13, 14, 18, 19 of a group
 
 
 def test_apply_matrix_is_the_same_for_any_thread_count(api, monkeypatch):
