@@ -15,6 +15,7 @@
  *   rtb_tonemap            mean, gamma 5.0, 8-bit truncation (raytracer.c:215-220)
  *   rtb_render             the whole of render() (raytracer.c:176-223), host buffers in/out
  *   rtb_trace_rays         intersect() for arbitrary rays (raytracer.c:393-464): parity probe
+ *   rtb_trace_rays_wf      the same records from the wavefront renderer's trace kernel: parity probe
  *   rtb_path_records       per-path vertex records: parity probe for the 1-bounce check
  *   rtb_cast_rays          cast_ray() for arbitrary rays (raytracer.c:556-641): parity probe of the
  *                          Whitted integrator (rtb_render_desc.integrator = RTB_INTEGRATOR_WHITTED)
@@ -115,6 +116,8 @@ typedef struct
                            (72 B per triangle) for the exact triangle test; 0: the float records are exact */
   int double_texcoords; /* 1: some texture coordinate is not float-representable, the scene keeps the caller's doubles
                            (48 B per triangle) for the checker pattern; 0: the float texture coordinates are exact */
+  int bvh4_depth;       /* levels of the compressed BVH4 the product path walks; 0 when it walks the BVH2 instead (a
+                           tree too deep for the BVH4 walk's stack) or there is no tree */
 } rtb_scene_info;
 
 const char *rtb_last_error(void);
@@ -163,6 +166,14 @@ int rtb_render_mean(rtb_scene *scene, const double *camera12, const rtb_render_d
 /* parity probes (host buffers) */
 int rtb_trace_rays(rtb_scene *scene, const double *rays6, size_t n_rays, int use_bvh, int32_t *ids,
                    int64_t *prims, double *ts, double *points, double *normals, double *uvs);
+/* same records as rtb_trace_rays, computed by the wavefront renderer's own trace kernel: the rays are queued with
+ * their hit records seeded from the oversized list, as the renderer queues them, and one launch of the trace kernel
+ * that `tune` selects (rtb_render_desc.reserved encoding, 0 = the renderer's default) finds the nearest hits.
+ * perm_or_null: the order the kernel fetches queue entries in (a permutation of [0, n_rays), else RTB_EINVAL).
+ * counters_or_null: prim_tests (oversized list + leaves) and node_visits of the call. */
+int rtb_trace_rays_wf(rtb_scene *scene, const double *rays6, size_t n_rays, int tune,
+                      const uint32_t *perm_or_null, int32_t *ids, int64_t *prims, double *ts,
+                      double *points, double *normals, double *uvs, rtb_counters *counters_or_null);
 int rtb_path_records(rtb_scene *scene, const double *camera12, const rtb_render_desc *desc, int sample,
                      int n_vertices, int32_t *ids, double *points, double *normals, double *dists,
                      float *radiance);

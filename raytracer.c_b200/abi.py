@@ -105,7 +105,8 @@ class RtbSceneInfo(C.Structure):
     _fields_ = [("n_objects", C.c_size_t), ("n_spheres", C.c_size_t), ("n_triangles", C.c_size_t),
                 ("n_bvh_prims", C.c_size_t), ("n_bvh_nodes", C.c_size_t), ("n_big_prims", C.c_size_t),
                 ("device_bytes", C.c_size_t), ("build_ms", C.c_float), ("bvh_depth", C.c_int),
-                ("device", C.c_int), ("double_triangles", C.c_int), ("double_texcoords", C.c_int)]
+                ("device", C.c_int), ("double_triangles", C.c_int), ("double_texcoords", C.c_int),
+                ("bvh4_depth", C.c_int)]
 
 
 EXPECTED_SIZES = {Vertex: 40, Material: 80, Sphere: 32, TriangleMesh: 16, Object: 88,

@@ -22,7 +22,7 @@ RTB_SYMBOLS = [
     "rtb_last_error", "rtb_version", "rtb_device_count", "rtb_scene_create_objects", "rtb_scene_create",
     "rtb_scene_create_objects_flags", "rtb_scene_create_flags",
     "rtb_scene_info_get", "rtb_scene_destroy", "rtb_release_workspace", "rtb_render_accum", "rtb_tonemap", "rtb_render",
-    "rtb_trace_rays", "rtb_path_records", "rtb_philox4x32_10", "rtb_probe_l2_bandwidth", "rtb_cast_rays",
+    "rtb_trace_rays", "rtb_trace_rays_wf", "rtb_path_records", "rtb_philox4x32_10", "rtb_probe_l2_bandwidth", "rtb_cast_rays",
     "rtb_probe_fp32_tflops", "rtb_render_mean", "rtb_comm_unique_id", "rtb_comm_create_rank", "rtb_comm_create_local", "rtb_comm_size",
     "rtb_warm_up", "rtb_comm_local_ranks", "rtb_comm_destroy", "rtb_comm_shard_samples", "rtb_comm_scene_create", "rtb_comm_render", "rtb_render_multi",
 ]
@@ -78,6 +78,8 @@ def _bind(cu, host):
     cu.rtb_render.argtypes = [C.c_void_p, dp, C.POINTER(abi.RtbRenderDesc), C.c_void_p, C.c_void_p,
                               C.POINTER(abi.RtbCounters)]
     cu.rtb_trace_rays.argtypes = [C.c_void_p, C.c_void_p, C.c_size_t, C.c_int] + [C.c_void_p] * 6
+    cu.rtb_trace_rays_wf.argtypes = [C.c_void_p, C.c_void_p, C.c_size_t, C.c_int] + [C.c_void_p] * 7 + [
+        C.POINTER(abi.RtbCounters)]
     cu.rtb_path_records.argtypes = [C.c_void_p, dp, C.POINTER(abi.RtbRenderDesc), C.c_int, C.c_int] + [C.c_void_p] * 5
     cu.rtb_philox4x32_10.argtypes = [C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, C.c_int]
     cu.rtb_cast_rays.argtypes = [C.c_void_p, C.c_void_p, C.c_size_t, C.c_int, C.c_void_p, C.c_void_p]
@@ -352,6 +354,25 @@ class Scene:
                                        out["prims"].ctypes.data, out["t"].ctypes.data, out["points"].ctypes.data,
                                        out["normals"].ctypes.data, out["uvs"].ctypes.data), "rtb_trace_rays")
         return out
+
+    def trace_rays_wf(self, rays, tune=0, perm=None):
+        """the same records as trace_rays, from the wavefront renderer's trace kernel (rtb_trace_rays_wf): `tune` is
+        a rtb_render_desc.reserved word (0 = the renderer's default kernel), `perm` the order the kernel fetches
+        the rays in -> (records, abi.RtbCounters with prim_tests and node_visits)"""
+        rays = np.ascontiguousarray(rays, dtype=np.float64).reshape(-1, 6)
+        n = len(rays)
+        out = dict(ids=np.zeros(n, np.int32), prims=np.zeros(n, np.int64), t=np.zeros(n, np.float64),
+                   points=np.zeros((n, 3), np.float64), normals=np.zeros((n, 3), np.float64),
+                   uvs=np.zeros((n, 2), np.float64))
+        p = None if perm is None else np.ascontiguousarray(perm, dtype=np.uint32)
+        if p is not None and p.shape != (n,):
+            raise ValueError(f"perm must have {n} entries")
+        ctr = abi.RtbCounters()
+        _check(self._cu.rtb_trace_rays_wf(self._h, rays.ctypes.data, n, int(tune), p.ctypes.data if p is not None else None,
+                                          out["ids"].ctypes.data, out["prims"].ctypes.data, out["t"].ctypes.data,
+                                          out["points"].ctypes.data, out["normals"].ctypes.data, out["uvs"].ctypes.data,
+                                          C.byref(ctr)), "rtb_trace_rays_wf")
+        return out, ctr
 
     def cast_rays(self, rays, max_depth=5):
         """cast_ray() of the Whitted integrator (raytracer.c:556-641) for arbitrary rays ->

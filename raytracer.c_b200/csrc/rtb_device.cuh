@@ -313,6 +313,17 @@ __device__ __forceinline__ bool rayf_walk_setup(const SceneView &sv, const d3 &o
                  ofy > sv.guard_hi[1] || ofz < sv.guard_lo[2] || ofz > sv.guard_hi[2];
   if (outside)
   {
+    /* an origin too far away for the culling walk to be conservative (SceneView::far_t, set by the build): every
+     * box is entered at distance 0 and no stack entry is culled, so every leaf gets its exact test */
+    const float dist = fmaxf(fmaxf(fmaxf(sv.guard_lo[0] - ofx, ofx - sv.guard_hi[0]), fmaxf(sv.guard_lo[1] - ofy, ofy - sv.guard_hi[1])),
+                             fmaxf(sv.guard_lo[2] - ofz, ofz - sv.guard_hi[2]));
+    if (dist > sv.far_t)
+    {
+      rf.idx = rf.idy = rf.idz = 0.0f;
+      rf.oodx = rf.oody = rf.oodz = 0.0f;
+      rf.tmax = 3.0e38f;
+      return true;
+    }
     float ax = (sv.guard_lo[0] - ofx) * rf.idx, bx = (sv.guard_hi[0] - ofx) * rf.idx;
     float ay = (sv.guard_lo[1] - ofy) * rf.idy, by = (sv.guard_hi[1] - ofy) * rf.idy;
     float az = (sv.guard_lo[2] - ofz) * rf.idz, bz = (sv.guard_hi[2] - ofz) * rf.idz;
@@ -818,6 +829,25 @@ __device__ __forceinline__ Surface surface_at(const SceneView &sv, const d3 &o, 
     }
   }
   return s;
+}
+
+/* record i of the nearest-hit probes (rtb_trace_rays, rtb_trace_rays_wf): object id (-1 = miss), primitive gid, t,
+ * point, normal and texture coordinates at the hit; any output pointer but ids may be NULL */
+__device__ __forceinline__ void store_hit_record(const SceneView &sv, const d3 &o, const d3 &d, const HitRec &best, size_t i,
+                                                 int *__restrict__ ids, long long *__restrict__ prims,
+                                                 double *__restrict__ ts, double *__restrict__ points,
+                                                 double *__restrict__ normals, double *__restrict__ uvs)
+{
+  bool hit = best.t < 1e300;
+  Surface s;
+  if (hit)
+    s = surface_at(sv, o, d, best, true);
+  ids[i] = hit ? s.object : -1;
+  if (prims) prims[i] = hit ? (long long)best.gid : -1ll;
+  if (ts) ts[i] = hit ? best.t : 0.0;
+  if (points)  { points[3 * i] = hit ? s.point.x : 0; points[3 * i + 1] = hit ? s.point.y : 0; points[3 * i + 2] = hit ? s.point.z : 0; }
+  if (normals) { normals[3 * i] = hit ? s.normal.x : 0; normals[3 * i + 1] = hit ? s.normal.y : 0; normals[3 * i + 2] = hit ? s.normal.z : 0; }
+  if (uvs)     { uvs[2 * i] = hit ? s.u : 0; uvs[2 * i + 1] = hit ? s.v : 0; }
 }
 
 /* ---- camera (raytracer.c:375-384) ------------------------------------------- */

@@ -100,6 +100,7 @@ struct SceneView
   /* last, so that the fields the trace kernels read keep their parameter offsets */
   const double *tex64;  /* 6 doubles per BVH primitive slot: texture coordinates exactly as the caller gave them, or
                            NULL when every texture coordinate is float-representable (the floats of `tex` are exact) */
+  float far_t; /* origins farther than this outside the guard box are walked without culling (rayf_walk_setup) */
 };
 
 struct rtb_scene
@@ -149,6 +150,14 @@ int rtb_shard_allgather(const rtb_scene_shard *shard, void *prims, size_t prim_c
 int rtb_shard_allgather_bytes(const rtb_scene_shard *shard, void *base, size_t chunk_bytes);
 int rtb_scene_create_sharded(const void *objects, size_t n_objects, int kind, int device, unsigned flags,
                              const rtb_scene_shard *shard, rtb_scene **out);
+
+/* a plain cudaMalloc'd buffer of the probes, freed on every return path */
+template <typename T>
+struct Dev
+{
+  T *p = nullptr;
+  ~Dev() { if (p) cudaFree(p); }
+};
 
 /* error plumbing */
 void rtb_set_error(const std::string &msg);

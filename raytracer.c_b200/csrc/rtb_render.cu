@@ -509,16 +509,7 @@ __global__ void k_trace_rays(const __grid_constant__ SceneView sv, const double 
     closest_hit<false, false>(sv, o, d, best, st);
   else
     closest_hit_bruteforce(sv, o, d, best);
-  bool hit = best.t < 1e300;
-  Surface s;
-  if (hit)
-    s = surface_at(sv, o, d, best, true);
-  ids[i] = hit ? s.object : -1;
-  if (prims) prims[i] = hit ? (long long)best.gid : -1ll;
-  if (ts) ts[i] = hit ? best.t : 0.0;
-  if (points)  { points[3 * i] = hit ? s.point.x : 0; points[3 * i + 1] = hit ? s.point.y : 0; points[3 * i + 2] = hit ? s.point.z : 0; }
-  if (normals) { normals[3 * i] = hit ? s.normal.x : 0; normals[3 * i + 1] = hit ? s.normal.y : 0; normals[3 * i + 2] = hit ? s.normal.z : 0; }
-  if (uvs)     { uvs[2 * i] = hit ? s.u : 0; uvs[2 * i + 1] = hit ? s.v : 0; }
+  store_hit_record(sv, o, d, best, i, ids, prims, ts, points, normals, uvs);
 }
 
 /* the first n_vertices vertices of sample `sample` of every pixel, through the very same
@@ -916,13 +907,6 @@ extern "C" int rtb_render_mean(rtb_scene *scene, const double *camera12, const r
   cudaFreeAsync(d_fb, 0);
   return rc;
 }
-
-template <typename T>
-struct Dev
-{
-  T *p = nullptr;
-  ~Dev() { if (p) cudaFree(p); }
-};
 
 extern "C" int rtb_trace_rays(rtb_scene *scene, const double *rays6, size_t n_rays, int use_bvh, int32_t *ids,
                               int64_t *prims, double *ts, double *points, double *normals, double *uvs)

@@ -1181,6 +1181,7 @@ int build_scene(HostScene &hs, int device, unsigned flags, const rtb_scene_shard
     view.guard_lo[k] = -FLT_MAX;
     view.guard_hi[k] = FLT_MAX;
   }
+  view.far_t = FLT_MAX;
   int bvh_depth = 0;
   size_t n_nodes = 0;
 
@@ -1214,6 +1215,7 @@ int build_scene(HostScene &hs, int device, unsigned flags, const rtb_scene_shard
   int *const h_misc = rb.misc;
   int &h_nodes4 = rb.nodes4;
   bool bvh4_ok = true;
+  int depth4 = 0; /* levels of the BVH4 */
 
   if (N > 0)
   {
@@ -1523,9 +1525,29 @@ int build_scene(HostScene &hs, int device, unsigned flags, const rtb_scene_shard
       view.guard_lo[k] = h_bp.guard_lo[k];
       view.guard_hi[k] = h_bp.guard_hi[k];
     }
+    /* How far outside the guard box an origin may lie for the culling FP32 walk to stay conservative (beyond it,
+     * rayf_walk_setup walks every box: the nearest hit is then the brute-force one by construction):
+     *  - the walk re-bases such a ray to 0.001 t_in before the guard box; within 300 guard diagonals that point
+     *    stays within one guard diagonal of it, inside the envelope the box padding was sized for (k_build_params);
+     *  - the exact sphere test (raytracer.c:77-118) computes d2 = L.L - tca^2 with an error of at most
+     *    16 |L|^2 2^-53; a box cull is safe while that stays below 2 r pad (a ray that passes the padded box
+     *    of a sphere of radius r cannot then be accepted by the exact test), which bounds |L| for the smallest
+     *    sphere in the tree. */
+    {
+      double gd = 0.0;
+      for (int k = 0; k < 3; k++)
+        gd += ((double)h_bp.guard_hi[k] - h_bp.guard_lo[k]) * ((double)h_bp.guard_hi[k] - h_bp.guard_lo[k]);
+      gd = sqrt(gd);
+      double far = 300.0 * gd;
+      double r_min = HUGE_VAL;
+      for (const SphereIn &s : bvh_spheres)
+        r_min = std::min(r_min, std::fabs(s.r));
+      if (r_min < HUGE_VAL)
+        far = std::min(far, sqrt(2.0 * r_min * (double)h_bp.pad * 9007199254740992.0 / 16.0) - gd);
+      view.far_t = (float)std::max(far, 0.0);
+    }
     bvh_depth = h_misc[0];
     n_nodes = (size_t)h_nodes4; /* nodes of the tree the default path walks */
-    int depth4 = 0;
     while (depth4 < RTB_STACK_SIZE && h_levels[depth4] > 0)
       depth4++;
     /* the BVH2 walk pushes at most one entry per level, the BVH4 walk at most three */
@@ -1564,6 +1586,7 @@ int build_scene(HostScene &hs, int device, unsigned flags, const rtb_scene_shard
   sc->info.device = device;
   sc->info.double_triangles = h_inexact ? 1 : 0;
   sc->info.double_texcoords = h_tex_inexact ? 1 : 0;
+  sc->info.bvh4_depth = view.nodes4q != nullptr ? depth4 : 0;
   *out = sc.release();
   return RTB_OK;
 }

@@ -27,6 +27,7 @@
 #include "rtb_path.cuh"
 
 #include <algorithm>
+#include <cstring>
 #include <mutex>
 #include <vector>
 #include <cub/cub.cuh>
@@ -853,6 +854,86 @@ __global__ void k_wf_iota(unsigned *v, unsigned n)
 
 static size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
 
+/* the trace kernel a tuning word selects (rtb_render_desc.reserved): bits 0-7 refill threshold, 8-15 node-phase
+ * exit threshold, 16-27 trace kernel variant; 0 = the measured defaults */
+struct WfTraceTune
+{
+  int variant;     /* template argument of k_wf_trace */
+  bool pool;       /* k_wf_trace_pool instead */
+  int refill_word; /* refill threshold | guided batch word << 8 */
+  int node_exit;   /* 0 = pure while-while */
+  int leaf_min;    /* k_wf_trace_pool: leaf-phase threshold */
+};
+
+static int wf_trace_tune(const SceneView &sv, int tune, WfTraceTune &t)
+{
+  int refill_idle = ((tune & 0xFF) > 0 && (tune & 0xFF) <= 32) ? (tune & 0xFF) : 8;
+  /* bits 8-15 of the word handed to k_wf_trace: guided self-scheduling of the ray batches -- a batch is
+   * min(512 << (g >> 4), rays left / (warps * (g & 15))), at least 32.  Measured default g = 1
+   * (profiles/r2_wf_tuning.md section 2i); development knob RTB_WF_GUIDED (0: fixed batches) */
+  {
+    const char *e = getenv("RTB_WF_GUIDED");
+    refill_idle |= (e ? (atoi(e) & 0xFF) : 1) << 8;
+  }
+  t.refill_word = refill_idle;
+  t.node_exit = (tune >> 8) & 0xFF;
+  t.variant = (tune >> 16) & 0xFFF;
+  if (tune == 0)
+  {
+    /* measured defaults (profiles/r1_wf_tuning.md) */
+    t.node_exit = 16;
+    t.variant = 22; /* compressed BVH4 + local stack + streaming queue loads */
+  }
+  if (t.node_exit == 0xFF)
+    t.node_exit = 0; /* pure while-while */
+  if ((t.variant & (8 | 16)) != 0 && sv.nodes4q == nullptr && sv.root_ref >= 0 && sv.root_ref != RTB_REF_NONE)
+    t.variant = 6; /* the scene has no BVH4 (tree too deep for its stack): BVH2 walk */
+  t.pool = t.variant == 1024 && sv.nodes4q != nullptr; /* the ray-pool form of the trace kernel */
+  t.leaf_min = (tune & 0xFF00) ? std::min(std::max(t.node_exit, 1), 32) : 32;
+  /* the BVH2 and the uncompressed BVH4 exist only in RTB_SCENE_ALL_TREES scenes (or as the fallback above) */
+  const bool walks = sv.root_ref >= 0 && sv.root_ref != RTB_REF_NONE;
+  const bool bvh2 = !t.pool && (t.variant & (8 | 16)) == 0, bvh4 = !t.pool && (t.variant & (8 | 16)) == 8;
+  if (walks && ((bvh2 && sv.nodes == nullptr) || (bvh4 && sv.nodes4 == nullptr)))
+  {
+    rtb_set_error("wavefront trace variant " + std::to_string(t.variant) +
+                  " walks the BVH2 / uncompressed BVH4: create the scene with RTB_SCENE_ALL_TREES");
+    return RTB_EINVAL;
+  }
+  return RTB_OK;
+}
+
+/* device bytes of the ray pool's traversal stacks (0 unless the tuning word selects the pool) */
+static size_t wf_pool_stack_bytes(const WfTraceTune &t, int sm_count)
+{
+  return t.pool ? align_up((size_t)sm_count * 8 * 4 * RTB_STACK_SIZE * WF_POOL_RAYS * sizeof(int2), 256) : 0;
+}
+
+/* one launch of the trace kernel `t` selects over queue q (the ray pool reads the queue in order: no perm) */
+static void wf_launch_trace(const WfTraceTune &t, bool stats, int sm_count, cudaStream_t st, const SceneView &sv,
+                            const WfQueue &q, const unsigned *n_ptr, unsigned *fetch, unsigned long long *totals,
+                            int2 *pool_stacks, const unsigned *perm)
+{
+  const int ri = t.refill_word, ne = t.node_exit;
+  if (t.pool)
+  {
+    launch_trace_pool(stats, sm_count, st, sv, q, n_ptr, fetch, totals, pool_stacks, t.leaf_min);
+    return;
+  }
+  switch (t.variant)
+  {
+  case 2: launch_trace<2>(stats, sm_count, st, sv, q, n_ptr, fetch, totals, ri, ne, perm); break;
+  case 22: launch_trace<22>(stats, sm_count, st, sv, q, n_ptr, fetch, totals, ri, ne, perm); break;
+  case 54: launch_trace<54>(stats, sm_count, st, sv, q, n_ptr, fetch, totals, ri, ne, perm); break;
+  case 86: launch_trace<86>(stats, sm_count, st, sv, q, n_ptr, fetch, totals, ri, ne, perm); break;
+  case 150: launch_trace<150>(stats, sm_count, st, sv, q, n_ptr, fetch, totals, ri, ne, perm); break;
+  case 182: launch_trace<182>(stats, sm_count, st, sv, q, n_ptr, fetch, totals, ri, ne, perm); break;
+  case 214: launch_trace<214>(stats, sm_count, st, sv, q, n_ptr, fetch, totals, ri, ne, perm); break;
+  case 10: launch_trace<10>(stats, sm_count, st, sv, q, n_ptr, fetch, totals, ri, ne, perm); break;
+  case 6: launch_trace<6>(stats, sm_count, st, sv, q, n_ptr, fetch, totals, ri, ne, perm); break;
+  default: launch_trace<0>(stats, sm_count, st, sv, q, n_ptr, fetch, totals, ri, ne, perm); break;
+  }
+}
+
 int wf_render(rtb_scene *scene, RenderArgs &A, const rtb_render_desc *desc, float *d_accum, cudaStream_t stream,
               bool stats, unsigned long long &launches, float *phase_ms)
 {
@@ -876,28 +957,11 @@ int wf_render(rtb_scene *scene, RenderArgs &A, const rtb_render_desc *desc, floa
     return RTB_EINVAL;
   }
 
-  /* tuning word (desc->reserved): bits 0-7 refill threshold, 8-15 node-phase exit threshold,
-   * 16-23 trace kernel variant; desc->reserved2: ray sorting mode (0 = off) */
-  int refill_idle = ((desc->reserved & 0xFF) > 0 && (desc->reserved & 0xFF) <= 32) ? (desc->reserved & 0xFF) : 8;
-  /* bits 8-15 of the word handed to k_wf_trace: guided self-scheduling of the ray batches -- a batch is
-   * min(512 << (g >> 4), rays left / (warps * (g & 15))), at least 32.  Measured default g = 1
-   * (profiles/r2_wf_tuning.md section 2i); development knob RTB_WF_GUIDED (0: fixed batches) */
-  {
-    const char *e = getenv("RTB_WF_GUIDED");
-    refill_idle |= (e ? (atoi(e) & 0xFF) : 1) << 8;
-  }
-  int node_exit = (desc->reserved >> 8) & 0xFF;
-  int variant = (desc->reserved >> 16) & 0xFFF;
-  if (desc->reserved == 0)
-  {
-    /* measured defaults (profiles/r1_wf_tuning.md) */
-    node_exit = 16;
-    variant = 22; /* compressed BVH4 + local stack + streaming queue loads */
-  }
-  if (node_exit == 0xFF)
-    node_exit = 0; /* pure while-while */
-  if ((variant & (8 | 16)) != 0 && A.sv.nodes4q == nullptr && A.sv.root_ref >= 0 && A.sv.root_ref != RTB_REF_NONE)
-    variant = 6; /* the scene has no BVH4 (tree too deep for its stack): BVH2 walk */
+  /* tuning word (desc->reserved): the trace kernel, wf_trace_tune; desc->reserved2: ray sorting mode (0 = off) */
+  WfTraceTune tune;
+  const int tune_rc = wf_trace_tune(A.sv, desc->reserved, tune);
+  if (tune_rc != RTB_OK)
+    return tune_rc;
   const int sort_mode = split ? 0 : (desc->reserved2 & 0xFF);
   const int sort_from = 1;                                           /* primary rays are coherent already */
   const int sort_until = (desc->reserved2 >> 8) & 0xFF ? (desc->reserved2 >> 8) & 0xFF : 255;
@@ -917,8 +981,8 @@ int wf_render(rtb_scene *scene, RenderArgs &A, const rtb_render_desc *desc, floa
   }
   int sm_count = 148;
   cudaDeviceGetAttribute(&sm_count, cudaDevAttrMultiProcessorCount, scene->device);
-  const bool pool = variant == 1024 && A.sv.nodes4q != nullptr; /* the ray-pool form of the trace kernel */
-  const size_t pool_bytes = pool ? align_up((size_t)sm_count * 8 * 4 * RTB_STACK_SIZE * WF_POOL_RAYS * sizeof(int2), 256) : 0;
+  const bool pool = tune.pool;
+  const size_t pool_bytes = wf_pool_stack_bytes(tune, sm_count);
   const size_t need = arr * 10 + arr_planes + ctr_bytes + (sort_mode ? arr4 * 4 + sort_tmp_bytes : 0) + (split ? arr4 * 2 : 0) + pool_bytes;
   if (scene->wf_bytes < need)
   {
@@ -1098,23 +1162,7 @@ int wf_render(rtb_scene *scene, RenderArgs &A, const rtb_render_desc *desc, floa
         const bool sort_out = sort_mode && b + 1 >= sort_from && b + 1 <= sort_until && b + 1 < n_bounces;
         const unsigned *use_perm = sorted_in ? perm : nullptr;
         mark();
-        if (pool)
-          launch_trace_pool(stats, sm_count, st, A.sv, qi, &cnt[b], &fch[b], A.counters, pool_stacks,
-                            (desc->reserved & 0xFF00) ? std::min(std::max(node_exit, 1), 32) : 32);
-        else
-        switch (variant)
-        {
-        case 2: launch_trace<2>(stats, sm_count, st, A.sv, qi, &cnt[b], &fch[b], A.counters, refill_idle, node_exit, use_perm); break;
-        case 22: launch_trace<22>(stats, sm_count, st, A.sv, qi, &cnt[b], &fch[b], A.counters, refill_idle, node_exit, use_perm); break;
-        case 54: launch_trace<54>(stats, sm_count, st, A.sv, qi, &cnt[b], &fch[b], A.counters, refill_idle, node_exit, use_perm); break;
-        case 86: launch_trace<86>(stats, sm_count, st, A.sv, qi, &cnt[b], &fch[b], A.counters, refill_idle, node_exit, use_perm); break;
-        case 150: launch_trace<150>(stats, sm_count, st, A.sv, qi, &cnt[b], &fch[b], A.counters, refill_idle, node_exit, use_perm); break;
-        case 182: launch_trace<182>(stats, sm_count, st, A.sv, qi, &cnt[b], &fch[b], A.counters, refill_idle, node_exit, use_perm); break;
-        case 214: launch_trace<214>(stats, sm_count, st, A.sv, qi, &cnt[b], &fch[b], A.counters, refill_idle, node_exit, use_perm); break;
-        case 10: launch_trace<10>(stats, sm_count, st, A.sv, qi, &cnt[b], &fch[b], A.counters, refill_idle, node_exit, use_perm); break;
-        case 6: launch_trace<6>(stats, sm_count, st, A.sv, qi, &cnt[b], &fch[b], A.counters, refill_idle, node_exit, use_perm); break;
-        default: launch_trace<0>(stats, sm_count, st, A.sv, qi, &cnt[b], &fch[b], A.counters, refill_idle, node_exit, use_perm); break;
-        }
+        wf_launch_trace(tune, stats, sm_count, st, A.sv, qi, &cnt[b], &fch[b], A.counters, pool_stacks, use_perm);
         mark();
         if (sort_out) /* slots beyond the queue's end keep the largest key and sort to the back */
           RTB_CUDA(cudaMemsetAsync(keys, 0xFF, slots * 4, st));
@@ -1169,6 +1217,156 @@ int wf_render(rtb_scene *scene, RenderArgs &A, const rtb_render_desc *desc, floa
     phase_ms[0] = trace;
     phase_ms[1] = total - trace; /* generate of later waves + shade + sum (the first generate is before ev[0]) */
     phase_ms[2] = (float)(ev.size() / 2);
+  }
+  return RTB_OK;
+}
+
+/* ---- parity probe: the product trace kernel on caller rays -------------------------------------- */
+
+/* queue entry i = ray i with its hit record seeded from the oversized list, exactly as k_wf_generate / k_wf_shade
+ * write it; the big-list exact tests go to totals[2] */
+__global__ void k_wf_fill(const __grid_constant__ SceneView sv, const double *__restrict__ rays, unsigned n, WfQueue q,
+                          unsigned long long *totals)
+{
+  const unsigned i = blockIdx.x * blockDim.x + threadIdx.x;
+  const int lane = threadIdx.x & 31;
+  unsigned exact = 0;
+  if (i < n)
+  {
+    const d3 o = d3_make(rays[6 * (size_t)i + 0], rays[6 * (size_t)i + 1], rays[6 * (size_t)i + 2]);
+    const d3 d = d3_make(rays[6 * (size_t)i + 3], rays[6 * (size_t)i + 4], rays[6 * (size_t)i + 5]);
+    HitRec seed;
+    ray_seed_hit(sv, o, d, seed, exact);
+    q.o_xy[i] = make_double2(o.x, o.y);
+    q.oz_dx[i] = make_double2(o.z, d.x);
+    q.d_yz[i] = make_double2(d.y, d.z);
+    q.path[i] = make_uint4(i, 0u, 0u, 0u);
+    q.hit[i] = pack_hit(seed);
+  }
+  wf_add_counters(totals, lane, 0ull, 0ull, exact, 0ull, 0ull);
+}
+
+/* hit record of queue entry i -> the probe's output arrays (the same read-out as rtb_trace_rays) */
+__global__ void k_wf_read_hits(const __grid_constant__ SceneView sv, WfQueue q, unsigned n, int *__restrict__ ids,
+                               long long *__restrict__ prims, double *__restrict__ ts, double *__restrict__ points,
+                               double *__restrict__ normals, double *__restrict__ uvs)
+{
+  const unsigned i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n)
+    return;
+  const double2 a = q.o_xy[i], b = q.oz_dx[i], c = q.d_yz[i];
+  const d3 o = d3_make(a.x, a.y, b.x), d = d3_make(b.y, c.x, c.y);
+  store_hit_record(sv, o, d, unpack_hit(q.hit[i]), i, ids, prims, ts, points, normals, uvs);
+}
+
+extern "C" int rtb_trace_rays_wf(rtb_scene *scene, const double *rays6, size_t n_rays, int tune,
+                                 const uint32_t *perm_or_null, int32_t *ids, int64_t *prims, double *ts, double *points,
+                                 double *normals, double *uvs, rtb_counters *counters_or_null)
+{
+  if (!scene || (n_rays && (!rays6 || !ids)))
+  {
+    rtb_set_error("rtb_trace_rays_wf: NULL argument");
+    return RTB_EINVAL;
+  }
+  if (n_rays >= (1ull << 31))
+  {
+    rtb_set_error("rtb_trace_rays_wf: n_rays must stay below 2^31");
+    return RTB_EINVAL;
+  }
+  if (perm_or_null)
+  {
+    /* the kernel reads queue entry perm[k]: anything but a permutation would read outside the queue */
+    std::vector<char> seen(n_rays, 0);
+    for (size_t k = 0; k < n_rays; k++)
+    {
+      if (perm_or_null[k] >= n_rays || seen[perm_or_null[k]])
+      {
+        rtb_set_error("rtb_trace_rays_wf: perm is not a permutation of [0, n_rays)");
+        return RTB_EINVAL;
+      }
+      seen[perm_or_null[k]] = 1;
+    }
+  }
+  const SceneView &sv = scene->view;
+  WfTraceTune t;
+  const int tune_rc = wf_trace_tune(sv, tune, t);
+  if (tune_rc != RTB_OK)
+    return tune_rc;
+  RTB_CUDA(cudaSetDevice(scene->device));
+  int sm_count = 148;
+  cudaDeviceGetAttribute(&sm_count, cudaDevAttrMultiProcessorCount, scene->device);
+  const unsigned n = (unsigned)n_rays;
+  const size_t m = n_rays > 0 ? n_rays : 1; /* no zero-byte allocations */
+
+  Dev<double> d_rays, d_ts, d_points, d_normals, d_uvs;
+  Dev<double2> d_oxy, d_ozdx, d_dyz;
+  Dev<uint4> d_path, d_hit;
+  Dev<unsigned> d_ctl, d_perm; /* d_ctl: queue length, fetch cursor */
+  Dev<unsigned long long> d_totals;
+  Dev<int2> d_stacks;
+  Dev<int> d_ids;
+  Dev<long long> d_prims;
+  RTB_CUDA(cudaMalloc(&d_rays.p, sizeof(double) * 6 * m));
+  RTB_CUDA(cudaMalloc(&d_oxy.p, sizeof(double2) * m));
+  RTB_CUDA(cudaMalloc(&d_ozdx.p, sizeof(double2) * m));
+  RTB_CUDA(cudaMalloc(&d_dyz.p, sizeof(double2) * m));
+  RTB_CUDA(cudaMalloc(&d_path.p, sizeof(uint4) * m));
+  RTB_CUDA(cudaMalloc(&d_hit.p, sizeof(uint4) * m));
+  RTB_CUDA(cudaMalloc(&d_ctl.p, sizeof(unsigned) * 2));
+  RTB_CUDA(cudaMalloc(&d_totals.p, sizeof(unsigned long long) * 5));
+  if (perm_or_null)
+    RTB_CUDA(cudaMalloc(&d_perm.p, sizeof(unsigned) * m));
+  if (t.pool)
+    RTB_CUDA(cudaMalloc(&d_stacks.p, wf_pool_stack_bytes(t, sm_count)));
+  RTB_CUDA(cudaMalloc(&d_ids.p, sizeof(int) * m));
+  RTB_CUDA(cudaMalloc(&d_prims.p, sizeof(long long) * m));
+  RTB_CUDA(cudaMalloc(&d_ts.p, sizeof(double) * m));
+  RTB_CUDA(cudaMalloc(&d_points.p, sizeof(double) * 3 * m));
+  RTB_CUDA(cudaMalloc(&d_normals.p, sizeof(double) * 3 * m));
+  RTB_CUDA(cudaMalloc(&d_uvs.p, sizeof(double) * 2 * m));
+  if (n_rays)
+    RTB_CUDA(cudaMemcpy(d_rays.p, rays6, sizeof(double) * 6 * n_rays, cudaMemcpyHostToDevice));
+  if (perm_or_null && n_rays)
+    RTB_CUDA(cudaMemcpy(d_perm.p, perm_or_null, sizeof(unsigned) * n_rays, cudaMemcpyHostToDevice));
+  const unsigned ctl[2] = { n, 0u };
+  RTB_CUDA(cudaMemcpy(d_ctl.p, ctl, sizeof(ctl), cudaMemcpyHostToDevice));
+  RTB_CUDA(cudaMemset(d_totals.p, 0, sizeof(unsigned long long) * 5));
+
+  WfQueue q;
+  q.o_xy = d_oxy.p;
+  q.oz_dx = d_ozdx.p;
+  q.d_yz = d_dyz.p;
+  q.path = d_path.p;
+  q.hit = d_hit.p;
+  q.branch = nullptr;
+  q.cap = n;
+  const unsigned blocks = (unsigned)((m + 127) / 128);
+  k_wf_fill<<<blocks, 128>>>(sv, d_rays.p, n, q, d_totals.p);
+  RTB_CUDA(cudaGetLastError());
+  wf_launch_trace(t, true, sm_count, 0, sv, q, d_ctl.p, d_ctl.p + 1, d_totals.p, d_stacks.p, d_perm.p);
+  RTB_CUDA(cudaGetLastError());
+  k_wf_read_hits<<<blocks, 128>>>(sv, q, n, d_ids.p, d_prims.p, d_ts.p, d_points.p, d_normals.p, d_uvs.p);
+  RTB_CUDA(cudaGetLastError());
+  RTB_CUDA(cudaDeviceSynchronize());
+  if (n_rays)
+  {
+    RTB_CUDA(cudaMemcpy(ids, d_ids.p, sizeof(int) * n_rays, cudaMemcpyDeviceToHost));
+    if (prims) RTB_CUDA(cudaMemcpy(prims, d_prims.p, sizeof(long long) * n_rays, cudaMemcpyDeviceToHost));
+    if (ts) RTB_CUDA(cudaMemcpy(ts, d_ts.p, sizeof(double) * n_rays, cudaMemcpyDeviceToHost));
+    if (points) RTB_CUDA(cudaMemcpy(points, d_points.p, sizeof(double) * 3 * n_rays, cudaMemcpyDeviceToHost));
+    if (normals) RTB_CUDA(cudaMemcpy(normals, d_normals.p, sizeof(double) * 3 * n_rays, cudaMemcpyDeviceToHost));
+    if (uvs) RTB_CUDA(cudaMemcpy(uvs, d_uvs.p, sizeof(double) * 2 * n_rays, cudaMemcpyDeviceToHost));
+  }
+  if (counters_or_null)
+  {
+    unsigned long long h[5];
+    RTB_CUDA(cudaMemcpy(h, d_totals.p, sizeof(h), cudaMemcpyDeviceToHost));
+    memset(counters_or_null, 0, sizeof(*counters_or_null));
+    counters_or_null->rays = n_rays;
+    counters_or_null->prim_tests = h[2];
+    counters_or_null->node_visits = h[3];
+    counters_or_null->launches = 3;
+    counters_or_null->trace_launches = 1;
   }
   return RTB_OK;
 }
