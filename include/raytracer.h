@@ -219,6 +219,25 @@ void render_scene(uint8_t *framebuffer, SceneObject *objects, size_t n_objects, 
 void render_ex(uint8_t *framebuffer, Object *objects, size_t n_objects, Camera *camera,
                Options *options, const RenderParams *params);
 
+/* First-hit feature buffers of a render (rtb_render_aov in rtb200.h), the inputs a denoiser (OIDN, OptiX) or a
+ * compositor wants next to the frame.  HOST arrays of H*W pixels, row 0 = top; any may be NULL:
+ *   albedo  float[H*W*3]  mean over the samples of the first hit's colour (times the checker factor), 0 on a miss
+ *   normal  float[H*W*3]  mean of the first hit's outward surface normal, 0 on a miss
+ *   depth   float[H*W]    mean distance to the first hit over the samples that hit, 0 where none did
+ *   object  int32[H*W]    object index hit by the first sample (params->sample_offset), -1 on a miss
+ * The frame itself is rendered exactly as without them.  Single GPU only (num_gpus == 1). */
+typedef struct
+{
+  float *albedo, *normal, *depth;
+  int32_t *object;
+} RenderAov;
+
+/* render_ex / render_scene that also fill `aov` (NULL = render_ex / render_scene) */
+void render_ex_aov(uint8_t *framebuffer, Object *objects, size_t n_objects, Camera *camera, Options *options,
+                   const RenderParams *params, const RenderAov *aov);
+void render_scene_aov(uint8_t *framebuffer, SceneObject *objects, size_t n_objects, Camera *camera, Options *options,
+                      const RenderParams *params, const RenderAov *aov);
+
 /* Optional: starts creating the CUDA context(s) a later render*() with these parameters will use (NULL = defaults)
  * on a background thread and returns at once.  A driver calls it first and then reads its scene -- the reference's
  * main.c:413-429 builds the scene between allocating the frame and calling render() -- so that driver start-up

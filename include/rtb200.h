@@ -14,6 +14,8 @@
  *                          trace_path (raytracer.c:482-554), RNG (raytracer.c:227)
  *   rtb_tonemap            mean, gamma 5.0, 8-bit truncation (raytracer.c:215-220)
  *   rtb_render             the whole of render() (raytracer.c:176-223), host buffers in/out
+ *   rtb_render_aov         no reference counterpart: first-hit feature buffers (albedo, normal, depth, hit count,
+ *                          object id) of the render's own camera samples, the inputs of a denoiser or a compositor
  *   rtb_trace_rays         intersect() for arbitrary rays (raytracer.c:393-464): parity probe
  *   rtb_trace_rays_wf      the same records from the wavefront renderer's trace kernel: parity probe
  *   rtb_path_records       per-path vertex records: parity probe for the 1-bounce check
@@ -162,6 +164,25 @@ int rtb_render(rtb_scene *scene, const double *camera12, const rtb_render_desc *
  * (sample_begin/end = its share) passes the job's total sample count */
 int rtb_render_mean(rtb_scene *scene, const double *camera12, const rtb_render_desc *desc, int total_samples,
                     uint8_t *framebuffer, float *accum_or_null, rtb_counters *counters);
+
+/* first-hit feature buffers of the call's primary rays (the render's own camera samples): SUMS over
+ * [sample_begin, sample_end); any output may be NULL, not all; desc->kernel/dielectric_mode/max_depth unused,
+ * desc->integrator selects the checker's M.  Asynchronous on `stream` unless `counters` is non-NULL.
+ * Per sample, in double, on a hit (0 on a miss): d_albedo3 += the object's colour, times the checker factor 0.3 or 0.7
+ * for an M_CHECKERED object at the integrator's M (100000 trace_path, raytracer.c:508; 10 cast_ray, :584); d_normal3
+ * += the outward surface normal (cross(v2-v0, v1-v0) normalised on triangles, raytracer.c:44; not flipped towards the
+ * camera); d_depth += t; d_hits += 1.  d_object: the object index hit by the first sample, -1 on a miss.
+ * Summation: samples in double per plane (desc->planes, else automatic), rounded to float once, planes summed in
+ * float in plane order, as the megakernel and Whitted renders sum; hits are an exact count.  Every buffer is
+ * [height*width] (times 3 for albedo and normal) of the scene's device; counters: rays = paths = primary rays, prim_tests,
+ * node_visits, launches, gpu_ms. */
+int rtb_render_aov(rtb_scene *scene, const double *camera12, const rtb_render_desc *desc,
+                   float *d_albedo3, float *d_normal3, float *d_depth, uint32_t *d_hits, int32_t *d_object,
+                   void *stream, rtb_counters *counters);
+/* the same with HOST buffers (blocking) */
+int rtb_render_aov_host(rtb_scene *scene, const double *camera12, const rtb_render_desc *desc,
+                        float *albedo3, float *normal3, float *depth, uint32_t *hits, int32_t *object,
+                        rtb_counters *counters);
 
 /* parity probes (host buffers) */
 int rtb_trace_rays(rtb_scene *scene, const double *rays6, size_t n_rays, int use_bvh, int32_t *ids,

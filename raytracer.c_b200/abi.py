@@ -82,6 +82,12 @@ class RenderParams(C.Structure):
                 ("accum_out", C.POINTER(C.c_float)), ("integrator", C.c_int), ("num_gpus", C.c_int)]
 
 
+class RenderAov(C.Structure):
+    """HOST feature buffers of render_ex_aov / render_scene_aov (raytracer.h); any may be NULL"""
+    _fields_ = [("albedo", C.POINTER(C.c_float)), ("normal", C.POINTER(C.c_float)), ("depth", C.POINTER(C.c_float)),
+                ("object", C.POINTER(C.c_int32))]
+
+
 class SceneMix(C.Structure):
     _fields_ = [("emissive", C.c_double), ("refraction", C.c_double), ("reflection", C.c_double)]
 

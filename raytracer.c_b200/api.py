@@ -25,6 +25,7 @@ RTB_SYMBOLS = [
     "rtb_trace_rays", "rtb_trace_rays_wf", "rtb_path_records", "rtb_philox4x32_10", "rtb_probe_l2_bandwidth", "rtb_cast_rays",
     "rtb_probe_fp32_tflops", "rtb_render_mean", "rtb_comm_unique_id", "rtb_comm_create_rank", "rtb_comm_create_local", "rtb_comm_size",
     "rtb_warm_up", "rtb_comm_local_ranks", "rtb_comm_destroy", "rtb_comm_shard_samples", "rtb_comm_scene_create", "rtb_comm_render", "rtb_render_multi",
+    "rtb_render_aov", "rtb_render_aov_host",
 ]
 # the reference's exported surface (raytracer.h:135-164) plus the documented extensions
 HOST_SYMBOLS = [
@@ -34,6 +35,7 @@ HOST_SYMBOLS = [
     "render_params_default", "render_scene", "render_ex", "free_mesh", "apply_matrix", "load_obj_ex", "render_warm_up",
     "scene_default", "scene_room_walls", "scene_random_spheres", "scene_sphere_field",
     "scene_heightfield_mesh", "scene_write_obj", "scene_mesh_room", "scene_from_objects", "rt_write_png",
+    "render_ex_aov", "render_scene_aov", "rt_write_pfm",
 ]
 
 
@@ -98,6 +100,10 @@ def _bind(cu, host):
                                    C.POINTER(abi.RtbCounters)]
     cu.rtb_render_multi.argtypes = [C.c_void_p, C.c_void_p, C.c_size_t, C.c_int, dp, C.POINTER(abi.RtbRenderDesc),
                                     C.c_void_p, C.c_void_p, C.POINTER(abi.RtbCounters)]
+    cu.rtb_render_aov.argtypes = [C.c_void_p, dp, C.POINTER(abi.RtbRenderDesc)] + [C.c_void_p] * 6 + [
+        C.POINTER(abi.RtbCounters)]
+    cu.rtb_render_aov_host.argtypes = [C.c_void_p, dp, C.POINTER(abi.RtbRenderDesc)] + [C.c_void_p] * 5 + [
+        C.POINTER(abi.RtbCounters)]
 
     host.init_camera.argtypes = [C.POINTER(abi.Camera), abi.Vec3, abi.Vec3, C.POINTER(abi.Options)]
     host.init_camera.restype = None
@@ -107,6 +113,10 @@ def _bind(cu, host):
     host.render_ex.restype = None
     host.render_scene.argtypes = host.render_ex.argtypes
     host.render_scene.restype = None
+    host.render_ex_aov.argtypes = host.render_ex.argtypes + [C.POINTER(abi.RenderAov)]
+    host.render_ex_aov.restype = None
+    host.render_scene_aov.argtypes = host.render_ex_aov.argtypes
+    host.render_scene_aov.restype = None
     host.render_params_default.argtypes = [C.POINTER(abi.RenderParams)]
     host.render_params_default.restype = None
     host.load_obj.argtypes = [C.c_char_p, C.POINTER(abi.TriangleMesh)]
@@ -133,6 +143,8 @@ def _bind(cu, host):
     host.scene_write_obj.restype = C.c_bool
     host.rt_write_png.argtypes = [C.c_char_p, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_int]
     host.rt_write_png.restype = C.c_int
+    host.rt_write_pfm.argtypes = [C.c_char_p, C.c_int, C.c_int, C.c_int, C.c_void_p]
+    host.rt_write_pfm.restype = C.c_int
 
 
 def _check(rc, what):
@@ -249,6 +261,26 @@ def write_obj(path, verts):
         raise RtbError(f"scene_write_obj({path!r}) failed")
 
 
+def render_scene_aov(holder, camera, width, height, samples, params=None):
+    """render_scene_aov (raytracer.h): the frame of render_scene with these parameters, and the MEANS of its first-hit
+    feature buffers -> (framebuffer u8 [H, W, 3], dict(albedo [H, W, 3] f32, normal, depth [H, W] f32,
+    object [H, W] i32)).  `holder` is an abi.SceneHolder, `params` an abi.RenderParams (None = defaults)."""
+    _, host = load()
+    if params is None:
+        params = abi.RenderParams()
+        host.render_params_default(C.byref(params))
+    fb = np.zeros((height, width, 3), dtype=np.uint8)
+    out = dict(albedo=np.zeros((height, width, 3), np.float32), normal=np.zeros((height, width, 3), np.float32),
+               depth=np.zeros((height, width), np.float32), object=np.zeros((height, width), np.int32))
+    aov = abi.RenderAov(*(out[k].ctypes.data_as(C.POINTER(C.c_float)) for k in ("albedo", "normal", "depth")),
+                        out["object"].ctypes.data_as(C.POINTER(C.c_int32)))
+    opt = abi.Options()
+    opt.width, opt.height, opt.samples = width, height, samples
+    host.render_scene_aov(fb.ctypes.data, C.addressof(holder.objects), holder.n, C.byref(camera), C.byref(opt),
+                          C.byref(params), C.byref(aov))
+    return fb, out
+
+
 def render(objects, camera, width, height, samples):
     """The drop-in call: the reference's render() signature (raytracer.h:156)."""
     _, host = load()
@@ -332,6 +364,33 @@ class Scene:
                                          C.c_void_p(d_accum_ptr), C.c_void_p(stream or 0),
                                          C.byref(ctr) if ctr is not None else None), "rtb_render_accum")
         return ctr
+
+    def render_aov_accum(self, camera, desc, d_albedo, d_normal, d_depth, d_hits, d_object, stream=None,
+                         want_counters=False):
+        """first-hit feature buffers of the call's camera samples as device SUMS (rtb_render_aov): float[H*W*3]
+        albedo and normal, float[H*W] depth, uint32[H*W] hits, int32[H*W] object id of the first sample; pointers,
+        any may be 0 (not all).  Asynchronous on `stream` unless counters are wanted."""
+        cam = camera.as_array()
+        ctr = abi.RtbCounters() if want_counters else None
+        _check(self._cu.rtb_render_aov(self._h, cam.ctypes.data_as(C.POINTER(C.c_double)), C.byref(desc),
+                                       *(C.c_void_p(p or 0) for p in (d_albedo, d_normal, d_depth, d_hits, d_object)),
+                                       C.c_void_p(stream or 0), C.byref(ctr) if ctr is not None else None),
+               "rtb_render_aov")
+        return ctr
+
+    def render_aov(self, camera, desc, want_counters=False):
+        """the same sums in host arrays (rtb_render_aov_host) -> dict(albedo [H, W, 3] f32, normal [H, W, 3] f32,
+        depth [H, W] f32, hits [H, W] u32, object [H, W] i32), plus abi.RtbCounters when want_counters"""
+        cam = camera.as_array()
+        h, w = desc.height, desc.width
+        out = dict(albedo=np.zeros((h, w, 3), np.float32), normal=np.zeros((h, w, 3), np.float32),
+                   depth=np.zeros((h, w), np.float32), hits=np.zeros((h, w), np.uint32),
+                   object=np.zeros((h, w), np.int32))
+        ctr = abi.RtbCounters() if want_counters else None
+        _check(self._cu.rtb_render_aov_host(self._h, cam.ctypes.data_as(C.POINTER(C.c_double)), C.byref(desc),
+                                            *(out[k].ctypes.data for k in ("albedo", "normal", "depth", "hits", "object")),
+                                            C.byref(ctr) if ctr is not None else None), "rtb_render_aov_host")
+        return (out, ctr) if want_counters else out
 
     def render(self, camera, desc, want_accum=False):
         """host u8 framebuffer (+ host float sums) through rtb_render"""

@@ -885,4 +885,33 @@ __device__ __forceinline__ float checker_factor(double u, double v, double M)
   return (float)__dadd_rn(__dmul_rn(0.3, __dsub_rn(1.0, on)), __dmul_rn(0.7, on));
 }
 
+/* raytracer.c:386-391 on a colour, all in double: the Whitted integrator's checker (rtb_whitted.cu) and the albedo
+ * of the first-hit feature buffers (rtb_aov.cu) */
+__device__ __forceinline__ d3 checker_color(const d3 &color, double u, double v, double M)
+{
+  bool a = fmod(__dmul_rn(u, M), 1.0) > 0.5;
+  bool b = fmod(__dmul_rn(v, M), 1.0) < 0.5;
+  double on = (a ^ b) ? 1.0 : 0.0;
+  double c = __dadd_rn(__dmul_rn(0.3, __dsub_rn(1.0, on)), __dmul_rn(0.7, on));
+  return d3_scale(color, c);
+}
+
+/* exact nearest hit of one ray on the product path's tree: the compressed BVH4, or the BVH2 when the scene has none (a
+ * tree too deep for the BVH4 stack); true on a hit.  STATS: counts into `ts` */
+template <bool STATS = false>
+__device__ __forceinline__ bool nearest_hit(const SceneView &sv, const d3 &o, const d3 &d, HitRec &best, TraceStats &ts)
+{
+  if (sv.nodes4q != nullptr)
+    closest_hit_ww<STATS, 0, 2>(sv, o, d, best, ts, nullptr, 0);
+  else
+    closest_hit_ww<STATS, 0>(sv, o, d, best, ts, nullptr, 0);
+  return best.t < 1e300;
+}
+
+__device__ __forceinline__ bool nearest_hit(const SceneView &sv, const d3 &o, const d3 &d, HitRec &best)
+{
+  TraceStats ts = { 0u, 0u };
+  return nearest_hit<false>(sv, o, d, best, ts);
+}
+
 #endif /* RTB_DEVICE_CUH */

@@ -151,6 +151,18 @@ int rtb_shard_allgather_bytes(const rtb_scene_shard *shard, void *base, size_t c
 int rtb_scene_create_sharded(const void *objects, size_t n_objects, int kind, int device, unsigned flags,
                              const rtb_scene_shard *shard, rtb_scene **out);
 
+/* ---- shared by the render entry points (rtb_render.cu) ---------------------------------------------- */
+int rtb_check_desc(const rtb_render_desc *d); /* RTB_OK or RTB_EINVAL with the error text set */
+/* threads the megakernels and the one-thread-per-(plane, pixel) kernels aim for: fill 148 SMs a few times over even
+ * for small frames */
+#define RTB_MEGAKERNEL_THREADS (148ll * 2048 * 2)
+/* Planes: `spp` samples cut into contiguous sub-ranges of *chunk samples that are accumulated separately and summed in
+ * order, which fixes the floating-point summation order.  `planes` > 0 pins the count (at most 1024), else enough
+ * planes for about `want_threads` threads over `n_px` pixels (at most 64).  Returns the plane count. */
+int rtb_plane_split(long long want_threads, size_t n_px, int planes, int spp, int *chunk);
+/* out[i] = sum over k < splits of planes[k * n + i], in float, in plane order (k_sum_planes), on `stream` */
+int rtb_sum_planes(const float *planes, int splits, size_t n, float *out, cudaStream_t stream);
+
 /* a plain cudaMalloc'd buffer of the probes, freed on every return path */
 template <typename T>
 struct Dev

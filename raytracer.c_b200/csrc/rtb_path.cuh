@@ -199,6 +199,9 @@ __device__ __forceinline__ void path_shade(const RenderArgs &A, PathState &st, c
   }
 }
 
+/* rtb_render.cu: the camera, frame, sample range, key and scene of a call (chunk, splits and out are the caller's) */
+void fill_args(RenderArgs &A, const rtb_scene *scene, const double *camera12, const rtb_render_desc *desc);
+
 /* rtb_wavefront.cu: render [A.s_begin, A.s_end) with the wavefront kernels into d_accum
  * (A.splits planes of A.chunk samples each must be set) */
 int wf_render(rtb_scene *scene, RenderArgs &A, const rtb_render_desc *desc, float *d_accum, cudaStream_t stream,

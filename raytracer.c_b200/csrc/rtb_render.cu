@@ -470,6 +470,13 @@ __global__ void k_sum_planes(const float *__restrict__ planes, int splits, size_
   out[i] = acc;
 }
 
+int rtb_sum_planes(const float *planes, int splits, size_t n, float *out, cudaStream_t stream)
+{
+  k_sum_planes<<<(int)((n + 255) / 256), 256, 0, stream>>>(planes, splits, n, out);
+  RTB_CUDA(cudaGetLastError());
+  return RTB_OK;
+}
+
 /* raytracer.c:215-220: mean, pow(c, 1/5.0), clamp, truncate.  NaN -> 255 (CLAMP macro). */
 __global__ void k_tonemap(const float *__restrict__ accum, size_t n, double inv_samples, uint8_t *__restrict__ fb)
 {
@@ -577,7 +584,7 @@ __global__ void k_philox(const uint4 *__restrict__ ctr, const uint2 *__restrict_
 
 /* ---- host entry points ---------------------------------------------------------------- */
 
-static int check_desc(const rtb_render_desc *d)
+int rtb_check_desc(const rtb_render_desc *d)
 {
   if (!d || d->width < 2 || d->height < 2 || d->sample_end < d->sample_begin || d->max_depth < 0 ||
       d->max_depth > 255 || (long long)d->width * d->height >= (1ll << 30))
@@ -611,7 +618,7 @@ static int check_desc(const rtb_render_desc *d)
   return RTB_OK;
 }
 
-static void fill_args(RenderArgs &A, const rtb_scene *scene, const double *camera12, const rtb_render_desc *desc)
+void fill_args(RenderArgs &A, const rtb_scene *scene, const double *camera12, const rtb_render_desc *desc)
 {
   A.sv = scene->view;
   for (int k = 0; k < 3; k++)
@@ -635,6 +642,18 @@ static void fill_args(RenderArgs &A, const rtb_scene *scene, const double *camer
   A.counters = scene->d_counters;
 }
 
+int rtb_plane_split(long long want_threads, size_t n_px, int planes, int spp, int *chunk)
+{
+  int splits = (int)std::min<long long>(std::max<long long>(1, (want_threads + (long long)n_px - 1) / (long long)n_px), 64);
+  if (planes > 0)
+    splits = std::min(planes, 1024);
+  splits = std::max(1, std::min(splits, spp));
+  *chunk = spp > 0 ? (spp + splits - 1) / splits : 0;
+  if (*chunk > 0)
+    splits = (spp + *chunk - 1) / *chunk;
+  return splits;
+}
+
 namespace
 {
 struct EventPair /* two CUDA events, destroyed on every return path */
@@ -656,7 +675,7 @@ extern "C" int rtb_render_accum(rtb_scene *scene, const double *camera12, const 
     rtb_set_error("rtb_render_accum: NULL argument");
     return RTB_EINVAL;
   }
-  int rc = check_desc(desc);
+  int rc = rtb_check_desc(desc);
   if (rc != RTB_OK)
     return rc;
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
@@ -682,7 +701,7 @@ extern "C" int rtb_render_accum(rtb_scene *scene, const double *camera12, const 
     rtb_set_error("rtb_render_desc.kernel 1..5 walk the BVH2: create the scene with RTB_SCENE_ALL_TREES");
     return RTB_EINVAL;
   }
-  long long want_threads = 148ll * 2048 * 2;
+  long long want_threads = RTB_MEGAKERNEL_THREADS;
   if (wavefront)
   {
     /* the free memory is read once per device (cudaMemGetInfo costs milliseconds, render() makes a
@@ -708,13 +727,8 @@ extern "C" int rtb_render_accum(rtb_scene *scene, const double *camera12, const 
       want_threads >>= std::min(desc->max_depth + 1, 6);
     want_threads = std::max<long long>(want_threads, (long long)n_px);
   }
-  int splits = (int)std::min<long long>(std::max<long long>(1, (want_threads + (long long)n_px - 1) / (long long)n_px), 64);
-  if (desc->planes > 0)
-    splits = std::min(desc->planes, 1024);
-  splits = std::max(1, std::min(splits, spp));
-  int chunk = spp > 0 ? (spp + splits - 1) / splits : 0;
-  if (chunk > 0)
-    splits = (spp + chunk - 1) / chunk;
+  int chunk = 0;
+  const int splits = rtb_plane_split(want_threads, n_px, desc->planes, spp, &chunk);
   A.chunk = chunk;
   A.splits = splits;
 
@@ -812,9 +826,9 @@ extern "C" int rtb_render_accum(rtb_scene *scene, const double *camera12, const 
     launches++;
     if (splits > 1)
     {
-      size_t n = 3 * n_px;
-      k_sum_planes<<<(int)((n + 255) / 256), 256, 0, stream>>>(scene->d_scratch, splits, n, d_accum);
-      RTB_CUDA(cudaGetLastError());
+      rc = rtb_sum_planes(scene->d_scratch, splits, 3 * n_px, d_accum, stream);
+      if (rc != RTB_OK)
+        return rc;
       launches++;
     }
     }
@@ -872,7 +886,7 @@ extern "C" int rtb_render_mean(rtb_scene *scene, const double *camera12, const r
     rtb_set_error("rtb_render: NULL argument or total_samples <= 0");
     return RTB_EINVAL;
   }
-  int rc = check_desc(desc);
+  int rc = rtb_check_desc(desc);
   if (rc != RTB_OK)
     return rc;
   RTB_CUDA(cudaSetDevice(scene->device));
@@ -958,7 +972,7 @@ extern "C" int rtb_path_records(rtb_scene *scene, const double *camera12, const 
     rtb_set_error("rtb_path_records: bad argument");
     return RTB_EINVAL;
   }
-  int rc = check_desc(desc);
+  int rc = rtb_check_desc(desc);
   if (rc != RTB_OK)
     return rc;
   RTB_CUDA(cudaSetDevice(scene->device));

@@ -34,26 +34,6 @@ struct WhFrame
   int stage; /* 0: before the reflection child, 1: before the refraction child, 2: refraction child running */
 };
 
-__device__ __forceinline__ bool wh_nearest(const SceneView &sv, const d3 &o, const d3 &d, HitRec &best)
-{
-  TraceStats ts = { 0u, 0u };
-  if (sv.nodes4q != nullptr)
-    closest_hit_ww<false, 0, 2>(sv, o, d, best, ts, nullptr, 0);
-  else
-    closest_hit_ww<false, 0>(sv, o, d, best, ts, nullptr, 0); /* tree too deep for the BVH4 stack */
-  return best.t < 1e300;
-}
-
-/* raytracer.c:386-391 on a colour */
-__device__ __forceinline__ d3 wh_checker(const d3 &color, double u, double v, double M)
-{
-  bool a = fmod(__dmul_rn(u, M), 1.0) > 0.5;
-  bool b = fmod(__dmul_rn(v, M), 1.0) < 0.5;
-  double on = (a ^ b) ? 1.0 : 0.0;
-  double c = __dadd_rn(__dmul_rn(0.3, __dsub_rn(1.0, on)), __dmul_rn(0.7, on));
-  return d3_scale(color, c);
-}
-
 __device__ __forceinline__ d3 d3_mul(const d3 &a, const d3 &b)
 {
   return d3_make(__dmul_rn(a.x, b.x), __dmul_rn(a.y, b.y), __dmul_rn(a.z, b.z));
@@ -79,7 +59,7 @@ __device__ d3 whitted_cast(const SceneView &sv, const d3 &o0, const d3 &d0, int 
       /* ---- cast_ray(&{o, d}, ..., depth = sp) up to the recursive calls ---- */
       rays++;
       HitRec best;
-      if (sp > max_depth || !wh_nearest(sv, o, d, best))
+      if (sp > max_depth || !nearest_hit(sv, o, d, best))
       {
         ret = BACKGROUND;
         phase = PH_RETURN;
@@ -97,12 +77,12 @@ __device__ d3 whitted_cast(const SceneView &sv, const d3 &o0, const d3 &d0, int 
       const d3 light_color = d3_make(1, 1, 1);
       const d3 light_dir = d3_normalize(d3_sub(light_pos, s.point));
       HitRec shadow;
-      const bool in_shadow = wh_nearest(sv, s.point, light_dir, shadow);
+      const bool in_shadow = nearest_hit(sv, s.point, light_dir, shadow);
 
       d3 object_color = d3_make(sv.colors[3 * slot_obj + 0], sv.colors[3 * slot_obj + 1], sv.colors[3 * slot_obj + 2]);
       const double ka = 0.25, kd = 0.5, ks = 0.8, alpha = 10.0;
       if (flags & RT_M_CHECKERED)
-        object_color = wh_checker(object_color, s.u, s.v, 10);
+        object_color = checker_color(object_color, s.u, s.v, 10);
 
       const d3 ambient = d3_scale(light_color, ka);
       const double ndl = d3_dot(s.normal, light_dir);

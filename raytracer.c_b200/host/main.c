@@ -14,6 +14,9 @@
  *   -D stochastic|split      dielectric estimator: one child per vertex (default) or the reference's two-way split
  *   -m <sx,sy,sz,ry,tx,ty,tz> with obj:FILE -- place the mesh like the reference's driver would: scale, rotation about
  *                            y (degrees), translation, composed into a mat4 and applied with apply_matrix (main.c:140-147)
+ *   -a <prefix>              also write the first-hit feature buffers of the frame (render_ex_aov): <prefix>_albedo.pfm,
+ *                            <prefix>_normal.pfm (RGB) and <prefix>_depth.pfm (grey), what oidnDenoise --alb --nrm reads;
+ *                            single GPU only
  * Deliberately NOT reproduced: the option parser's mis-parse of values whose second
  * character is h/w/s/o (SURVEY.md section 5) and the SIGINT handler's double free.
  */
@@ -24,13 +27,14 @@
 #include "scenes.h"
 
 int rt_write_png(const char *filename, int w, int h, int comp, const void *data, int stride_in_bytes);
+int rt_write_pfm(const char *filename, int w, int h, int comp, const float *data);
 
 typedef struct
 {
   Options options;
   int max_depth, device, integrator, gpus, dielectric;
   uint64_t seed;
-  const char *scene, *placement;
+  const char *scene, *placement, *aov_prefix;
 } Cli;
 
 static void usage(const char *prog)
@@ -38,6 +42,7 @@ static void usage(const char *prog)
   fprintf(stderr, "Usage: %s -w <width> -h <height> -s <samples per pixel> -o <filename>\n", prog);
   fprintf(stderr, "       [-d <max depth>] [-S <seed>] [-g <cuda device>] [-c default|spheres:N|mesh:GRID|obj:FILE]\n");
   fprintf(stderr, "       [-i path|whitted] [-G <gpus>] [-D stochastic|split] [-m sx,sy,sz,ry_deg,tx,ty,tz]\n");
+  fprintf(stderr, "       [-a <prefix>: also write <prefix>_albedo.pfm, <prefix>_normal.pfm, <prefix>_depth.pfm]\n");
 }
 
 static bool parse_cli(int argc, char **argv, Cli *cli)
@@ -70,12 +75,33 @@ static bool parse_cli(int argc, char **argv, Cli *cli)
     case 'G': cli->gpus = atoi(val); break;
     case 'D': cli->dielectric = (strcmp(val, "split") == 0) ? RT_DIELECTRIC_SPLIT : RT_DIELECTRIC_STOCHASTIC; break;
     case 'm': cli->placement = val; break;
+    case 'a': cli->aov_prefix = val; break;
     default:
       fprintf(stderr, "unknown option '%s'\n", a);
       return false;
     }
   }
+  if (cli->aov_prefix && cli->gpus > 1)
+  {
+    fprintf(stderr, "-a (feature buffers) renders on one GPU: it cannot be combined with -G %d\n", cli->gpus);
+    return false;
+  }
   return cli->options.width >= 2 && cli->options.height >= 2 && cli->options.samples >= 1;
+}
+
+/* <prefix><suffix>.pfm */
+static bool write_pfm(const char *prefix, const char *suffix, int w, int h, int comp, const float *data)
+{
+  char *name = (char *)malloc(strlen(prefix) + strlen(suffix) + 5);
+  if (!name)
+    return false;
+  sprintf(name, "%s%s.pfm", prefix, suffix);
+  printf("writing %s...\n", name);
+  bool ok = rt_write_pfm(name, w, h, comp, data) != 0;
+  if (!ok)
+    fprintf(stderr, "could not write '%s'\n", name);
+  free(name);
+  return ok;
 }
 
 int main(int argc, char **argv)
@@ -120,6 +146,22 @@ int main(int argc, char **argv)
   if (cli.gpus > 0)
     rp.num_gpus = cli.gpus;
 
+  RenderAov aov_bufs = { NULL, NULL, NULL, NULL };
+  const RenderAov *aov = NULL;
+  if (cli.aov_prefix)
+  {
+    const size_t n_px = (size_t)opt->width * opt->height;
+    aov_bufs.albedo = (float *)calloc(3 * n_px, sizeof(float));
+    aov_bufs.normal = (float *)calloc(3 * n_px, sizeof(float));
+    aov_bufs.depth = (float *)calloc(n_px, sizeof(float));
+    if (!aov_bufs.albedo || !aov_bufs.normal || !aov_bufs.depth)
+    {
+      fprintf(stderr, "could not allocate the feature buffers\n");
+      return EXIT_FAILURE;
+    }
+    aov = &aov_bufs;
+  }
+
   struct timespec t0, t1;
   clock_gettime(CLOCK_MONOTONIC, &t0);
   /* the CUDA context comes up on a second thread while the scene is generated or read from disk */
@@ -134,14 +176,14 @@ int main(int argc, char **argv)
   {
     Object scene[SCENE_DEFAULT_COUNT];
     size_t n = scene_default(scene, opt->width, opt->height);
-    render_ex(framebuffer, scene, n, &camera, opt, &rp);
+    render_ex_aov(framebuffer, scene, n, &camera, opt, &rp, aov);
   }
   else if (strncmp(cli.scene, "spheres:", 8) == 0)
   {
     Object *scene = NULL;
     SceneMix mix = { 0.5, 0.2, 0.2 }; /* main.c:104-119 */
     size_t n = scene_sphere_field(&scene, (size_t)atol(cli.scene + 8), opt->width, opt->height, mix, cli.seed);
-    render_ex(framebuffer, scene, n, &camera, opt, &rp);
+    render_ex_aov(framebuffer, scene, n, &camera, opt, &rp, aov);
     free(scene);
   }
   else if (strncmp(cli.scene, "mesh:", 5) == 0 || strncmp(cli.scene, "obj:", 4) == 0)
@@ -171,7 +213,7 @@ int main(int argc, char **argv)
     SceneObject *scene = NULL;
     Sphere *spheres = NULL;
     size_t n = scene_mesh_room(&scene, &spheres, &mesh, opt->width, opt->height);
-    render_scene(framebuffer, scene, n, &camera, opt, &rp);
+    render_scene_aov(framebuffer, scene, n, &camera, opt, &rp, aov);
     CLI_MARK("render_scene (first call: CUDA context + upload + BVH + render + read-back)");
     free(scene);
     free(spheres);
@@ -198,7 +240,14 @@ int main(int argc, char **argv)
     return EXIT_FAILURE;
   }
   CLI_MARK("write PNG");
+  if (aov && !(write_pfm(cli.aov_prefix, "_albedo", opt->width, opt->height, 3, aov->albedo) &&
+               write_pfm(cli.aov_prefix, "_normal", opt->width, opt->height, 3, aov->normal) &&
+               write_pfm(cli.aov_prefix, "_depth", opt->width, opt->height, 1, aov->depth)))
+    return EXIT_FAILURE;
   printf("done.\n");
   free(framebuffer);
+  free(aov_bufs.albedo);
+  free(aov_bufs.normal);
+  free(aov_bufs.depth);
   return EXIT_SUCCESS;
 }

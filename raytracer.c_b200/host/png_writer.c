@@ -6,6 +6,9 @@
  * copied.  rt_write_png() has the same argument meaning and return convention (0 on
  * failure) and writes a valid, uncompressed PNG: zlib "stored" blocks, filter type 0.
  * Any consumer of the reference's output (an image viewer, PIL) reads it the same way.
+ *
+ * rt_write_pfm() writes float images (the feature buffers of render_ex_aov / render_scene_aov) as Portable FloatMap,
+ * the format denoisers read (oidnDenoise --alb --nrm).
  */
 #include <stdint.h>
 #include <stdio.h>
@@ -163,5 +166,36 @@ int rt_write_png(const char *filename, int w, int h, int comp, const void *data,
   }
   free(raw);
   free(z);
+  return ok;
+}
+
+/* Portable FloatMap: "PF" (RGB, comp 3) or "Pf" (grey, comp 1), "<w> <h>", scale -1.0 (= little-endian samples),
+ * then the rows BOTTOM to top.  `data` is row-major with row 0 at the top, like the framebuffer.  1 on success. */
+int rt_write_pfm(const char *filename, int w, int h, int comp, const float *data)
+{
+  if (!filename || !data || w <= 0 || h <= 0 || (comp != 1 && comp != 3))
+    return 0;
+  const size_t row = (size_t)w * comp;
+  uint8_t *buf = (uint8_t *)malloc(4 * row);
+  if (!buf)
+    return 0;
+  FILE *f = fopen(filename, "wb");
+  int ok = f != NULL && fprintf(f, "%s\n%d %d\n-1.0\n", comp == 3 ? "PF" : "Pf", w, h) > 0;
+  for (int y = h - 1; ok && y >= 0; y--)
+  {
+    for (size_t i = 0; i < row; i++)
+    {
+      uint32_t v;
+      memcpy(&v, data + (size_t)y * row + i, 4);
+      buf[4 * i + 0] = (uint8_t)v;
+      buf[4 * i + 1] = (uint8_t)(v >> 8);
+      buf[4 * i + 2] = (uint8_t)(v >> 16);
+      buf[4 * i + 3] = (uint8_t)(v >> 24);
+    }
+    ok = fwrite(buf, 1, 4 * row, f) == 4 * row;
+  }
+  if (f)
+    ok = (fclose(f) == 0) && ok;
+  free(buf);
   return ok;
 }

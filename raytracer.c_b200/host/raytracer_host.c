@@ -256,9 +256,41 @@ static rtb_comm *local_comm(int num_gpus)
   return g_comm;
 }
 
+/* the feature buffers of the frame just rendered, on the same scene: device sums -> means, in float */
+static void render_aov_means(rtb_scene *scene, const double *cam, const rtb_render_desc *desc, const RenderAov *aov)
+{
+  const size_t n_px = (size_t)desc->width * desc->height;
+  const int spp = desc->sample_end - desc->sample_begin;
+  uint32_t *hits = aov->depth ? (uint32_t *)malloc(sizeof(uint32_t) * n_px) : NULL;
+  if (aov->depth && !hits)
+  {
+    rtb_scene_destroy(scene);
+    fprintf(stderr, "render: out of host memory for the hit counts\n");
+    exit(EXIT_FAILURE);
+  }
+  if (rtb_render_aov_host(scene, cam, desc, aov->albedo, aov->normal, aov->depth, hits, aov->object, NULL) != RTB_OK)
+  {
+    free(hits);
+    rtb_scene_destroy(scene);
+    die("render: feature buffers");
+  }
+  const float n_samples = spp > 0 ? (float)spp : 1.0f; /* spp == 0: the sums are 0 */
+  for (size_t i = 0; i < 3 * n_px; i++)
+  {
+    if (aov->albedo)
+      aov->albedo[i] = aov->albedo[i] / n_samples;
+    if (aov->normal)
+      aov->normal[i] = aov->normal[i] / n_samples;
+  }
+  if (aov->depth)
+    for (size_t i = 0; i < n_px; i++)
+      aov->depth[i] = hits[i] ? aov->depth[i] / (float)hits[i] : 0.0f;
+  free(hits);
+}
+
 /* the body of render(): objects are Object (88-byte) or SceneObject (96-byte) records */
 static void render_records(uint8_t *framebuffer, const void *objects, size_t n_objects, int record_bytes,
-                           Camera *camera, Options *options, const RenderParams *params)
+                           Camera *camera, Options *options, const RenderParams *params, const RenderAov *aov)
 {
   RenderParams p;
   if (params)
@@ -276,9 +308,16 @@ static void render_records(uint8_t *framebuffer, const void *objects, size_t n_o
   const double *cam = (const double *)camera; /* 12 doubles, raytracer.h:121-124 */
   const int divisor = p.total_samples > 0 ? p.total_samples : options->samples;
   rtb_counters counters;
+  if (aov && !aov->albedo && !aov->normal && !aov->depth && !aov->object)
+    aov = NULL;
 
   if (p.num_gpus > 1)
   {
+    if (aov)
+    {
+      fprintf(stderr, "render: feature buffers (RenderAov) are single-GPU; render them with num_gpus = 1\n");
+      exit(EXIT_FAILURE);
+    }
     /* all GPUs of the box: spp-sharded, one ncclReduce of the float sums (rtb200.h) */
     if (p.total_samples > 0 && p.total_samples != options->samples)
     {
@@ -305,6 +344,8 @@ static void render_records(uint8_t *framebuffer, const void *objects, size_t n_o
       rtb_scene_destroy(scene);
       die("render");
     }
+    if (aov)
+      render_aov_means(scene, cam, &desc, aov);
     clock_gettime(CLOCK_MONOTONIC, &t2);
     rtb_scene_destroy(scene);
     if (timing)
@@ -320,7 +361,13 @@ static void render_records(uint8_t *framebuffer, const void *objects, size_t n_o
 void render_ex(uint8_t *framebuffer, Object *objects, size_t n_objects, Camera *camera, Options *options,
                const RenderParams *params)
 {
-  render_records(framebuffer, objects, n_objects, 88, camera, options, params);
+  render_records(framebuffer, objects, n_objects, 88, camera, options, params, NULL);
+}
+
+void render_ex_aov(uint8_t *framebuffer, Object *objects, size_t n_objects, Camera *camera, Options *options,
+                   const RenderParams *params, const RenderAov *aov)
+{
+  render_records(framebuffer, objects, n_objects, 88, camera, options, params, aov);
 }
 
 void render(uint8_t *framebuffer, Object *objects, size_t n_objects, Camera *camera, Options *options)
@@ -331,5 +378,11 @@ void render(uint8_t *framebuffer, Object *objects, size_t n_objects, Camera *cam
 void render_scene(uint8_t *framebuffer, SceneObject *objects, size_t n_objects, Camera *camera,
                   Options *options, const RenderParams *params)
 {
-  render_records(framebuffer, objects, n_objects, 96, camera, options, params);
+  render_records(framebuffer, objects, n_objects, 96, camera, options, params, NULL);
+}
+
+void render_scene_aov(uint8_t *framebuffer, SceneObject *objects, size_t n_objects, Camera *camera, Options *options,
+                      const RenderParams *params, const RenderAov *aov)
+{
+  render_records(framebuffer, objects, n_objects, 96, camera, options, params, aov);
 }
