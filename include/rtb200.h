@@ -18,6 +18,8 @@
  *                          object id) of the render's own camera samples, the inputs of a denoiser or a compositor
  *   rtb_trace_rays         intersect() for arbitrary rays (raytracer.c:393-464): parity probe
  *   rtb_trace_rays_wf      the same records from the wavefront renderer's trace kernel: parity probe
+ *   rtb_wf_generate, rtb_wf_bounce   the wavefront renderer's camera-ray and shade kernels, one launch at a time
+ *                          (trace_path's vertices, raytracer.c:482-554): parity probes
  *   rtb_path_records       per-path vertex records: parity probe for the 1-bounce check
  *   rtb_cast_rays          cast_ray() for arbitrary rays (raytracer.c:556-641): parity probe of the
  *                          Whitted integrator (rtb_render_desc.integrator = RTB_INTEGRATOR_WHITTED)
@@ -195,6 +197,27 @@ int rtb_trace_rays(rtb_scene *scene, const double *rays6, size_t n_rays, int use
 int rtb_trace_rays_wf(rtb_scene *scene, const double *rays6, size_t n_rays, int tune,
                       const uint32_t *perm_or_null, int32_t *ids, int64_t *prims, double *ts,
                       double *points, double *normals, double *uvs, rtb_counters *counters_or_null);
+/* The wavefront renderer's generate and shade kernels, one launch at a time, on the renderer's own arguments, plane
+ * groups, trace kernel (desc->reserved) and shade grid.  desc must fix the plane count (desc->planes > 0): path slot
+ * pid = plane * width * height + pixel carries sample sample_begin + plane * chunk + wave, chunk = ceil(spp / planes).
+ * Rays are 6 doubles (origin, direction), throughputs 3 floats, branch ids 1 on the camera ray (children 2b, 2b+1 of a
+ * split dielectric vertex).  Queue order is the kernels' (atomics).  Host buffers, blocking.
+ * rtb_wf_generate: camera rays of sample number `wave` of every plane (k_wf_generate): queue 0 of that wave; the
+ * arrays hold `cap` >= planes * width * height entries, *n_out gets the queue length. */
+int rtb_wf_generate(rtb_scene *scene, const double *camera12, const rtb_render_desc *desc, int wave, size_t cap,
+                    double *rays6, uint32_t *pid, float *throughput3, uint32_t *branch, size_t *n_out);
+/* rtb_wf_bounce: bounce `depth` of wave `wave` for n_rays queued rays (branch_or_null: NULL = 1 each; the split
+ * estimator needs them): the rays are queued as the renderer queues them, one trace launch finds their hits and one
+ * k_wf_shade launch shades them into planes4 (float[planes][height*width][4], read and written: planes_len floats) and
+ * appends the survivors to the output queue (cap_out >= 2 * n_rays entries; *n_out its length).  ids/prims/ts
+ * (optional): the hit record of every input ray (rtb_trace_rays' read-out).  counters_or_null: rays (the renderer's
+ * ray count of this bounce), rays_intersected, prim_tests (oversized-list tests of the outgoing rays).
+ * RTB_EINVAL on a path slot beyond the planes, a branch id 0 (or not 1 without split), depth outside [0, max_depth]. */
+int rtb_wf_bounce(rtb_scene *scene, const double *camera12, const rtb_render_desc *desc, int wave, int depth,
+                  size_t n_rays, const double *rays6, const uint32_t *pid, const float *throughput3,
+                  const uint32_t *branch_or_null, float *planes4, size_t planes_len, int32_t *ids_or_null,
+                  int64_t *prims_or_null, double *ts_or_null, size_t cap_out, double *rays6_out, uint32_t *pid_out,
+                  float *throughput3_out, uint32_t *branch_out, size_t *n_out, rtb_counters *counters_or_null);
 int rtb_path_records(rtb_scene *scene, const double *camera12, const rtb_render_desc *desc, int sample,
                      int n_vertices, int32_t *ids, double *points, double *normals, double *dists,
                      float *radiance);

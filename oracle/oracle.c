@@ -135,6 +135,8 @@ typedef struct
 {
   uint32_t bounce_word;
   uint32_t block0[4];
+  int tries;   /* hemisphere_dir: cube-rejection tries, i.e. Philox blocks of the keyed layout */
+  int flipped; /* hemisphere_dir: the direction was flipped into the normal's hemisphere */
 } VertexRng;
 
 static double rng_rr(Rng *g, VertexRng *v, int depth, uint32_t branch)
@@ -157,6 +159,7 @@ static double rng_choice(Rng *g, VertexRng *v)
 
 static void rng_try(Rng *g, VertexRng *v, int k, double xyz[3])
 {
+  v->tries = k + 1;
   if (g->mode == ORACLE_RNG_PHILOX)
   {
     if (k == 0)
@@ -455,6 +458,7 @@ static vec3 hemisphere_dir(Rng *g, VertexRng *vr, vec3 normal)
     p = (vec3){ r[0] * (1.0 - -1.0) + -1.0, r[1] * (1.0 - -1.0) + -1.0, r[2] * (1.0 - -1.0) + -1.0 };
   } while (vec3_length(p) > 1);
   vec3 d = vec3_normalize(p);
+  vr->flipped = vec3_dot(d, normal) < 0;
   if (vec3_dot(d, normal) < 0)
     return vec3_scalar_mult(d, -1);
   return d;
@@ -680,6 +684,240 @@ static void tracer_setup(Tracer *T, const SceneObject *objects, size_t n, const 
   T->n = n;
   T->max_depth = p->max_depth;
   T->dielectric_mode = p->dielectric_mode;
+}
+
+/* ---- trace() in forward form, one vertex at a time ------------------------------------------
+ * The same helpers and draws as trace(), but the throughput is carried forward: the vertex adds
+ * tp * emission (tp * background on a miss) and hands each child tp * albedo * weight.  A child at
+ * depth > max_depth is not traced: it adds its throughput * background and one ray (raytracer.c:487).
+ * Summed over a path (its whole tree for the split estimator), the contributions are trace()'s value
+ * up to the association of the products. */
+static void path_vertex(const Tracer *T, Rng *g, const Ray *ray, int depth, uint32_t branch, const double tp[3],
+                        OracleVertex *o)
+{
+  memset(o, 0, sizeof(*o));
+  memcpy(o->ray, &ray->origin, 3 * sizeof(double));
+  memcpy(o->ray + 3, &ray->direction, 3 * sizeof(double));
+  memcpy(o->tp, tp, 3 * sizeof(double));
+  o->pixel = g->pixel;
+  o->sample = g->sample;
+  o->branch = branch;
+  o->depth = depth;
+  o->id = -1;
+  o->prim = -1;
+  o->rays = 1;
+  const vec3 background = BACKGROUND;
+  const vec3 t = { tp[0], tp[1], tp[2] };
+  vec3 contrib;
+  Nearest hit;
+  if (depth > T->max_depth || !(hit = nearest_hit(ray, T->objects, T->n, &g->tests)).found)
+  {
+    contrib = vec3_mult(t, background);
+    memcpy(o->contrib, &contrib, sizeof(contrib));
+    return;
+  }
+  o->id = (int32_t)hit.object_id;
+  o->prim = hit.prim;
+  o->t = hit.t;
+  const Material *m = &T->objects[hit.object_id].material;
+  vec3 albedo = m->color;
+  contrib = vec3_mult(t, m->emission);
+
+  VertexRng vr;
+  memset(&vr, 0, sizeof(vr));
+  double prob = MAX(albedo.x, MAX(albedo.y, albedo.z));
+  if (rng_rr(g, &vr, depth, branch) < prob)
+    albedo = vec3_scalar_mult(albedo, 1 / prob);
+  else
+  {
+    memcpy(o->contrib, &contrib, sizeof(contrib));
+    return;
+  }
+  o->survived = 1;
+  uint flags = m->flags;
+  if (flags & M_CHECKERED)
+    albedo = checker(albedo, hit.u, hit.v, 100000);
+
+  vec3 dir[2];
+  double weight[2];
+  uint32_t child_branch[2] = { branch, branch };
+  int n_children = 1;
+  if (flags & M_REFRACTION)
+  {
+    double transparency = 1.0;
+    double facing = -vec3_dot(ray->direction, hit.normal);
+    double fresnel = mix(pow(1 - facing, 3), 1, 0.1);
+    double kr = fresnel;
+    double kt = (1 - fresnel) * transparency;
+    vec3 dir_t = vec3_normalize(refract_dir(vec3_scalar_mult(ray->direction, -1), hit.normal, 1.0));
+    vec3 dir_r = vec3_normalize(reflect_dir(vec3_scalar_mult(ray->direction, 1), hit.normal));
+    if (T->dielectric_mode == ORACLE_DIELECTRIC_SPLIT)
+    {
+      n_children = 2;
+      dir[0] = dir_t; weight[0] = kt; child_branch[0] = branch << 1;
+      dir[1] = dir_r; weight[1] = kr; child_branch[1] = (branch << 1) | 1u;
+    }
+    else
+    {
+      double p = kr < 0.05 ? 0.05 : (kr > 0.95 ? 0.95 : kr);
+      if (rng_choice(g, &vr) < p)
+      {
+        dir[0] = dir_r; weight[0] = kr / p;
+      }
+      else
+      {
+        dir[0] = dir_t; weight[0] = kt / (1 - p);
+      }
+    }
+  }
+  else if (flags & M_REFLECTION)
+  {
+    dir[0] = reflect_dir(ray->direction, hit.normal); /* not renormalised (quirk Q8) */
+    weight[0] = 1.0;
+  }
+  else
+  {
+    dir[0] = hemisphere_dir(g, &vr, hit.normal);
+    weight[0] = vec3_dot(dir[0], hit.normal);
+    o->tries = vr.tries;
+    o->flipped = vr.flipped;
+  }
+  o->n_children = n_children;
+  for (int k = 0; k < n_children; k++)
+  {
+    vec3 ct = vec3_scalar_mult(vec3_mult(t, albedo), weight[k]);
+    memcpy(o->child_ray[k], &hit.point, sizeof(vec3));
+    memcpy(o->child_ray[k] + 3, &dir[k], sizeof(vec3));
+    memcpy(o->child_tp[k], &ct, sizeof(vec3));
+    o->child_branch[k] = child_branch[k];
+    if (depth + 1 > T->max_depth)
+    {
+      o->cut[k] = 1;
+      o->rays++;
+      contrib = vec3_add(contrib, vec3_mult(ct, background));
+    }
+  }
+  memcpy(o->contrib, &contrib, sizeof(contrib));
+}
+
+void oracle_path_vertex(const SceneObject *objects, size_t n, const OracleParams *p, const double *rays6,
+                        const int32_t *depth, const uint32_t *branch, const uint32_t *pixel, const uint32_t *sample,
+                        const double *tp3, long long count, OracleVertex *out)
+{
+  int threads = p->threads > 0 ? p->threads : 1;
+#pragma omp parallel for num_threads(threads) schedule(dynamic, 256)
+  for (long long i = 0; i < count; i++)
+  {
+    OracleParams q = *p;
+    q.rng_mode = ORACLE_RNG_PHILOX;
+    Rng g;
+    rng_setup(&g, &q);
+    g.pixel = pixel[i];
+    g.sample = sample[i];
+    Tracer T;
+    tracer_setup(&T, objects, n, &q);
+    Ray ray = { { rays6[6 * i], rays6[6 * i + 1], rays6[6 * i + 2] }, { rays6[6 * i + 3], rays6[6 * i + 4], rays6[6 * i + 5] } };
+    path_vertex(&T, &g, &ray, depth[i], branch[i], tp3 + 3 * i, &out[i]);
+  }
+}
+
+typedef struct
+{
+  OracleVertex *v;
+  long long n, cap;
+} VertexList;
+
+static void vertex_push(VertexList *l, const OracleVertex *v)
+{
+  if (l->n == l->cap)
+  {
+    l->cap = l->cap ? 2 * l->cap : 1024;
+    l->v = (OracleVertex *)realloc(l->v, sizeof(OracleVertex) * (size_t)l->cap);
+    if (!l->v)
+    {
+      fprintf(stderr, "oracle: out of memory\n");
+      exit(EXIT_FAILURE);
+    }
+  }
+  l->v[l->n++] = *v;
+}
+
+long long oracle_path_log(const SceneObject *objects, size_t n, const Camera *camera, int width, int height,
+                          int samples, const OracleParams *p, OracleVertex *out, long long cap)
+{
+  int threads = p->threads > 0 ? p->threads : 1;
+  VertexList *rows = (VertexList *)calloc((size_t)height, sizeof(VertexList));
+  if (!rows)
+  {
+    fprintf(stderr, "oracle: out of memory\n");
+    exit(EXIT_FAILURE);
+  }
+#pragma omp parallel for num_threads(threads) schedule(dynamic, 1)
+  for (int y = 0; y < height; y++)
+  {
+    OracleParams q = *p;
+    q.rng_mode = ORACLE_RNG_PHILOX;
+    Rng g;
+    rng_setup(&g, &q);
+    Tracer T;
+    tracer_setup(&T, objects, n, &q);
+    /* pending rays of one path: at most one per depth and branch bit, so depth + 2 per level suffices */
+    int stack_cap = 2 * (q.max_depth + 2) + 2;
+    OracleVertex *stack = (OracleVertex *)malloc(sizeof(OracleVertex) * (size_t)stack_cap);
+    for (int x = 0; x < width; x++)
+      for (int s = 0; s < samples; s++)
+      {
+        g.pixel = (uint32_t)(y * width + x);
+        g.sample = (uint32_t)(p->sample_offset + s);
+        double j1, j2;
+        rng_jitter(&g, &j1, &j2);
+        double u = (double)(x + j1) / ((double)width - 1.0);
+        double v = (double)(y + j2) / ((double)height - 1.0);
+        Ray ray = camera_ray(camera, u, v);
+        /* stack entries use ray[], tp[], depth and branch only */
+        int top = 0;
+        memcpy(stack[0].ray, &ray.origin, 3 * sizeof(double));
+        memcpy(stack[0].ray + 3, &ray.direction, 3 * sizeof(double));
+        stack[0].tp[0] = stack[0].tp[1] = stack[0].tp[2] = 1.0;
+        stack[0].depth = 0;
+        stack[0].branch = 1u;
+        top = 1;
+        while (top > 0)
+        {
+          OracleVertex e = stack[--top], o;
+          Ray r = { { e.ray[0], e.ray[1], e.ray[2] }, { e.ray[3], e.ray[4], e.ray[5] } };
+          path_vertex(&T, &g, &r, e.depth, e.branch, e.tp, &o);
+          vertex_push(&rows[y], &o);
+          for (int k = o.n_children - 1; k >= 0; k--) /* child 0 first, as trace() recurses */
+            if (!o.cut[k])
+            {
+              OracleVertex *c = &stack[top++];
+              memcpy(c->ray, o.child_ray[k], sizeof(c->ray));
+              memcpy(c->tp, o.child_tp[k], sizeof(c->tp));
+              c->depth = o.depth + 1;
+              c->branch = o.child_branch[k];
+            }
+        }
+      }
+    free(stack);
+  }
+  long long total = 0;
+  for (int y = 0; y < height; y++)
+    total += rows[y].n;
+  if (total <= cap)
+  {
+    long long at = 0;
+    for (int y = 0; y < height; y++)
+    {
+      if (rows[y].n)
+        memcpy(out + at, rows[y].v, sizeof(OracleVertex) * (size_t)rows[y].n);
+      at += rows[y].n;
+    }
+  }
+  for (int y = 0; y < height; y++)
+    free(rows[y].v);
+  free(rows);
+  return total;
 }
 
 /* sum over samples [sample_offset, sample_offset+samples) per pixel, in double.

@@ -56,6 +56,35 @@ void oracle_path_records(const SceneObject *objects, size_t n, const Camera *cam
                          int sample, int n_vertices, const OracleParams *p, int32_t *ids, double *points,
                          double *normals, double *dists, double *radiance);
 
+/* One vertex of trace_path in forward form (oracle.c, path_vertex).  Field order is ABI: tests/oracle_lib.py. */
+typedef struct
+{
+  double ray[6];          /* the incoming ray: origin, direction */
+  double tp[3];           /* incoming throughput */
+  double contrib[3];      /* tp * emission (tp * background on a miss) + child tp * background per cut child */
+  double t;               /* nearest hit distance (0 on a miss) */
+  double child_ray[2][6]; /* origin (the hit point) and direction of each child */
+  double child_tp[2][3];  /* tp * albedo / prob [* checker] * weight */
+  int64_t prim;           /* primitive hit in loop order, -1 on a miss */
+  uint32_t pixel, sample, branch, child_branch[2];
+  int32_t depth, id;      /* id: object hit, -1 on a miss */
+  int32_t survived;       /* Russian roulette let the path go on (0 on a miss) */
+  int32_t rays;           /* ray-counter increment: this ray plus every cut child */
+  int32_t n_children;     /* 0, 1 or 2 (split dielectric), cut children included */
+  int32_t cut[2];         /* child k has depth > max_depth: it adds background and a ray, and is not traced */
+  int32_t tries;          /* cube-rejection tries (Philox blocks) of a diffuse vertex, else 0 */
+  int32_t flipped;        /* the hemisphere sample was flipped into the normal's side */
+} OracleVertex;
+
+/* vertex i of `count`: rays6[6i..], depth[i], branch[i], keyed by (pixel[i], sample[i]), incoming throughput tp3[3i..] */
+void oracle_path_vertex(const SceneObject *objects, size_t n, const OracleParams *p, const double *rays6,
+                        const int32_t *depth, const uint32_t *branch, const uint32_t *pixel, const uint32_t *sample,
+                        const double *tp3, long long count, OracleVertex *out);
+/* every vertex of every path (the whole tree for the split estimator) of samples [sample_offset, +samples) of the
+ * frame, rows in order; returns the number of vertices and writes them only when it is <= cap */
+long long oracle_path_log(const SceneObject *objects, size_t n, const Camera *camera, int width, int height,
+                          int samples, const OracleParams *p, OracleVertex *out, long long cap);
+
 void oracle_cast_rays(const SceneObject *objects, size_t n_obj, const double *rays, long long n_rays,
                       int max_depth, double *rgb, long long *ray_counts, int threads);
 

@@ -25,7 +25,7 @@ RTB_SYMBOLS = [
     "rtb_trace_rays", "rtb_trace_rays_wf", "rtb_path_records", "rtb_philox4x32_10", "rtb_probe_l2_bandwidth", "rtb_cast_rays",
     "rtb_probe_fp32_tflops", "rtb_render_mean", "rtb_comm_unique_id", "rtb_comm_create_rank", "rtb_comm_create_local", "rtb_comm_size",
     "rtb_warm_up", "rtb_comm_local_ranks", "rtb_comm_destroy", "rtb_comm_shard_samples", "rtb_comm_scene_create", "rtb_comm_render", "rtb_render_multi",
-    "rtb_render_aov", "rtb_render_aov_host",
+    "rtb_render_aov", "rtb_render_aov_host", "rtb_wf_generate", "rtb_wf_bounce",
 ]
 # the reference's exported surface (raytracer.h:135-164) plus the documented extensions
 HOST_SYMBOLS = [
@@ -82,6 +82,10 @@ def _bind(cu, host):
     cu.rtb_trace_rays.argtypes = [C.c_void_p, C.c_void_p, C.c_size_t, C.c_int] + [C.c_void_p] * 6
     cu.rtb_trace_rays_wf.argtypes = [C.c_void_p, C.c_void_p, C.c_size_t, C.c_int] + [C.c_void_p] * 7 + [
         C.POINTER(abi.RtbCounters)]
+    cu.rtb_wf_generate.argtypes = [C.c_void_p, dp, C.POINTER(abi.RtbRenderDesc), C.c_int, C.c_size_t] + [C.c_void_p] * 5
+    cu.rtb_wf_bounce.argtypes = ([C.c_void_p, dp, C.POINTER(abi.RtbRenderDesc), C.c_int, C.c_int, C.c_size_t] + [C.c_void_p] * 5
+                                 + [C.c_size_t] + [C.c_void_p] * 3 + [C.c_size_t] + [C.c_void_p] * 5
+                                 + [C.POINTER(abi.RtbCounters)])
     cu.rtb_path_records.argtypes = [C.c_void_p, dp, C.POINTER(abi.RtbRenderDesc), C.c_int, C.c_int] + [C.c_void_p] * 5
     cu.rtb_philox4x32_10.argtypes = [C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, C.c_int]
     cu.rtb_cast_rays.argtypes = [C.c_void_p, C.c_void_p, C.c_size_t, C.c_int, C.c_void_p, C.c_void_p]
@@ -311,6 +315,26 @@ def make_desc(width, height, sample_begin, sample_end, max_depth=5, seed=abi.SCE
     return d
 
 
+def wf_planes(desc):
+    """(planes, samples per plane) of a desc with a fixed plane count, as rtb_plane_split cuts them: path slot
+    plane * width * height + pixel carries sample sample_begin + plane * chunk + wave"""
+    spp = desc.sample_end - desc.sample_begin
+    if desc.planes <= 0 or spp <= 0:
+        raise ValueError("the wavefront probes need desc.planes > 0 and at least one sample")
+    splits = max(1, min(min(desc.planes, 1024), spp))
+    chunk = (spp + splits - 1) // splits
+    return (spp + chunk - 1) // chunk, chunk
+
+
+def _queue(n):
+    return dict(rays=np.zeros((n, 6), np.float64), pid=np.zeros(n, np.uint32), throughput=np.zeros((n, 3), np.float32),
+                branch=np.zeros(n, np.uint32))
+
+
+def _queue_ptrs(q):
+    return [q[k].ctypes.data for k in ("rays", "pid", "throughput", "branch")]
+
+
 class Scene:
     """Device-resident scene (SoA geometry + BVH).  `source` is a structured Object array
     (spheres) or an abi.SceneHolder (spheres and meshes)."""
@@ -455,6 +479,42 @@ class Scene:
                                          out["normals"].ctypes.data, out["dists"].ctypes.data,
                                          out["radiance"].ctypes.data), "rtb_path_records")
         return out
+
+    def wf_generate(self, camera, desc, wave):
+        """queue 0 of wave `wave` from the renderer's camera-ray kernel (rtb_wf_generate) -> dict(rays [n, 6] f64,
+        pid [n] u32, throughput [n, 3] f32, branch [n] u32), in queue order"""
+        cam = camera.as_array()
+        cap = wf_planes(desc)[0] * desc.width * desc.height
+        q = _queue(cap)
+        n = C.c_size_t()
+        _check(self._cu.rtb_wf_generate(self._h, cam.ctypes.data_as(C.POINTER(C.c_double)), C.byref(desc), int(wave),
+                                        cap, *_queue_ptrs(q), C.byref(n)), "rtb_wf_generate")
+        return {k: v[:n.value] for k, v in q.items()}
+
+    def wf_bounce(self, camera, desc, wave, depth, queue, planes):
+        """bounce `depth` of wave `wave` for `queue` (a wf_generate / wf_bounce result) through the renderer's trace
+        and shade kernels (rtb_wf_bounce).  `planes` (float32 [planes, H*W, 4]) is shaded into in place.
+        -> (outgoing queue, dict(ids, prims, t) of the input rays' hits, abi.RtbCounters)"""
+        cam = camera.as_array()
+        rays = np.ascontiguousarray(queue["rays"], np.float64).reshape(-1, 6)
+        n = len(rays)
+        pid = np.ascontiguousarray(queue["pid"], np.uint32)
+        tp = np.ascontiguousarray(queue["throughput"], np.float32).reshape(-1, 3)
+        branch = np.ascontiguousarray(queue["branch"], np.uint32)
+        if pid.shape != (n,) or tp.shape != (n, 3) or branch.shape != (n,):
+            raise ValueError("queue arrays of different lengths")
+        if planes.dtype != np.float32 or not planes.flags.c_contiguous:
+            raise ValueError("planes must be a C-contiguous float32 array")
+        hits = dict(ids=np.zeros(n, np.int32), prims=np.zeros(n, np.int64), t=np.zeros(n, np.float64))
+        out = _queue(2 * n)
+        n_out = C.c_size_t()
+        ctr = abi.RtbCounters()
+        _check(self._cu.rtb_wf_bounce(self._h, cam.ctypes.data_as(C.POINTER(C.c_double)), C.byref(desc), int(wave),
+                                      int(depth), n, rays.ctypes.data, pid.ctypes.data, tp.ctypes.data, branch.ctypes.data,
+                                      planes.ctypes.data, planes.size, hits["ids"].ctypes.data,
+                                      hits["prims"].ctypes.data, hits["t"].ctypes.data, 2 * n, *_queue_ptrs(out),
+                                      C.byref(n_out), C.byref(ctr)), "rtb_wf_bounce")
+        return {k: v[:n_out.value] for k, v in out.items()}, hits, ctr
 
 
 # ---- all the GPUs of one box (rtb_comm_*, include/rtb200.h) ---------------------------------------

@@ -934,6 +934,75 @@ static void wf_launch_trace(const WfTraceTune &t, bool stats, int sm_count, cuda
   }
 }
 
+/* blocks of the grid-stride shade kernel */
+static int wf_shade_blocks(int sm_count)
+{
+  if (const char *e = getenv("RTB_WF_SHADE_BLOCKS")) /* development knob: blocks per SM */
+    return sm_count * std::max(1, atoi(e));
+  return sm_count * 16;
+}
+
+/* Two groups of planes, each with its own queues and its own stream: the persistent kernels of one group
+ * drain (their last warps finishing the longest rays) while the other group's next kernel fills the SMs that
+ * become free.  A path slot belongs to one group, so the order of additions per slot -- and the result, bit
+ * for bit -- is that of the one-stream schedule.  Not with per-kernel timing, the split estimator, ray sorting
+ * or the ray-pool kernel (one set of their buffers). */
+static int wf_group_count(const RenderArgs &A, bool timed, bool split, bool sorted, bool pool)
+{
+  const bool may = !timed && !split && !sorted && !pool;
+  int n_groups = may ? 2 : 1;
+  if (const char *e = getenv("RTB_WF_STREAMS"))
+    n_groups = may ? atoi(e) : 1;
+  return std::max(1, std::min(std::min(n_groups, WF_MAX_GROUPS), A.splits));
+}
+
+/* one group of planes: planes [A.plane_base, A.plane_base + planes), its slices of the two queues, its queue
+ * lengths and trace fetch cursors (the stream is the caller's) */
+struct WfGroup
+{
+  cudaStream_t stream;
+  RenderArgs A;
+  WfQueue q[2];
+  unsigned *counts, *fetch;
+  int planes, gen_blocks;
+  bool has_last;
+};
+
+/* the groups of wf_render: queues q[] hold `cap` entries; group g's counters start at ctr_base + g * ctr_one */
+static void wf_groups(const RenderArgs &A, int n_groups, const WfQueue q[2], size_t cap, char *ctr_base, size_t ctr_one,
+                      int n_bounces, WfGroup *G)
+{
+  const size_t n_px = (size_t)A.width * A.height;
+  for (int g = 0; g < n_groups; g++)
+  {
+    WfGroup &R = G[g];
+    R.stream = nullptr;
+    R.A = A;
+    R.A.plane_base = (int)((long long)A.splits * g / n_groups);
+    R.planes = (int)((long long)A.splits * (g + 1) / n_groups) - R.A.plane_base;
+    R.has_last = g == n_groups - 1;
+    const size_t first_slot = (size_t)R.A.plane_base * n_px;
+    for (int k = 0; k < 2; k++)
+    {
+      R.q[k] = q[k];
+      R.q[k].o_xy += first_slot; R.q[k].oz_dx += first_slot; R.q[k].d_yz += first_slot;
+      R.q[k].path += first_slot; R.q[k].hit += first_slot;
+      if (R.q[k].branch) R.q[k].branch += first_slot;
+      R.q[k].cap = n_groups == 1 ? (unsigned)cap : (unsigned)((size_t)R.planes * n_px);
+    }
+    R.counts = reinterpret_cast<unsigned *>(ctr_base + (size_t)g * ctr_one);
+    R.fetch = R.counts + (n_bounces + 2);
+    R.gen_blocks = (int)(((long long)A.n_tiles * R.planes * 32 + 255) / 256);
+  }
+}
+
+/* planes of group R whose sub-range still has a sample number `wave`: all, or all but the (shorter) last */
+static int wf_valid_planes(const WfGroup &R, const RenderArgs &A, int wave)
+{
+  const int last_len = (A.s_end - A.s_begin) - (A.splits - 1) * A.chunk;
+  return (R.has_last && wave >= last_len) ? R.planes - 1 : R.planes;
+}
+
 int wf_render(rtb_scene *scene, RenderArgs &A, const rtb_render_desc *desc, float *d_accum, cudaStream_t stream,
               bool stats, unsigned long long &launches, float *phase_ms)
 {
@@ -1056,9 +1125,7 @@ int wf_render(rtb_scene *scene, RenderArgs &A, const rtb_render_desc *desc, floa
 
   RTB_CUDA(cudaMemsetAsync(planes, 0, slots * 16, stream));
 
-  int shade_blocks = sm_count * 16;
-  if (const char *e = getenv("RTB_WF_SHADE_BLOCKS")) /* development knob: blocks per SM of the grid-stride shade kernel */
-    shade_blocks = sm_count * std::max(1, atoi(e));
+  const int shade_blocks = wf_shade_blocks(sm_count);
 
   /* per-kernel timing (only with counters): events around every trace launch */
   struct EventList : std::vector<cudaEvent_t> /* destroyed on every return path */
@@ -1077,15 +1144,7 @@ int wf_render(rtb_scene *scene, RenderArgs &A, const rtb_render_desc *desc, floa
     cudaEventRecord(e, stream);
     ev.push_back(e);
   };
-  /* Two groups of planes, each with its own queues and its own stream: the persistent kernels of one group
-   * drain (their last warps finishing the longest rays) while the other group's next kernel fills the SMs that
-   * become free.  A path slot belongs to one group, so the order of additions per slot -- and the result, bit
-   * for bit -- is that of the one-stream schedule.  Not with per-kernel timing, the split estimator, ray sorting
-   * or the ray-pool kernel (one set of their buffers). */
-  int n_groups = (!phase_ms && !split && !sort_mode && !pool) ? 2 : 1;
-  if (const char *e = getenv("RTB_WF_STREAMS"))
-    n_groups = (!phase_ms && !split && !sort_mode && !pool) ? atoi(e) : 1;
-  n_groups = std::max(1, std::min(std::min(n_groups, WF_MAX_GROUPS), A.splits));
+  const int n_groups = wf_group_count(A, phase_ms != nullptr, split, sort_mode != 0, pool);
   for (int g = 1; g < n_groups; g++)
     if (!scene->wf_streams[g])
     {
@@ -1103,37 +1162,10 @@ int wf_render(rtb_scene *scene, RenderArgs &A, const rtb_render_desc *desc, floa
       if (!scene->wf_fork)
         RTB_CUDA(cudaEventCreateWithFlags(&scene->wf_fork, cudaEventDisableTiming));
     }
-  const int last_len = (A.s_end - A.s_begin) - (A.splits - 1) * A.chunk; /* samples of the (shorter) last plane */
-  struct Group
-  {
-    cudaStream_t stream;
-    RenderArgs A;
-    WfQueue q[2];
-    unsigned *counts, *fetch;
-    int planes, gen_blocks;
-    bool has_last;
-  } G[WF_MAX_GROUPS];
+  WfGroup G[WF_MAX_GROUPS];
+  wf_groups(A, n_groups, q, cap, ctr_base, ctr_one, n_bounces, G);
   for (int g = 0; g < n_groups; g++)
-  {
-    Group &R = G[g];
-    R.stream = g == 0 ? stream : scene->wf_streams[g];
-    R.A = A;
-    R.A.plane_base = (int)((long long)A.splits * g / n_groups);
-    R.planes = (int)((long long)A.splits * (g + 1) / n_groups) - R.A.plane_base;
-    R.has_last = g == n_groups - 1;
-    const size_t first_slot = (size_t)R.A.plane_base * n_px;
-    for (int k = 0; k < 2; k++)
-    {
-      R.q[k] = q[k];
-      R.q[k].o_xy += first_slot; R.q[k].oz_dx += first_slot; R.q[k].d_yz += first_slot;
-      R.q[k].path += first_slot; R.q[k].hit += first_slot;
-      if (R.q[k].branch) R.q[k].branch += first_slot;
-      R.q[k].cap = n_groups == 1 ? (unsigned)cap : (unsigned)((size_t)R.planes * n_px);
-    }
-    R.counts = reinterpret_cast<unsigned *>(ctr_base + (size_t)g * ctr_one);
-    R.fetch = R.counts + (n_bounces + 2);
-    R.gen_blocks = (int)(((long long)A.n_tiles * R.planes * 32 + 255) / 256);
-  }
+    G[g].stream = g == 0 ? stream : scene->wf_streams[g];
   if (n_groups > 1)
   {
     RTB_CUDA(cudaEventRecord(scene->wf_fork, stream)); /* the planes are zeroed, the scene is built */
@@ -1144,17 +1176,15 @@ int wf_render(rtb_scene *scene, RenderArgs &A, const rtb_render_desc *desc, floa
   {
     for (int g = 0; g < n_groups; g++)
     {
-      Group &R = G[g];
+      WfGroup &R = G[g];
       RTB_CUDA(cudaMemsetAsync(R.counts, 0, sizeof(unsigned) * 2 * (size_t)(n_bounces + 2), R.stream));
-      /* planes whose sub-range still has a sample number `wave`: all, or all but the last */
-      const int n_valid_planes = (R.has_last && wave >= last_len) ? R.planes - 1 : R.planes;
-      k_wf_generate<<<R.gen_blocks, 256, 0, R.stream>>>(R.A, wave, n_valid_planes, R.q[0], &R.counts[0]);
+      k_wf_generate<<<R.gen_blocks, 256, 0, R.stream>>>(R.A, wave, wf_valid_planes(R, A, wave), R.q[0], &R.counts[0]);
       launches++;
     }
     for (int b = 0; b < n_bounces; b++)
       for (int g = 0; g < n_groups; g++)
       {
-        Group &R = G[g];
+        WfGroup &R = G[g];
         cudaStream_t st = R.stream;
         unsigned *cnt = R.counts, *fch = R.fetch;
         const WfQueue &qi = R.q[b & 1], &qo = R.q[(b + 1) & 1];
@@ -1224,9 +1254,11 @@ int wf_render(rtb_scene *scene, RenderArgs &A, const rtb_render_desc *desc, floa
 /* ---- parity probe: the product trace kernel on caller rays -------------------------------------- */
 
 /* queue entry i = ray i with its hit record seeded from the oversized list, exactly as k_wf_generate / k_wf_shade
- * write it; the big-list exact tests go to totals[2] */
-__global__ void k_wf_fill(const __grid_constant__ SceneView sv, const double *__restrict__ rays, unsigned n, WfQueue q,
-                          unsigned long long *totals)
+ * write it, and path slot pid[i] (else i), throughput tp3[3i..] (else 0) and branch[i] (else 1); the big-list exact
+ * tests go to totals[2] */
+__global__ void k_wf_fill(const __grid_constant__ SceneView sv, const double *__restrict__ rays,
+                          const unsigned *__restrict__ pid, const float *__restrict__ tp3, const unsigned *__restrict__ branch,
+                          unsigned n, WfQueue q, unsigned long long *totals)
 {
   const unsigned i = blockIdx.x * blockDim.x + threadIdx.x;
   const int lane = threadIdx.x & 31;
@@ -1240,8 +1272,12 @@ __global__ void k_wf_fill(const __grid_constant__ SceneView sv, const double *__
     q.o_xy[i] = make_double2(o.x, o.y);
     q.oz_dx[i] = make_double2(o.z, d.x);
     q.d_yz[i] = make_double2(d.y, d.z);
-    q.path[i] = make_uint4(i, 0u, 0u, 0u);
+    const float r = tp3 ? tp3[3 * (size_t)i + 0] : 0.0f, g = tp3 ? tp3[3 * (size_t)i + 1] : 0.0f,
+                b = tp3 ? tp3[3 * (size_t)i + 2] : 0.0f;
+    q.path[i] = make_uint4(pid ? pid[i] : i, __float_as_uint(r), __float_as_uint(g), __float_as_uint(b));
     q.hit[i] = pack_hit(seed);
+    if (q.branch)
+      q.branch[i] = branch ? branch[i] : 1u;
   }
   wf_add_counters(totals, lane, 0ull, 0ull, exact, 0ull, 0ull);
 }
@@ -1341,7 +1377,7 @@ extern "C" int rtb_trace_rays_wf(rtb_scene *scene, const double *rays6, size_t n
   q.branch = nullptr;
   q.cap = n;
   const unsigned blocks = (unsigned)((m + 127) / 128);
-  k_wf_fill<<<blocks, 128>>>(sv, d_rays.p, n, q, d_totals.p);
+  k_wf_fill<<<blocks, 128>>>(sv, d_rays.p, nullptr, nullptr, nullptr, n, q, d_totals.p);
   RTB_CUDA(cudaGetLastError());
   wf_launch_trace(t, true, sm_count, 0, sv, q, d_ctl.p, d_ctl.p + 1, d_totals.p, d_stacks.p, d_perm.p);
   RTB_CUDA(cudaGetLastError());
@@ -1366,6 +1402,288 @@ extern "C" int rtb_trace_rays_wf(rtb_scene *scene, const double *rays6, size_t n
     counters_or_null->prim_tests = h[2];
     counters_or_null->node_visits = h[3];
     counters_or_null->launches = 3;
+    counters_or_null->trace_launches = 1;
+  }
+  return RTB_OK;
+}
+
+/* ---- parity probes: the product generate and shade kernels, one launch at a time ------------------------------
+ * They run what wf_render runs -- the same RenderArgs (fill_args, rtb_plane_split), plane groups (wf_groups), trace
+ * dispatch (wf_trace_tune, wf_launch_trace) and shade grid -- on queues they own, so that a test can compare every
+ * ray of every bounce with the oracle.  The plane count must be fixed (desc->planes > 0): it decides which sample
+ * a path slot carries.  Queue ORDER is the kernels' (atomics); the caller sorts. */
+
+/* the device arrays of one probe queue of `cap` entries; branch ids only for the split estimator */
+struct WfProbeQueue
+{
+  Dev<double2> oxy, ozdx, dyz;
+  Dev<uint4> path, hit;
+  Dev<unsigned> branch;
+  WfQueue q;
+  int alloc(size_t cap, bool split)
+  {
+    const size_t m = cap > 0 ? cap : 1;
+    RTB_CUDA(cudaMalloc(&oxy.p, sizeof(double2) * m));
+    RTB_CUDA(cudaMalloc(&ozdx.p, sizeof(double2) * m));
+    RTB_CUDA(cudaMalloc(&dyz.p, sizeof(double2) * m));
+    RTB_CUDA(cudaMalloc(&path.p, sizeof(uint4) * m));
+    RTB_CUDA(cudaMalloc(&hit.p, sizeof(uint4) * m));
+    if (split)
+      RTB_CUDA(cudaMalloc(&branch.p, sizeof(unsigned) * m));
+    q.o_xy = oxy.p; q.oz_dx = ozdx.p; q.d_yz = dyz.p; q.path = path.p; q.hit = hit.p; q.branch = branch.p;
+    q.cap = (unsigned)cap;
+    return RTB_OK;
+  }
+};
+
+/* entries [first, first + n) of q -> host rays (origin, direction), path slot, throughput, branch (1 without ids) */
+static int wf_probe_read(const WfQueue &q, size_t first, size_t n, double *rays6, uint32_t *pid, float *tp3, uint32_t *branch)
+{
+  if (n == 0)
+    return RTB_OK;
+  std::vector<double2> a(n), b(n), c(n);
+  std::vector<uint4> p(n);
+  std::vector<unsigned> br(n, 1u);
+  RTB_CUDA(cudaMemcpy(a.data(), q.o_xy + first, sizeof(double2) * n, cudaMemcpyDeviceToHost));
+  RTB_CUDA(cudaMemcpy(b.data(), q.oz_dx + first, sizeof(double2) * n, cudaMemcpyDeviceToHost));
+  RTB_CUDA(cudaMemcpy(c.data(), q.d_yz + first, sizeof(double2) * n, cudaMemcpyDeviceToHost));
+  RTB_CUDA(cudaMemcpy(p.data(), q.path + first, sizeof(uint4) * n, cudaMemcpyDeviceToHost));
+  if (q.branch)
+    RTB_CUDA(cudaMemcpy(br.data(), q.branch + first, sizeof(unsigned) * n, cudaMemcpyDeviceToHost));
+  for (size_t i = 0; i < n; i++)
+  {
+    const double r[6] = { a[i].x, a[i].y, b[i].x, b[i].y, c[i].x, c[i].y };
+    memcpy(rays6 + 6 * i, r, sizeof(r));
+    pid[i] = p[i].x;
+    memcpy(tp3 + 3 * i, &p[i].y, 3 * sizeof(float));
+    branch[i] = br[i];
+  }
+  return RTB_OK;
+}
+
+/* the RenderArgs and trace kernel of a probe call, with wf_render's chunk and splits */
+static int wf_probe_args(const char *who, rtb_scene *scene, const double *camera12, const rtb_render_desc *desc, int wave,
+                         RenderArgs &A, WfTraceTune &tune, int &sm_count)
+{
+  const std::string name(who);
+  if (!scene || !camera12 || !desc)
+  {
+    rtb_set_error(name + ": NULL argument");
+    return RTB_EINVAL;
+  }
+  int rc = rtb_check_desc(desc);
+  if (rc != RTB_OK)
+    return rc;
+  if (desc->integrator != RTB_INTEGRATOR_PATH || (desc->kernel != 0 && desc->kernel != 6))
+  {
+    rtb_set_error(name + ": the wavefront path tracer only (integrator RTB_INTEGRATOR_PATH, kernel 0 or 6)");
+    return RTB_EINVAL;
+  }
+  const int spp = desc->sample_end - desc->sample_begin;
+  if (desc->planes <= 0 || spp <= 0)
+  {
+    rtb_set_error(name + ": need desc->planes > 0 (it fixes the sample of every path slot) and at least one sample");
+    return RTB_EINVAL;
+  }
+  fill_args(A, scene, camera12, desc);
+  const size_t n_px = (size_t)A.width * A.height;
+  int chunk = 0;
+  A.splits = rtb_plane_split((long long)n_px, n_px, desc->planes, spp, &chunk);
+  A.chunk = chunk;
+  if (n_px * (size_t)A.splits >= (1ull << 31))
+  {
+    rtb_set_error(name + ": width*height*planes must stay below 2^31");
+    return RTB_EINVAL;
+  }
+  if (wave < 0 || wave >= A.chunk)
+  {
+    rtb_set_error(name + ": wave must lie in [0, samples per plane)");
+    return RTB_EINVAL;
+  }
+  rc = wf_trace_tune(A.sv, desc->reserved, tune);
+  if (rc != RTB_OK)
+    return rc;
+  RTB_CUDA(cudaSetDevice(scene->device));
+  sm_count = 148;
+  cudaDeviceGetAttribute(&sm_count, cudaDevAttrMultiProcessorCount, scene->device);
+  return RTB_OK;
+}
+
+extern "C" int rtb_wf_generate(rtb_scene *scene, const double *camera12, const rtb_render_desc *desc, int wave,
+                               size_t cap, double *rays6, uint32_t *pid, float *throughput3, uint32_t *branch,
+                               size_t *n_out)
+{
+  RenderArgs A;
+  WfTraceTune tune;
+  int sm_count = 0;
+  int rc = wf_probe_args("rtb_wf_generate", scene, camera12, desc, wave, A, tune, sm_count);
+  if (rc != RTB_OK)
+    return rc;
+  const size_t n_px = (size_t)A.width * A.height, slots = n_px * (size_t)A.splits;
+  if (!rays6 || !pid || !throughput3 || !branch || !n_out || cap < slots)
+  {
+    rtb_set_error("rtb_wf_generate: NULL output, or cap below planes*width*height");
+    return RTB_EINVAL;
+  }
+  const bool split = A.dielectric_mode == RTB_DIELECTRIC_SPLIT;
+  const int sort_mode = split ? 0 : (desc->reserved2 & 0xFF);
+  const int n_groups = wf_group_count(A, false, split, sort_mode != 0, tune.pool);
+  const int n_bounces = A.max_depth + 1;
+  const size_t ctr_one = align_up(sizeof(unsigned) * (2 * (size_t)(n_bounces + 2) + 1), 256);
+  WfProbeQueue pq;
+  rc = pq.alloc(slots, split);
+  if (rc != RTB_OK)
+    return rc;
+  Dev<char> d_ctr;
+  Dev<unsigned long long> d_totals;
+  RTB_CUDA(cudaMalloc(&d_ctr.p, ctr_one * WF_MAX_GROUPS));
+  RTB_CUDA(cudaMalloc(&d_totals.p, sizeof(unsigned long long) * 8));
+  RTB_CUDA(cudaMemset(d_ctr.p, 0, ctr_one * WF_MAX_GROUPS));
+  RTB_CUDA(cudaMemset(d_totals.p, 0, sizeof(unsigned long long) * 8));
+  A.counters = d_totals.p;
+  const WfQueue q[2] = { pq.q, pq.q };
+  WfGroup G[WF_MAX_GROUPS];
+  wf_groups(A, n_groups, q, slots, d_ctr.p, ctr_one, n_bounces, G);
+  for (int g = 0; g < n_groups; g++)
+    k_wf_generate<<<G[g].gen_blocks, 256>>>(G[g].A, wave, wf_valid_planes(G[g], A, wave), G[g].q[0], &G[g].counts[0]);
+  RTB_CUDA(cudaGetLastError());
+  RTB_CUDA(cudaDeviceSynchronize());
+  size_t n = 0;
+  for (int g = 0; g < n_groups; g++)
+  {
+    unsigned len = 0;
+    RTB_CUDA(cudaMemcpy(&len, G[g].counts, sizeof(unsigned), cudaMemcpyDeviceToHost));
+    rc = wf_probe_read(pq.q, (size_t)G[g].A.plane_base * n_px, len, rays6 + 6 * n, pid + n, throughput3 + 3 * n, branch + n);
+    if (rc != RTB_OK)
+      return rc;
+    n += len;
+  }
+  *n_out = n;
+  return RTB_OK;
+}
+
+extern "C" int rtb_wf_bounce(rtb_scene *scene, const double *camera12, const rtb_render_desc *desc, int wave, int depth,
+                             size_t n_rays, const double *rays6, const uint32_t *pid, const float *throughput3,
+                             const uint32_t *branch_or_null, float *planes4, size_t planes_len, int32_t *ids_or_null,
+                             int64_t *prims_or_null, double *ts_or_null, size_t cap_out, double *rays6_out,
+                             uint32_t *pid_out, float *throughput3_out, uint32_t *branch_out, size_t *n_out,
+                             rtb_counters *counters_or_null)
+{
+  RenderArgs A;
+  WfTraceTune tune;
+  int sm_count = 0;
+  int rc = wf_probe_args("rtb_wf_bounce", scene, camera12, desc, wave, A, tune, sm_count);
+  if (rc != RTB_OK)
+    return rc;
+  const size_t n_px = (size_t)A.width * A.height, slots = n_px * (size_t)A.splits;
+  const bool split = A.dielectric_mode == RTB_DIELECTRIC_SPLIT;
+  auto bad = [](const char *why) {
+    rtb_set_error(std::string("rtb_wf_bounce: ") + why);
+    return RTB_EINVAL;
+  };
+  if (n_rays >= (1ull << 31))
+    return bad("n_rays must stay below 2^31");
+  if ((n_rays && (!rays6 || !pid || !throughput3)) || !planes4 || !rays6_out || !pid_out || !throughput3_out ||
+      !branch_out || !n_out)
+    return bad("NULL argument");
+  if (depth < 0 || depth > A.max_depth)
+    return bad("depth must lie in [0, max_depth]");
+  if (planes_len != 4 * slots)
+    return bad("planes must hold 4 floats per path slot (planes * width * height slots)");
+  if (cap_out < 2 * n_rays)
+    return bad("the output queue must hold two children per ray");
+  if (split && n_rays && !branch_or_null)
+    return bad("the split estimator needs the branch id of every ray");
+  for (size_t i = 0; i < n_rays; i++)
+  {
+    if (pid[i] >= slots)
+      return bad("path slot id beyond planes * width * height");
+    if (branch_or_null && (branch_or_null[i] == 0u || (!split && branch_or_null[i] != 1u)))
+      return bad("branch ids start at 1, and the stochastic estimator carries no other");
+  }
+  const unsigned n = (unsigned)n_rays;
+  const size_t m = n_rays > 0 ? n_rays : 1;
+  WfProbeQueue qin, qout;
+  if ((rc = qin.alloc(n_rays, split)) != RTB_OK || (rc = qout.alloc(2 * n_rays, split)) != RTB_OK)
+    return rc;
+  Dev<double> d_rays, d_ts;
+  Dev<unsigned> d_pid, d_branch, d_ctl; /* d_ctl: queue length in, trace fetch cursor, queue length out, overflow */
+  Dev<float> d_tp;
+  Dev<float4> d_planes;
+  Dev<unsigned long long> d_totals, d_trace_totals;
+  Dev<int2> d_stacks;
+  Dev<int> d_ids;
+  Dev<long long> d_prims;
+  RTB_CUDA(cudaMalloc(&d_rays.p, sizeof(double) * 6 * m));
+  RTB_CUDA(cudaMalloc(&d_pid.p, sizeof(unsigned) * m));
+  RTB_CUDA(cudaMalloc(&d_tp.p, sizeof(float) * 3 * m));
+  RTB_CUDA(cudaMalloc(&d_ctl.p, sizeof(unsigned) * 4));
+  RTB_CUDA(cudaMalloc(&d_planes.p, sizeof(float4) * slots));
+  RTB_CUDA(cudaMalloc(&d_totals.p, sizeof(unsigned long long) * 8));
+  RTB_CUDA(cudaMalloc(&d_trace_totals.p, sizeof(unsigned long long) * 5));
+  RTB_CUDA(cudaMalloc(&d_ids.p, sizeof(int) * m));
+  RTB_CUDA(cudaMalloc(&d_prims.p, sizeof(long long) * m));
+  RTB_CUDA(cudaMalloc(&d_ts.p, sizeof(double) * m));
+  if (branch_or_null)
+    RTB_CUDA(cudaMalloc(&d_branch.p, sizeof(unsigned) * m));
+  if (tune.pool)
+    RTB_CUDA(cudaMalloc(&d_stacks.p, wf_pool_stack_bytes(tune, sm_count)));
+  if (n_rays)
+  {
+    RTB_CUDA(cudaMemcpy(d_rays.p, rays6, sizeof(double) * 6 * n_rays, cudaMemcpyHostToDevice));
+    RTB_CUDA(cudaMemcpy(d_pid.p, pid, sizeof(unsigned) * n_rays, cudaMemcpyHostToDevice));
+    RTB_CUDA(cudaMemcpy(d_tp.p, throughput3, sizeof(float) * 3 * n_rays, cudaMemcpyHostToDevice));
+    if (branch_or_null)
+      RTB_CUDA(cudaMemcpy(d_branch.p, branch_or_null, sizeof(unsigned) * n_rays, cudaMemcpyHostToDevice));
+  }
+  RTB_CUDA(cudaMemcpy(d_planes.p, planes4, sizeof(float4) * slots, cudaMemcpyHostToDevice));
+  const unsigned ctl[4] = { n, 0u, 0u, 0u };
+  RTB_CUDA(cudaMemcpy(d_ctl.p, ctl, sizeof(ctl), cudaMemcpyHostToDevice));
+  RTB_CUDA(cudaMemset(d_totals.p, 0, sizeof(unsigned long long) * 8));
+  RTB_CUDA(cudaMemset(d_trace_totals.p, 0, sizeof(unsigned long long) * 5));
+  A.counters = d_totals.p;
+
+  const unsigned blocks = (unsigned)((m + 127) / 128);
+  k_wf_fill<<<blocks, 128>>>(A.sv, d_rays.p, d_pid.p, d_tp.p, d_branch.p, n, qin.q, d_trace_totals.p);
+  wf_launch_trace(tune, false, sm_count, 0, A.sv, qin.q, d_ctl.p, d_ctl.p + 1, d_trace_totals.p, d_stacks.p, nullptr);
+  if (split)
+    k_wf_shade<true><<<wf_shade_blocks(sm_count), 128>>>(A, wave, depth, qin.q, d_ctl.p, qout.q, d_ctl.p + 2, d_planes.p,
+                                                         nullptr, 0, d_ctl.p + 3);
+  else
+    k_wf_shade<false><<<wf_shade_blocks(sm_count), 128>>>(A, wave, depth, qin.q, d_ctl.p, qout.q, d_ctl.p + 2, d_planes.p,
+                                                          nullptr, 0, nullptr);
+  if (ids_or_null)
+    k_wf_read_hits<<<blocks, 128>>>(A.sv, qin.q, n, d_ids.p, d_prims.p, d_ts.p, nullptr, nullptr, nullptr);
+  RTB_CUDA(cudaGetLastError());
+  RTB_CUDA(cudaDeviceSynchronize());
+
+  unsigned got[4];
+  RTB_CUDA(cudaMemcpy(got, d_ctl.p, sizeof(got), cudaMemcpyDeviceToHost));
+  if (got[3] || got[2] > 2 * n)
+  {
+    rtb_set_error("rtb_wf_bounce: the output queue overflowed");
+    return RTB_ECUDA;
+  }
+  rc = wf_probe_read(qout.q, 0, got[2], rays6_out, pid_out, throughput3_out, branch_out);
+  if (rc != RTB_OK)
+    return rc;
+  *n_out = got[2];
+  RTB_CUDA(cudaMemcpy(planes4, d_planes.p, sizeof(float4) * slots, cudaMemcpyDeviceToHost));
+  if (ids_or_null && n_rays)
+  {
+    RTB_CUDA(cudaMemcpy(ids_or_null, d_ids.p, sizeof(int) * n_rays, cudaMemcpyDeviceToHost));
+    if (prims_or_null) RTB_CUDA(cudaMemcpy(prims_or_null, d_prims.p, sizeof(long long) * n_rays, cudaMemcpyDeviceToHost));
+    if (ts_or_null) RTB_CUDA(cudaMemcpy(ts_or_null, d_ts.p, sizeof(double) * n_rays, cudaMemcpyDeviceToHost));
+  }
+  if (counters_or_null)
+  {
+    unsigned long long h[8];
+    RTB_CUDA(cudaMemcpy(h, d_totals.p, sizeof(h), cudaMemcpyDeviceToHost));
+    memset(counters_or_null, 0, sizeof(*counters_or_null));
+    counters_or_null->rays = h[0];
+    counters_or_null->rays_intersected = h[1];
+    counters_or_null->prim_tests = h[2];
+    counters_or_null->launches = ids_or_null ? 4 : 3;
     counters_or_null->trace_launches = 1;
   }
   return RTB_OK;

@@ -191,6 +191,49 @@ def path_records(scene, cam, width, height, sample, n_vertices=2, dielectric="st
     return out
 
 
+# oracle.h OracleVertex: one vertex of trace_path in forward form
+VERTEX_DTYPE = np.dtype([("ray", "f8", 6), ("tp", "f8", 3), ("contrib", "f8", 3), ("t", "f8"), ("child_ray", "f8", (2, 6)),
+                         ("child_tp", "f8", (2, 3)), ("prim", "i8"), ("pixel", "u4"), ("sample", "u4"), ("branch", "u4"),
+                         ("child_branch", "u4", 2), ("depth", "i4"), ("id", "i4"), ("survived", "i4"), ("rays", "i4"),
+                         ("n_children", "i4"), ("cut", "i4", 2), ("tries", "i4"), ("flipped", "i4")], align=True)
+assert VERTEX_DTYPE.itemsize == 312
+
+
+def path_vertex(scene, rays, depth, branch, pixel, sample, tp, dielectric="stochastic", max_depth=5,
+                seed=abi.SCENE_SEED, threads=None):
+    """one forward vertex of trace_path per ray (oracle_path_vertex), keyed by (pixel, sample, depth | branch << 8),
+    from the incoming throughput `tp` [n, 3] -> VERTEX_DTYPE [n]"""
+    h = _holder(scene)
+    rays = np.ascontiguousarray(rays, np.float64).reshape(-1, 6)
+    n = len(rays)
+    cols = [np.ascontiguousarray(np.broadcast_to(v, (n,)), dt) for v, dt in
+            ((depth, np.int32), (branch, np.uint32), (pixel, np.uint32), (sample, np.uint32))]
+    tp = np.ascontiguousarray(tp, np.float64).reshape(n, 3)
+    out = np.zeros(n, VERTEX_DTYPE)
+    p = params("philox", dielectric, max_depth, seed, 0, threads)
+    oracle().oracle_path_vertex(h.objects, C.c_size_t(h.n), C.byref(p), _dptr(rays), *(_dptr(c) for c in cols), _dptr(tp),
+                                C.c_longlong(n), _dptr(out))
+    return out
+
+
+def path_log(scene, cam, width, height, samples, dielectric="stochastic", max_depth=5, seed=abi.SCENE_SEED,
+             sample_offset=0, threads=None):
+    """every vertex of every path of samples [sample_offset, sample_offset + samples) (oracle_path_log) ->
+    VERTEX_DTYPE [n], rows in order"""
+    h = _holder(scene)
+    p = params("philox", dielectric, max_depth, seed, sample_offset, threads)
+    lib = oracle()
+    lib.oracle_path_log.restype = C.c_longlong
+    cap = width * height * samples * 4
+    while True:
+        out = np.zeros(cap, VERTEX_DTYPE)
+        n = lib.oracle_path_log(h.objects, C.c_size_t(h.n), C.byref(cam), width, height, samples, C.byref(p),
+                                _dptr(out), C.c_longlong(cap))
+        if n <= cap:
+            return out[:n]
+        cap = n
+
+
 def philox(ctr, key):
     ctr = np.ascontiguousarray(ctr, dtype=np.uint32).reshape(-1, 4)
     key = np.ascontiguousarray(key, dtype=np.uint32).reshape(-1, 2)
