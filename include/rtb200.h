@@ -144,6 +144,31 @@ int rtb_scene_create_flags(const void *scene_objects96, size_t n_objects, int de
 int rtb_scene_info_get(const rtb_scene *scene, rtb_scene_info *info);
 void rtb_scene_destroy(rtb_scene *scene);
 
+/* What the build made, for a checker to hold against the caller's geometry (tests/bvh_check.py). */
+typedef struct
+{
+  size_t n_prims;   /* N: primitives in the tree */
+  size_t n_big;     /* oversized spheres, tested for every ray */
+  size_t n_nodes4q; /* compressed BVH4 nodes written */
+  size_t n_nodes4;  /* uncompressed BVH4 nodes (RTB_SCENE_ALL_TREES), else 0 */
+  size_t n_nodes2;  /* BVH2 node slots (N - 1, indexed like the build's binary hierarchy) when the BVH2 exists, else 0 */
+  int root_ref;     /* 0 = node 0; < 0 a leaf, ~ref = (first << 3) | (count - 1); 0x7FFFFFFF when N = 0 */
+  int leaf_max;     /* most primitives per leaf */
+  int depth4;       /* levels of the BVH4 the build emitted */
+  int walks_bvh4;   /* 1: the product path walks the compressed BVH4; 0: the BVH2 (or there is no tree) */
+  int has_tex, has_tri64, has_tex64; /* which of the optional arrays exist */
+  float scene_lo[3], scene_hi[3]; /* min / max of the primitives' float boxes */
+  float guard_lo[3], guard_hi[3], pad, far_t;
+} rtb_scene_tree_info;
+/* Read-out probe (blocking copies to HOST buffers): *info, and those of the arrays below that are not NULL, in the
+ * device layouts of csrc/rtb_internal.h.  Sizes:
+ *   nodes4q 64 B x n_nodes4q; nodes4 128 B x n_nodes4; nodes 64 B x n_nodes2;
+ *   prims 48 B x (N + 1) (BVH order, then the all-zero record empty BVH4 slots refer to; nothing when N = 0);
+ *   big 80 B x n_big (the n_big 48-byte records, then their 32-byte FP32 copies);
+ *   tri64 72 B x (N + 1), tex 24 B x N, tex64 48 B x N, each only when it exists (has_*). */
+int rtb_scene_tree(const rtb_scene *scene, rtb_scene_tree_info *info, void *nodes4q, void *nodes4, void *nodes,
+                   void *prims, void *big, void *tri64, void *tex, void *tex64);
+
 /* A destroyed scene parks its device buffers (scene arrays and the wavefront kernels' ray queues, up
  * to 23.4 GB) in a per-device cache and the next scene reuses them, so that render() -- one scene per
  * call -- allocates nothing in steady state.  This returns everything cached for `device` to the driver. */

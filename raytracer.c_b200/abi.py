@@ -115,6 +115,14 @@ class RtbSceneInfo(C.Structure):
                 ("bvh4_depth", C.c_int)]
 
 
+class RtbSceneTreeInfo(C.Structure):
+    _fields_ = [("n_prims", C.c_size_t), ("n_big", C.c_size_t), ("n_nodes4q", C.c_size_t), ("n_nodes4", C.c_size_t),
+                ("n_nodes2", C.c_size_t), ("root_ref", C.c_int), ("leaf_max", C.c_int), ("depth4", C.c_int),
+                ("walks_bvh4", C.c_int), ("has_tex", C.c_int), ("has_tri64", C.c_int), ("has_tex64", C.c_int),
+                ("scene_lo", C.c_float * 3), ("scene_hi", C.c_float * 3), ("guard_lo", C.c_float * 3),
+                ("guard_hi", C.c_float * 3), ("pad", C.c_float), ("far_t", C.c_float)]
+
+
 EXPECTED_SIZES = {Vertex: 40, Material: 80, Sphere: 32, TriangleMesh: 16, Object: 88,
                   SceneObject: 96, Camera: 96, Options: 56}
 for _t, _n in EXPECTED_SIZES.items():

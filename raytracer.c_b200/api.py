@@ -25,7 +25,7 @@ RTB_SYMBOLS = [
     "rtb_trace_rays", "rtb_trace_rays_wf", "rtb_path_records", "rtb_philox4x32_10", "rtb_probe_l2_bandwidth", "rtb_cast_rays",
     "rtb_probe_fp32_tflops", "rtb_render_mean", "rtb_comm_unique_id", "rtb_comm_create_rank", "rtb_comm_create_local", "rtb_comm_size",
     "rtb_warm_up", "rtb_comm_local_ranks", "rtb_comm_destroy", "rtb_comm_shard_samples", "rtb_comm_scene_create", "rtb_comm_render", "rtb_render_multi",
-    "rtb_render_aov", "rtb_render_aov_host", "rtb_wf_generate", "rtb_wf_bounce",
+    "rtb_render_aov", "rtb_render_aov_host", "rtb_wf_generate", "rtb_wf_bounce", "rtb_scene_tree",
 ]
 # the reference's exported surface (raytracer.h:135-164) plus the documented extensions
 HOST_SYMBOLS = [
@@ -72,6 +72,7 @@ def _bind(cu, host):
     cu.rtb_scene_create_objects_flags.argtypes = [C.c_void_p, C.c_size_t, C.c_int, C.c_uint, C.POINTER(C.c_void_p)]
     cu.rtb_scene_create_flags.argtypes = [C.c_void_p, C.c_size_t, C.c_int, C.c_uint, C.POINTER(C.c_void_p)]
     cu.rtb_scene_info_get.argtypes = [C.c_void_p, C.POINTER(abi.RtbSceneInfo)]
+    cu.rtb_scene_tree.argtypes = [C.c_void_p, C.POINTER(abi.RtbSceneTreeInfo)] + [C.c_void_p] * 8
     cu.rtb_scene_destroy.argtypes = [C.c_void_p]
     cu.rtb_scene_destroy.restype = None
     cu.rtb_render_accum.argtypes = [C.c_void_p, dp, C.POINTER(abi.RtbRenderDesc), C.c_void_p, C.c_void_p,
@@ -379,6 +380,28 @@ class Scene:
         i = abi.RtbSceneInfo()
         _check(self._cu.rtb_scene_info_get(self._h, C.byref(i)), "rtb_scene_info_get")
         return i
+
+    def tree(self):
+        """the build's arrays as the device holds them (rtb_scene_tree) -> dict: `info` (abi.RtbSceneTreeInfo);
+        nodes4q uint32 [n, 16], nodes4 uint32 [n, 32], nodes uint32 [n, 16], prims uint32 [N + 1, 12] (raw words of
+        the float4 layouts, rtb_internal.h); big uint32 [n_big, 12] records and big_fp32 float32 [n_big, 8] copies;
+        tri64 float64 [N + 1, 9], tex float32 [N, 6], tex64 float64 [N, 6] or None where the scene has none"""
+        info = abi.RtbSceneTreeInfo()
+        _check(self._cu.rtb_scene_tree(self._h, C.byref(info), *([None] * 8)), "rtb_scene_tree")
+        N = info.n_prims
+        out = dict(info=info, nodes4q=np.zeros((info.n_nodes4q, 16), np.uint32),
+                   nodes4=np.zeros((info.n_nodes4, 32), np.uint32), nodes=np.zeros((info.n_nodes2, 16), np.uint32),
+                   prims=np.zeros((N + 1 if N else 0, 12), np.uint32), big=np.zeros(info.n_big * 20, np.uint32),
+                   tri64=np.zeros((N + 1, 9)) if info.has_tri64 else None,
+                   tex=np.zeros((N, 6), np.float32) if info.has_tex else None,
+                   tex64=np.zeros((N, 6)) if info.has_tex64 else None)
+        keys = ("nodes4q", "nodes4", "nodes", "prims", "big", "tri64", "tex", "tex64")
+        _check(self._cu.rtb_scene_tree(self._h, C.byref(info), *(out[k].ctypes.data if out[k] is not None else None
+                                                                for k in keys)), "rtb_scene_tree")
+        big = out.pop("big")
+        out["big"] = big[:12 * info.n_big].reshape(-1, 12)
+        out["big_fp32"] = big[12 * info.n_big:].view(np.float32).reshape(-1, 8)
+        return out
 
     def render_accum(self, camera, desc, d_accum_ptr, stream=None, want_counters=False):
         """device float[H*W*3] sum; asynchronous on `stream` unless counters are wanted"""

@@ -71,10 +71,10 @@ struct Bvh4Node { float4 q[8]; };
 /* Compressed BVH4 node, 64 bytes (two 256-bit loads): child boxes quantised to 8 bits per
  * coordinate on a per-node grid (origin + q * 2^e per axis, after Ylitie et al. 2017); lo is
  * rounded down and hi up, so a decoded box always contains the padded float box.
- *   w0 = {origin.x, origin.y, origin.z, ex | ey << 8 | ez << 16}   e = IEEE-754 exponent byte of the cell size
- *   w1 = child references (int bits, RTB_REF_NONE = empty slot)
+ *   w0 = {origin.x, origin.y, origin.z, cell.x}                    cell = a power of two in the normal float range
+ *   w1 = child references (int bits; an empty slot refers to the one-primitive leaf at N, an all-zero record)
  *   w2 = {qlo.x[0..3], qlo.y[0..3], qlo.z[0..3], qhi.x[0..3]}      one byte per child
- *   w3 = {qhi.y[0..3], qhi.z[0..3], -, -}
+ *   w3 = {qhi.y[0..3], qhi.z[0..3], cell.y, cell.z}
  * The L1 data pipe is the bound of the walk (one wavefront per 32-byte sector a lane touches):
  * this node costs 2 wavefronts per visit instead of 4 (Bvh4Node) or 2 x 2 (two BvhNode). */
 struct Bvh4QNode { float4 w[4]; };
@@ -122,6 +122,7 @@ struct rtb_scene
   size_t wf_bytes = 0;
   unsigned long long *d_counters = nullptr;
   rtb_scene_info info{};
+  rtb_scene_tree_info tree{}; /* what rtb_scene_tree reports besides the arrays */
   std::vector<std::pair<void *, size_t>> owned; /* every device buffer of the scene arrays, with its size */
 };
 

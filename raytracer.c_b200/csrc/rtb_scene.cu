@@ -111,7 +111,7 @@ __global__ void k_marshal_tris(const RefVertex *__restrict__ verts, int n_tris, 
   /* 3 vertices x 5 doubles, contiguous */
   float v[3][3], t[3][2];
   float lo[3] = { FLT_MAX, FLT_MAX, FLT_MAX }, hi[3] = { -FLT_MAX, -FLT_MAX, -FLT_MAX };
-  bool exact = true, tex_exact = true;
+  bool exact = true, tex_exact = true, nan = false;
 #pragma unroll
   for (int k = 0; k < 3; k++)
   {
@@ -121,6 +121,7 @@ __global__ void k_marshal_tris(const RefVertex *__restrict__ verts, int n_tris, 
       const double x = p[5 * k + a];
       v[k][a] = __double2float_rn(x);
       exact = exact && ((double)v[k][a] == x);
+      nan = nan || isnan(x);
       lo[a] = fminf(lo[a], __double2float_rd(x)); /* the box contains the double triangle */
       hi[a] = fmaxf(hi[a], __double2float_ru(x));
       if (tri64)
@@ -141,6 +142,8 @@ __global__ void k_marshal_tris(const RefVertex *__restrict__ verts, int n_tris, 
     inexact[0] = 1;
   if (!tex_exact && inexact)
     inexact[1] = 1;
+  if (nan) /* fminf above drops a NaN: put it back into the box, where k_bounds reports it */
+    lo[0] = __int_as_float(0x7FC00000);
   PrimRec r;
   r.a = make_float4(v[0][0], v[0][1], v[0][2], v[1][0]);
   r.b = make_float4(v[1][1], v[1][2], v[2][0], v[2][1]);
@@ -233,17 +236,21 @@ __device__ __forceinline__ unsigned float_to_ordered(float f)
   return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
 }
 
-/* bounds[0..2] = min of box_lo, bounds[3..5] = max of box_hi (ordered-uint encoded) */
+/* bounds[0..2] = min of box_lo, bounds[3..5] = max of box_hi (ordered-uint encoded).  fminf / fmaxf drop NaN, so a
+ * NaN in any box is reported separately: bounds[3] becomes +inf, which k_build_params rejects as non-finite. */
 __global__ void k_bounds(const float4 *__restrict__ box_lo, const float4 *__restrict__ box_hi, int n,
                          unsigned *__restrict__ bounds)
 {
   float lo[3] = { FLT_MAX, FLT_MAX, FLT_MAX }, hi[3] = { -FLT_MAX, -FLT_MAX, -FLT_MAX };
+  bool nan = false;
   for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x)
   {
     float4 a = box_lo[i], b = box_hi[i];
     lo[0] = fminf(lo[0], a.x); lo[1] = fminf(lo[1], a.y); lo[2] = fminf(lo[2], a.z);
     hi[0] = fmaxf(hi[0], b.x); hi[1] = fmaxf(hi[1], b.y); hi[2] = fmaxf(hi[2], b.z);
+    nan = nan || isnan(a.x) || isnan(a.y) || isnan(a.z) || isnan(b.x) || isnan(b.y) || isnan(b.z);
   }
+  nan = __any_sync(0xFFFFFFFFu, nan);
 #pragma unroll
   for (int k = 0; k < 3; k++)
   {
@@ -261,6 +268,8 @@ __global__ void k_bounds(const float4 *__restrict__ box_lo, const float4 *__rest
       atomicMin(&bounds[k], float_to_ordered(lo[k]));
       atomicMax(&bounds[3 + k], float_to_ordered(hi[k]));
     }
+    if (nan)
+      atomicMax(&bounds[3], float_to_ordered(INFINITY));
   }
 }
 
@@ -1130,6 +1139,13 @@ int build_scene(HostScene &hs, int device, unsigned flags, const rtb_scene_shard
   int leaf_max = hs.meshes.empty() ? 1 : 2;
   if (const char *e = getenv("RTB_LEAF_MAX"))
     leaf_max = std::max(1, std::min(8, atoi(e)));
+  /* NaN would break choose_big's ordering (a NaN radius is a candidate); triangles are checked on the device */
+  for (const SphereIn &s : hs.spheres)
+    if (std::isnan(s.cx) || std::isnan(s.cy) || std::isnan(s.cz) || std::isnan(s.r))
+    {
+      rtb_set_error("non-finite geometry");
+      return RTB_EINVAL;
+    }
   std::vector<char> big = choose_big(hs);
   std::vector<SphereIn> big_spheres, bvh_spheres;
   for (size_t i = 0; i < hs.spheres.size(); i++)
@@ -1216,6 +1232,7 @@ int build_scene(HostScene &hs, int device, unsigned flags, const rtb_scene_shard
   int &h_nodes4 = rb.nodes4;
   bool bvh4_ok = true;
   int depth4 = 0; /* levels of the BVH4 */
+  int emitted_levels = 0; /* BVH4 levels k_emit4 ran for */
 
   if (N > 0)
   {
@@ -1422,6 +1439,7 @@ int build_scene(HostScene &hs, int device, unsigned flags, const rtb_scene_shard
         /* (a tree over N primitives has fewer than N levels: small scenes skip the empty launches; a BVH4 deeper
          * than (RTB_STACK_SIZE - 2) / 3 levels is not walked anyway -- see bvh4_ok below -- so it is not finished) */
         const int max_levels = (int)std::min<size_t>((RTB_STACK_SIZE - 2) / 3 + 2, N);
+        emitted_levels = max_levels;
         for (int level = 0; level < max_levels; level++)
           k_emit4<<<half_blocks, T>>>(d_vals_sorted.p, d_lo.p, d_hi.p, (int)N, d_children.p, d_first.p, d_node_lo.p,
                                       d_node_hi.p, d_bp.p, sc->d_nodes4, sc->d_nodes4q, eq, level, leaf_max,
@@ -1547,7 +1565,6 @@ int build_scene(HostScene &hs, int device, unsigned flags, const rtb_scene_shard
       view.far_t = (float)std::max(far, 0.0);
     }
     bvh_depth = h_misc[0];
-    n_nodes = (size_t)h_nodes4; /* nodes of the tree the default path walks */
     while (depth4 < RTB_STACK_SIZE && h_levels[depth4] > 0)
       depth4++;
     /* the BVH2 walk pushes at most one entry per level, the BVH4 walk at most three */
@@ -1561,7 +1578,11 @@ int build_scene(HostScene &hs, int device, unsigned flags, const rtb_scene_shard
     bvh4_ok = 3 * depth4 <= RTB_STACK_SIZE - 2;
     if (!bvh4_ok && !all_trees)
       return build_scene(hs, device, flags | RTB_SCENE_ALL_TREES, shard, out); /* rare: build the BVH2 as well */
+    n_nodes = (size_t)(bvh4_ok ? h_nodes4 : h_misc[1]); /* nodes of the tree the default path walks */
   }
+  size_t nodes4_written = 0; /* a fallback scene's BVH4 stops after emitted_levels levels */
+  for (int l = 0; l < emitted_levels; l++)
+    nodes4_written += (size_t)h_levels[l];
 
   view.nodes = sc->d_nodes;
   view.nodes4 = bvh4_ok ? sc->d_nodes4 : nullptr;
@@ -1587,6 +1608,29 @@ int build_scene(HostScene &hs, int device, unsigned flags, const rtb_scene_shard
   sc->info.double_triangles = h_inexact ? 1 : 0;
   sc->info.double_texcoords = h_tex_inexact ? 1 : 0;
   sc->info.bvh4_depth = view.nodes4q != nullptr ? depth4 : 0;
+
+  rtb_scene_tree_info &t = sc->tree;
+  t.n_prims = N;
+  t.n_big = big_spheres.size();
+  t.n_nodes4q = nodes4_written;
+  t.n_nodes4 = sc->d_nodes4 ? nodes4_written : 0;
+  t.n_nodes2 = all_trees && (int)N > leaf_max ? N - 1 : 0;
+  t.root_ref = view.root_ref;
+  t.leaf_max = leaf_max;
+  t.depth4 = depth4;
+  t.walks_bvh4 = view.nodes4q != nullptr ? 1 : 0;
+  t.has_tex = sc->d_tex != nullptr;
+  t.has_tri64 = sc->d_tri64 != nullptr;
+  t.has_tex64 = sc->d_tex64 != nullptr;
+  for (int k = 0; k < 3; k++)
+  {
+    t.scene_lo[k] = N > 0 ? h_bp.lo[k] : 0.0f;
+    t.scene_hi[k] = N > 0 ? h_bp.hi[k] : 0.0f;
+    t.guard_lo[k] = view.guard_lo[k];
+    t.guard_hi[k] = view.guard_hi[k];
+  }
+  t.pad = N > 0 ? h_bp.pad : 0.0f;
+  t.far_t = view.far_t;
   *out = sc.release();
   return RTB_OK;
 }
@@ -1688,6 +1732,34 @@ extern "C" int rtb_scene_info_get(const rtb_scene *scene, rtb_scene_info *info)
     return RTB_EINVAL;
   }
   *info = scene->info;
+  return RTB_OK;
+}
+
+extern "C" int rtb_scene_tree(const rtb_scene *scene, rtb_scene_tree_info *info, void *nodes4q, void *nodes4, void *nodes,
+                              void *prims, void *big, void *tri64, void *tex, void *tex64)
+{
+  if (!scene || !info)
+  {
+    rtb_set_error("rtb_scene_tree: NULL argument");
+    return RTB_EINVAL;
+  }
+  const rtb_scene_tree_info &t = scene->tree;
+  *info = t;
+  const size_t N = t.n_prims;
+  const struct { void *dst; const void *src; size_t bytes; } copies[] = {
+    { nodes4q, scene->d_nodes4q, sizeof(Bvh4QNode) * t.n_nodes4q },
+    { nodes4, scene->d_nodes4, sizeof(Bvh4Node) * t.n_nodes4 },
+    { nodes, scene->d_nodes, sizeof(BvhNode) * t.n_nodes2 },
+    { prims, scene->d_prims, N ? sizeof(PrimRec) * (N + 1) : 0 },
+    { big, scene->d_big, (sizeof(PrimRec) + 2 * sizeof(float4)) * t.n_big },
+    { tri64, scene->d_tri64, t.has_tri64 ? sizeof(double) * 9 * (N + 1) : 0 },
+    { tex, scene->d_tex, t.has_tex ? sizeof(float2) * 3 * N : 0 },
+    { tex64, scene->d_tex64, t.has_tex64 ? sizeof(double) * 6 * N : 0 },
+  };
+  RTB_CUDA(cudaSetDevice(scene->device));
+  for (const auto &c : copies)
+    if (c.dst && c.bytes)
+      RTB_CUDA(cudaMemcpy(c.dst, c.src, c.bytes, cudaMemcpyDeviceToHost));
   return RTB_OK;
 }
 
