@@ -238,6 +238,28 @@ void render_ex_aov(uint8_t *framebuffer, Object *objects, size_t n_objects, Came
 void render_scene_aov(uint8_t *framebuffer, SceneObject *objects, size_t n_objects, Camera *camera, Options *options,
                       const RenderParams *params, const RenderAov *aov);
 
+/* Built-in denoiser (rtb_denoise in rtb200.h, DESIGN.md section 4.6): an edge-avoiding a-trous filter guided by the
+ * frame's first-hit feature buffers.  A field 0 takes the library's default; iterations < 0 turns the filter off. */
+typedef struct
+{
+  int iterations;        /* a-trous passes, default 5 */
+  float sigma_luminance; /* default 48 */
+  float sigma_normal;    /* default 128 */
+  float sigma_depth;     /* default 0.1 */
+  float albedo_epsilon;  /* default 1e-3 */
+} DenoiseParams;
+
+/* fills the library's defaults */
+void denoise_params_default(DenoiseParams *p);
+
+/* render_ex_aov / render_scene_aov whose framebuffer gets the DENOISED frame (the denoised mean through the
+ * reference's transfer); params->accum_out still gets the raw sums, the same bits as without denoising, and `aov`
+ * (may be NULL) the feature means.  `dn` NULL = defaults.  Single GPU only (num_gpus == 1). */
+void render_ex_denoised(uint8_t *framebuffer, Object *objects, size_t n_objects, Camera *camera, Options *options,
+                        const RenderParams *params, const RenderAov *aov, const DenoiseParams *dn);
+void render_scene_denoised(uint8_t *framebuffer, SceneObject *objects, size_t n_objects, Camera *camera,
+                           Options *options, const RenderParams *params, const RenderAov *aov, const DenoiseParams *dn);
+
 /* Optional: starts creating the CUDA context(s) a later render*() with these parameters will use (NULL = defaults)
  * on a background thread and returns at once.  A driver calls it first and then reads its scene -- the reference's
  * main.c:413-429 builds the scene between allocating the frame and calling render() -- so that driver start-up

@@ -16,6 +16,10 @@
  *   rtb_render             the whole of render() (raytracer.c:176-223), host buffers in/out
  *   rtb_render_aov         no reference counterpart: first-hit feature buffers (albedo, normal, depth, hit count,
  *                          object id) of the render's own camera samples, the inputs of a denoiser or a compositor
+ *   rtb_denoise            no reference counterpart: edge-avoiding a-trous denoiser of a frame's sums, guided by the
+ *                          feature buffers of rtb_render_aov
+ *   rtb_render_denoised    render() + feature pass + denoiser + tonemap of the denoised mean, host buffers out
+ *                          (rtb_render_denoised_aov: also the feature sums)
  *   rtb_trace_rays         intersect() for arbitrary rays (raytracer.c:393-464): parity probe
  *   rtb_trace_rays_wf      the same records from the wavefront renderer's trace kernel: parity probe
  *   rtb_wf_generate, rtb_wf_bounce   the wavefront renderer's camera-ray and shade kernels, one launch at a time
@@ -210,6 +214,45 @@ int rtb_render_aov(rtb_scene *scene, const double *camera12, const rtb_render_de
 int rtb_render_aov_host(rtb_scene *scene, const double *camera12, const rtb_render_desc *desc,
                         float *albedo3, float *normal3, float *depth, uint32_t *hits, int32_t *object,
                         rtb_counters *counters);
+
+/* Denoiser: edge-avoiding a-trous filter (Dammertz et al. 2010) with SVGF's variance-guided weights (Schied et al.
+ * 2017, spatial part only), DESIGN.md section 4.6.  A field 0 (or a NULL desc) takes the default below. */
+typedef struct
+{
+  int iterations;        /* a-trous passes (steps 1, 2, 4, ...); < 0: no filtering, the output is accum / total_samples;
+                            2^(iterations - 1) must be below the frame's smaller side */
+  float sigma_luminance; /* luminance term exp(-|l_p - l_q| / (sigma_luminance sqrt(var_p) + tiny)) */
+  float sigma_normal;    /* normal term max(0, n_p . n_q)^sigma_normal */
+  float sigma_depth;     /* depth term exp(-|z_p - z_q| / (sigma_depth z_p |offset| + tiny)) */
+  float albedo_epsilon;  /* the colour is filtered as colour / max(albedo, albedo_epsilon) and multiplied back */
+} rtb_denoise_desc;
+#define RTB_DENOISE_DEFAULT_ITERATIONS 5
+#define RTB_DENOISE_DEFAULT_SIGMA_LUMINANCE 48.0f
+#define RTB_DENOISE_DEFAULT_SIGMA_NORMAL 128.0f
+#define RTB_DENOISE_DEFAULT_SIGMA_DEPTH 0.1f
+#define RTB_DENOISE_DEFAULT_ALBEDO_EPSILON 1e-3f
+/* d_out3: DEVICE float[height*width*3], the denoised MEAN radiance of a frame, from the SUMS of rtb_render_accum
+ * (d_accum3) and rtb_render_aov (the other inputs) over total_samples samples; the means (colour, albedo, normal /
+ * total_samples, depth / hits) are formed on the device.  d_out3 must not overlap an input.  Pixels of different
+ * object ids never contribute to each other.  Asynchronous on `stream`; scratch (64 B per pixel) comes from the
+ * stream-ordered pool.  RTB_EINVAL: a NULL buffer, width or height < 2, total_samples <= 0, a negative or non-finite
+ * sigma, or more passes than the frame can use. */
+int rtb_denoise(const rtb_denoise_desc *dn, int width, int height, int total_samples, const float *d_accum3,
+                const float *d_albedo3, const float *d_normal3, const float *d_depth, const uint32_t *d_hits,
+                const int32_t *d_object, float *d_out3, int device, void *stream);
+/* render (rtb_render_accum) + feature pass (rtb_render_aov) + rtb_denoise + rtb_tonemap of the denoised mean (total
+ * samples 1), all on the device; HOST buffers out (blocking): framebuffer u8[H*W*3]; denoised3_or_null the denoised
+ * mean; accum_or_null the raw sums, the very bits rtb_render_mean returns.  counters: the render's.  dn_or_null: NULL
+ * = defaults. */
+int rtb_render_denoised(rtb_scene *scene, const double *camera12, const rtb_render_desc *desc, int total_samples,
+                        const rtb_denoise_desc *dn_or_null, uint8_t *framebuffer, float *denoised3_or_null,
+                        float *accum_or_null, rtb_counters *counters);
+/* the same, and the feature sums the filter used (rtb_render_aov's for desc, HOST buffers, each may be NULL), so that
+ * a caller who wants the frame's feature buffers too does not run the feature pass twice */
+int rtb_render_denoised_aov(rtb_scene *scene, const double *camera12, const rtb_render_desc *desc, int total_samples,
+                            const rtb_denoise_desc *dn_or_null, uint8_t *framebuffer, float *denoised3_or_null,
+                            float *accum_or_null, float *albedo3_or_null, float *normal3_or_null, float *depth_or_null,
+                            uint32_t *hits_or_null, int32_t *object_or_null, rtb_counters *counters);
 
 /* parity probes (host buffers) */
 int rtb_trace_rays(rtb_scene *scene, const double *rays6, size_t n_rays, int use_bvh, int32_t *ids,

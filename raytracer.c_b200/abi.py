@@ -88,6 +88,16 @@ class RenderAov(C.Structure):
                 ("object", C.POINTER(C.c_int32))]
 
 
+class DenoiseParams(C.Structure):
+    """DenoiseParams of raytracer.h and rtb_denoise_desc of rtb200.h (same layout): a field 0 takes the default,
+    iterations < 0 turns the filter off"""
+    _fields_ = [("iterations", C.c_int), ("sigma_luminance", C.c_float), ("sigma_normal", C.c_float),
+                ("sigma_depth", C.c_float), ("albedo_epsilon", C.c_float)]
+
+
+RtbDenoiseDesc = DenoiseParams
+
+
 class SceneMix(C.Structure):
     _fields_ = [("emissive", C.c_double), ("refraction", C.c_double), ("reflection", C.c_double)]
 

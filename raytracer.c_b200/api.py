@@ -26,6 +26,7 @@ RTB_SYMBOLS = [
     "rtb_probe_fp32_tflops", "rtb_render_mean", "rtb_comm_unique_id", "rtb_comm_create_rank", "rtb_comm_create_local", "rtb_comm_size",
     "rtb_warm_up", "rtb_comm_local_ranks", "rtb_comm_destroy", "rtb_comm_shard_samples", "rtb_comm_scene_create", "rtb_comm_render", "rtb_render_multi",
     "rtb_render_aov", "rtb_render_aov_host", "rtb_wf_generate", "rtb_wf_bounce", "rtb_scene_tree",
+    "rtb_denoise", "rtb_render_denoised", "rtb_render_denoised_aov",
 ]
 # the reference's exported surface (raytracer.h:135-164) plus the documented extensions
 HOST_SYMBOLS = [
@@ -36,6 +37,7 @@ HOST_SYMBOLS = [
     "scene_default", "scene_room_walls", "scene_random_spheres", "scene_sphere_field",
     "scene_heightfield_mesh", "scene_write_obj", "scene_mesh_room", "scene_from_objects", "rt_write_png",
     "render_ex_aov", "render_scene_aov", "rt_write_pfm",
+    "denoise_params_default", "render_ex_denoised", "render_scene_denoised",
 ]
 
 
@@ -109,6 +111,14 @@ def _bind(cu, host):
         C.POINTER(abi.RtbCounters)]
     cu.rtb_render_aov_host.argtypes = [C.c_void_p, dp, C.POINTER(abi.RtbRenderDesc)] + [C.c_void_p] * 5 + [
         C.POINTER(abi.RtbCounters)]
+    cu.rtb_denoise.argtypes = [C.POINTER(abi.RtbDenoiseDesc), C.c_int, C.c_int, C.c_int] + [C.c_void_p] * 7 + [
+        C.c_int, C.c_void_p]
+    cu.rtb_render_denoised.argtypes = [C.c_void_p, dp, C.POINTER(abi.RtbRenderDesc), C.c_int,
+                                       C.POINTER(abi.RtbDenoiseDesc), C.c_void_p, C.c_void_p, C.c_void_p,
+                                       C.POINTER(abi.RtbCounters)]
+    cu.rtb_render_denoised_aov.argtypes = [C.c_void_p, dp, C.POINTER(abi.RtbRenderDesc), C.c_int,
+                                           C.POINTER(abi.RtbDenoiseDesc)] + [C.c_void_p] * 8 + [
+        C.POINTER(abi.RtbCounters)]
 
     host.init_camera.argtypes = [C.POINTER(abi.Camera), abi.Vec3, abi.Vec3, C.POINTER(abi.Options)]
     host.init_camera.restype = None
@@ -122,6 +132,12 @@ def _bind(cu, host):
     host.render_ex_aov.restype = None
     host.render_scene_aov.argtypes = host.render_ex_aov.argtypes
     host.render_scene_aov.restype = None
+    host.render_ex_denoised.argtypes = host.render_ex_aov.argtypes + [C.POINTER(abi.DenoiseParams)]
+    host.render_ex_denoised.restype = None
+    host.render_scene_denoised.argtypes = host.render_ex_denoised.argtypes
+    host.render_scene_denoised.restype = None
+    host.denoise_params_default.argtypes = [C.POINTER(abi.DenoiseParams)]
+    host.denoise_params_default.restype = None
     host.render_params_default.argtypes = [C.POINTER(abi.RenderParams)]
     host.render_params_default.restype = None
     host.load_obj.argtypes = [C.c_char_p, C.POINTER(abi.TriangleMesh)]
@@ -284,6 +300,44 @@ def render_scene_aov(holder, camera, width, height, samples, params=None):
     host.render_scene_aov(fb.ctypes.data, C.addressof(holder.objects), holder.n, C.byref(camera), C.byref(opt),
                           C.byref(params), C.byref(aov))
     return fb, out
+
+
+def denoise_params(iterations=0, sigma_luminance=0.0, sigma_normal=0.0, sigma_depth=0.0, albedo_epsilon=0.0):
+    """an abi.DenoiseParams (= rtb_denoise_desc); 0 = the library's default, iterations < 0 = no filtering"""
+    return abi.DenoiseParams(iterations, sigma_luminance, sigma_normal, sigma_depth, albedo_epsilon)
+
+
+def render_scene_denoised(holder, camera, width, height, samples, params=None, dn=None, want_aov=False):
+    """render_scene_denoised (raytracer.h): the DENOISED frame of render_scene with these parameters -> framebuffer
+    u8 [H, W, 3], and with want_aov also the feature means as render_scene_aov returns them (-> (fb, dict)).
+    params.accum_out (if set) gets the raw sums.  `dn`: abi.DenoiseParams, None = defaults."""
+    _, host = load()
+    if params is None:
+        params = abi.RenderParams()
+        host.render_params_default(C.byref(params))
+    fb = np.zeros((height, width, 3), dtype=np.uint8)
+    out = aov = None
+    if want_aov:
+        out = dict(albedo=np.zeros((height, width, 3), np.float32), normal=np.zeros((height, width, 3), np.float32),
+                   depth=np.zeros((height, width), np.float32), object=np.zeros((height, width), np.int32))
+        aov = abi.RenderAov(*(out[k].ctypes.data_as(C.POINTER(C.c_float)) for k in ("albedo", "normal", "depth")),
+                            out["object"].ctypes.data_as(C.POINTER(C.c_int32)))
+    opt = abi.Options()
+    opt.width, opt.height, opt.samples = width, height, samples
+    host.render_scene_denoised(fb.ctypes.data, C.addressof(holder.objects), holder.n, C.byref(camera), C.byref(opt),
+                               C.byref(params), C.byref(aov) if aov is not None else None,
+                               C.byref(dn) if dn is not None else None)
+    return (fb, out) if want_aov else fb
+
+
+def denoise(width, height, total_samples, d_accum, d_albedo, d_normal, d_depth, d_hits, d_object, d_out, dn=None,
+            device=0, stream=None):
+    """rtb_denoise on DEVICE pointers (the sums of Scene.render_accum and Scene.render_aov_accum): d_out gets the
+    denoised mean float[H*W*3].  Asynchronous on `stream`."""
+    cu, _ = load()
+    _check(cu.rtb_denoise(C.byref(dn) if dn is not None else None, width, height, total_samples,
+                          *(C.c_void_p(p) for p in (d_accum, d_albedo, d_normal, d_depth, d_hits, d_object, d_out)),
+                          device, C.c_void_p(stream or 0)), "rtb_denoise")
 
 
 def render(objects, camera, width, height, samples):
@@ -449,6 +503,25 @@ class Scene:
                                    fb.ctypes.data, acc.ctypes.data if want_accum else None, C.byref(ctr)),
                "rtb_render")
         return fb, acc, ctr
+
+    def render_denoised(self, camera, desc, total_samples=None, dn=None, want_accum=False, want_denoised=True):
+        """rtb_render_denoised: render + feature pass + denoiser on the device -> (framebuffer u8 [H, W, 3] of the
+        denoised mean, denoised mean f32 [H, W, 3] or None, raw sums f32 [H, W, 3] or None, abi.RtbCounters of the
+        render).  total_samples: divisor of the means (None = the desc's sample count); dn: abi.DenoiseParams,
+        None = defaults"""
+        cam = camera.as_array()
+        if total_samples is None:
+            total_samples = max(1, desc.sample_end - desc.sample_begin)
+        fb = np.zeros((desc.height, desc.width, 3), dtype=np.uint8)
+        out = np.zeros((desc.height, desc.width, 3), dtype=np.float32) if want_denoised else None
+        acc = np.zeros((desc.height, desc.width, 3), dtype=np.float32) if want_accum else None
+        ctr = abi.RtbCounters()
+        _check(self._cu.rtb_render_denoised(self._h, cam.ctypes.data_as(C.POINTER(C.c_double)), C.byref(desc),
+                                            int(total_samples), C.byref(dn) if dn is not None else None,
+                                            fb.ctypes.data, out.ctypes.data if want_denoised else None,
+                                            acc.ctypes.data if want_accum else None,
+                                            C.byref(ctr)), "rtb_render_denoised")
+        return fb, out, acc, ctr
 
     def trace_rays(self, rays, use_bvh=True):
         rays = np.ascontiguousarray(rays, dtype=np.float64).reshape(-1, 6)

@@ -116,40 +116,6 @@ __global__ void __launch_bounds__(128, 1) k_render_aov(const __grid_constant__ R
   }
 }
 
-namespace
-{
-/* stream-ordered pool allocations of one call, returned on every path (the AOV pass never touches the scene's own
- * scratch, so it cannot disturb a render of the same scene) */
-struct PoolBufs
-{
-  cudaStream_t stream = nullptr;
-  void *p[8] = {};
-  int n = 0;
-  cudaError_t alloc(void **out, size_t bytes)
-  {
-    cudaError_t e = cudaMallocAsync(out, bytes, stream);
-    if (e == cudaSuccess)
-      p[n++] = *out;
-    return e;
-  }
-  ~PoolBufs()
-  {
-    for (int k = 0; k < n; k++)
-      cudaFreeAsync(p[k], stream);
-  }
-};
-
-struct Events
-{
-  cudaEvent_t a = nullptr, b = nullptr;
-  ~Events()
-  {
-    if (a) cudaEventDestroy(a);
-    if (b) cudaEventDestroy(b);
-  }
-};
-} // namespace
-
 extern "C" int rtb_render_aov(rtb_scene *scene, const double *camera12, const rtb_render_desc *desc, float *d_albedo3,
                               float *d_normal3, float *d_depth, uint32_t *d_hits, int32_t *d_object, void *stream_,
                               rtb_counters *counters)

@@ -164,6 +164,38 @@ int rtb_plane_split(long long want_threads, size_t n_px, int planes, int spp, in
 /* out[i] = sum over k < splits of planes[k * n + i], in float, in plane order (k_sum_planes), on `stream` */
 int rtb_sum_planes(const float *planes, int splits, size_t n, float *out, cudaStream_t stream);
 
+/* stream-ordered pool allocations of one call, returned on every path (the feature pass and the denoiser never touch
+ * the scene's own scratch, so they cannot disturb a render of the same scene) */
+struct PoolBufs
+{
+  cudaStream_t stream = nullptr;
+  void *p[8] = {};
+  int n = 0;
+  cudaError_t alloc(void **out, size_t bytes)
+  {
+    cudaError_t e = cudaMallocAsync(out, bytes, stream);
+    if (e == cudaSuccess)
+      p[n++] = *out;
+    return e;
+  }
+  ~PoolBufs()
+  {
+    for (int k = 0; k < n; k++)
+      cudaFreeAsync(p[k], stream);
+  }
+};
+
+/* a pair of CUDA events, destroyed on every return path */
+struct Events
+{
+  cudaEvent_t a = nullptr, b = nullptr;
+  ~Events()
+  {
+    if (a) cudaEventDestroy(a);
+    if (b) cudaEventDestroy(b);
+  }
+};
+
 /* a plain cudaMalloc'd buffer of the probes, freed on every return path */
 template <typename T>
 struct Dev

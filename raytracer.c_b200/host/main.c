@@ -15,8 +15,10 @@
  *   -m <sx,sy,sz,ry,tx,ty,tz> with obj:FILE -- place the mesh like the reference's driver would: scale, rotation about
  *                            y (degrees), translation, composed into a mat4 and applied with apply_matrix (main.c:140-147)
  *   -a <prefix>              also write the first-hit feature buffers of the frame (render_ex_aov): <prefix>_albedo.pfm,
- *                            <prefix>_normal.pfm (RGB) and <prefix>_depth.pfm (grey), what oidnDenoise --alb --nrm reads;
- *                            single GPU only
+ *                            <prefix>_normal.pfm (RGB) and <prefix>_depth.pfm (grey), the guides of the built-in
+ *                            denoiser (-n) and what an external one such as oidnDenoise --alb --nrm reads; single GPU only
+ *   -n <passes>              write the DENOISED frame to the PNG (render_ex_denoised: the built-in a-trous denoiser
+ *                            guided by the feature buffers, <passes> a-trous passes, 0 = the default); single GPU only
  * Deliberately NOT reproduced: the option parser's mis-parse of values whose second
  * character is h/w/s/o (SURVEY.md section 5) and the SIGINT handler's double free.
  */
@@ -35,6 +37,8 @@ typedef struct
   int max_depth, device, integrator, gpus, dielectric;
   uint64_t seed;
   const char *scene, *placement, *aov_prefix;
+  int denoise; /* -n given */
+  DenoiseParams dn;
 } Cli;
 
 static void usage(const char *prog)
@@ -43,6 +47,7 @@ static void usage(const char *prog)
   fprintf(stderr, "       [-d <max depth>] [-S <seed>] [-g <cuda device>] [-c default|spheres:N|mesh:GRID|obj:FILE]\n");
   fprintf(stderr, "       [-i path|whitted] [-G <gpus>] [-D stochastic|split] [-m sx,sy,sz,ry_deg,tx,ty,tz]\n");
   fprintf(stderr, "       [-a <prefix>: also write <prefix>_albedo.pfm, <prefix>_normal.pfm, <prefix>_depth.pfm]\n");
+  fprintf(stderr, "       [-n <passes>: denoise the frame with the built-in a-trous filter, 0 = default passes]\n");
 }
 
 static bool parse_cli(int argc, char **argv, Cli *cli)
@@ -76,6 +81,12 @@ static bool parse_cli(int argc, char **argv, Cli *cli)
     case 'D': cli->dielectric = (strcmp(val, "split") == 0) ? RT_DIELECTRIC_SPLIT : RT_DIELECTRIC_STOCHASTIC; break;
     case 'm': cli->placement = val; break;
     case 'a': cli->aov_prefix = val; break;
+    case 'n':
+      cli->denoise = 1;
+      denoise_params_default(&cli->dn);
+      if (atoi(val) != 0)
+        cli->dn.iterations = atoi(val);
+      break;
     default:
       fprintf(stderr, "unknown option '%s'\n", a);
       return false;
@@ -84,6 +95,11 @@ static bool parse_cli(int argc, char **argv, Cli *cli)
   if (cli->aov_prefix && cli->gpus > 1)
   {
     fprintf(stderr, "-a (feature buffers) renders on one GPU: it cannot be combined with -G %d\n", cli->gpus);
+    return false;
+  }
+  if (cli->denoise && cli->gpus > 1)
+  {
+    fprintf(stderr, "-n (denoiser) renders on one GPU: it cannot be combined with -G %d\n", cli->gpus);
     return false;
   }
   return cli->options.width >= 2 && cli->options.height >= 2 && cli->options.samples >= 1;
@@ -162,6 +178,7 @@ int main(int argc, char **argv)
     aov = &aov_bufs;
   }
 
+  const DenoiseParams *dn = cli.denoise ? &cli.dn : NULL;
   struct timespec t0, t1;
   clock_gettime(CLOCK_MONOTONIC, &t0);
   /* the CUDA context comes up on a second thread while the scene is generated or read from disk */
@@ -172,18 +189,21 @@ int main(int argc, char **argv)
 #define CLI_MARK(what) do { if (timing) { struct timespec now_; clock_gettime(CLOCK_MONOTONIC, &now_); \
     fprintf(stderr, "main: %s %.1f ms\n", what, 1e3 * (double)(now_.tv_sec - tm.tv_sec) + 1e-6 * (double)(now_.tv_nsec - tm.tv_nsec)); tm = now_; } } while (0)
 
+/* with -n the denoised frame, else exactly the frame of render_ex_aov / render_scene_aov */
+#define RENDER_EX(...) (dn ? render_ex_denoised(__VA_ARGS__, dn) : render_ex_aov(__VA_ARGS__))
+#define RENDER_SCENE(...) (dn ? render_scene_denoised(__VA_ARGS__, dn) : render_scene_aov(__VA_ARGS__))
   if (strcmp(cli.scene, "default") == 0)
   {
     Object scene[SCENE_DEFAULT_COUNT];
     size_t n = scene_default(scene, opt->width, opt->height);
-    render_ex_aov(framebuffer, scene, n, &camera, opt, &rp, aov);
+    RENDER_EX(framebuffer, scene, n, &camera, opt, &rp, aov);
   }
   else if (strncmp(cli.scene, "spheres:", 8) == 0)
   {
     Object *scene = NULL;
     SceneMix mix = { 0.5, 0.2, 0.2 }; /* main.c:104-119 */
     size_t n = scene_sphere_field(&scene, (size_t)atol(cli.scene + 8), opt->width, opt->height, mix, cli.seed);
-    render_ex_aov(framebuffer, scene, n, &camera, opt, &rp, aov);
+    RENDER_EX(framebuffer, scene, n, &camera, opt, &rp, aov);
     free(scene);
   }
   else if (strncmp(cli.scene, "mesh:", 5) == 0 || strncmp(cli.scene, "obj:", 4) == 0)
@@ -213,7 +233,7 @@ int main(int argc, char **argv)
     SceneObject *scene = NULL;
     Sphere *spheres = NULL;
     size_t n = scene_mesh_room(&scene, &spheres, &mesh, opt->width, opt->height);
-    render_scene_aov(framebuffer, scene, n, &camera, opt, &rp, aov);
+    RENDER_SCENE(framebuffer, scene, n, &camera, opt, &rp, aov);
     CLI_MARK("render_scene (first call: CUDA context + upload + BVH + render + read-back)");
     free(scene);
     free(spheres);

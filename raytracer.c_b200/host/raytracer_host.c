@@ -256,41 +256,57 @@ static rtb_comm *local_comm(int num_gpus)
   return g_comm;
 }
 
-/* the feature buffers of the frame just rendered, on the same scene: device sums -> means, in float */
-static void render_aov_means(rtb_scene *scene, const double *cam, const rtb_render_desc *desc, const RenderAov *aov)
+/* the frame on one scene (denoised when `dn` is given) and, with `aov`, the means of its feature buffers in float.
+ * The denoiser runs the feature pass itself and hands its sums back, so that pass runs once either way. */
+static int render_on_scene(rtb_scene *scene, const double *cam, const rtb_render_desc *desc, int divisor,
+                           const DenoiseParams *dn, const RenderAov *aov, uint8_t *framebuffer, float *accum_out,
+                           rtb_counters *counters)
 {
   const size_t n_px = (size_t)desc->width * desc->height;
   const int spp = desc->sample_end - desc->sample_begin;
-  uint32_t *hits = aov->depth ? (uint32_t *)malloc(sizeof(uint32_t) * n_px) : NULL;
-  if (aov->depth && !hits)
+  uint32_t *hits = aov && aov->depth ? (uint32_t *)malloc(sizeof(uint32_t) * n_px) : NULL;
+  if (aov && aov->depth && !hits)
   {
-    rtb_scene_destroy(scene);
     fprintf(stderr, "render: out of host memory for the hit counts\n");
-    exit(EXIT_FAILURE);
+    return RTB_ENOMEM;
   }
-  if (rtb_render_aov_host(scene, cam, desc, aov->albedo, aov->normal, aov->depth, hits, aov->object, NULL) != RTB_OK)
+  int rc;
+  if (dn)
   {
-    free(hits);
-    rtb_scene_destroy(scene);
-    die("render: feature buffers");
+    const rtb_denoise_desc d = { dn->iterations, dn->sigma_luminance, dn->sigma_normal, dn->sigma_depth,
+                                 dn->albedo_epsilon };
+    rc = rtb_render_denoised_aov(scene, cam, desc, divisor, &d, framebuffer, NULL, accum_out,
+                                 aov ? aov->albedo : NULL, aov ? aov->normal : NULL, aov ? aov->depth : NULL, hits,
+                                 aov ? aov->object : NULL, counters);
   }
-  const float n_samples = spp > 0 ? (float)spp : 1.0f; /* spp == 0: the sums are 0 */
-  for (size_t i = 0; i < 3 * n_px; i++)
+  else
   {
-    if (aov->albedo)
-      aov->albedo[i] = aov->albedo[i] / n_samples;
-    if (aov->normal)
-      aov->normal[i] = aov->normal[i] / n_samples;
+    rc = rtb_render_mean(scene, cam, desc, divisor, framebuffer, accum_out, counters);
+    if (rc == RTB_OK && aov)
+      rc = rtb_render_aov_host(scene, cam, desc, aov->albedo, aov->normal, aov->depth, hits, aov->object, NULL);
   }
-  if (aov->depth)
-    for (size_t i = 0; i < n_px; i++)
-      aov->depth[i] = hits[i] ? aov->depth[i] / (float)hits[i] : 0.0f;
+  if (rc == RTB_OK && aov)
+  {
+    const float n_samples = spp > 0 ? (float)spp : 1.0f; /* spp == 0: the sums are 0 */
+    for (size_t i = 0; i < 3 * n_px; i++)
+    {
+      if (aov->albedo)
+        aov->albedo[i] = aov->albedo[i] / n_samples;
+      if (aov->normal)
+        aov->normal[i] = aov->normal[i] / n_samples;
+    }
+    if (aov->depth)
+      for (size_t i = 0; i < n_px; i++)
+        aov->depth[i] = hits[i] ? aov->depth[i] / (float)hits[i] : 0.0f;
+  }
   free(hits);
+  return rc;
 }
 
 /* the body of render(): objects are Object (88-byte) or SceneObject (96-byte) records */
 static void render_records(uint8_t *framebuffer, const void *objects, size_t n_objects, int record_bytes,
-                           Camera *camera, Options *options, const RenderParams *params, const RenderAov *aov)
+                           Camera *camera, Options *options, const RenderParams *params, const RenderAov *aov,
+                           const DenoiseParams *dn)
 {
   RenderParams p;
   if (params)
@@ -318,6 +334,11 @@ static void render_records(uint8_t *framebuffer, const void *objects, size_t n_o
       fprintf(stderr, "render: feature buffers (RenderAov) are single-GPU; render them with num_gpus = 1\n");
       exit(EXIT_FAILURE);
     }
+    if (dn)
+    {
+      fprintf(stderr, "render: the denoiser is single-GPU; denoise with num_gpus = 1\n");
+      exit(EXIT_FAILURE);
+    }
     /* all GPUs of the box: spp-sharded, one ncclReduce of the float sums (rtb200.h) */
     if (p.total_samples > 0 && p.total_samples != options->samples)
     {
@@ -339,13 +360,11 @@ static void render_records(uint8_t *framebuffer, const void *objects, size_t n_o
     if (rc != RTB_OK)
       die("render: scene upload");
     clock_gettime(CLOCK_MONOTONIC, &t1);
-    if (rtb_render_mean(scene, cam, &desc, divisor, framebuffer, p.accum_out, &counters) != RTB_OK)
+    if (render_on_scene(scene, cam, &desc, divisor, dn, aov, framebuffer, p.accum_out, &counters) != RTB_OK)
     {
       rtb_scene_destroy(scene);
       die("render");
     }
-    if (aov)
-      render_aov_means(scene, cam, &desc, aov);
     clock_gettime(CLOCK_MONOTONIC, &t2);
     rtb_scene_destroy(scene);
     if (timing)
@@ -361,13 +380,13 @@ static void render_records(uint8_t *framebuffer, const void *objects, size_t n_o
 void render_ex(uint8_t *framebuffer, Object *objects, size_t n_objects, Camera *camera, Options *options,
                const RenderParams *params)
 {
-  render_records(framebuffer, objects, n_objects, 88, camera, options, params, NULL);
+  render_records(framebuffer, objects, n_objects, 88, camera, options, params, NULL, NULL);
 }
 
 void render_ex_aov(uint8_t *framebuffer, Object *objects, size_t n_objects, Camera *camera, Options *options,
                    const RenderParams *params, const RenderAov *aov)
 {
-  render_records(framebuffer, objects, n_objects, 88, camera, options, params, aov);
+  render_records(framebuffer, objects, n_objects, 88, camera, options, params, aov, NULL);
 }
 
 void render(uint8_t *framebuffer, Object *objects, size_t n_objects, Camera *camera, Options *options)
@@ -378,11 +397,38 @@ void render(uint8_t *framebuffer, Object *objects, size_t n_objects, Camera *cam
 void render_scene(uint8_t *framebuffer, SceneObject *objects, size_t n_objects, Camera *camera,
                   Options *options, const RenderParams *params)
 {
-  render_records(framebuffer, objects, n_objects, 96, camera, options, params, NULL);
+  render_records(framebuffer, objects, n_objects, 96, camera, options, params, NULL, NULL);
 }
 
 void render_scene_aov(uint8_t *framebuffer, SceneObject *objects, size_t n_objects, Camera *camera, Options *options,
                       const RenderParams *params, const RenderAov *aov)
 {
-  render_records(framebuffer, objects, n_objects, 96, camera, options, params, aov);
+  render_records(framebuffer, objects, n_objects, 96, camera, options, params, aov, NULL);
+}
+
+void denoise_params_default(DenoiseParams *p)
+{
+  p->iterations = RTB_DENOISE_DEFAULT_ITERATIONS;
+  p->sigma_luminance = RTB_DENOISE_DEFAULT_SIGMA_LUMINANCE;
+  p->sigma_normal = RTB_DENOISE_DEFAULT_SIGMA_NORMAL;
+  p->sigma_depth = RTB_DENOISE_DEFAULT_SIGMA_DEPTH;
+  p->albedo_epsilon = RTB_DENOISE_DEFAULT_ALBEDO_EPSILON;
+}
+
+void render_ex_denoised(uint8_t *framebuffer, Object *objects, size_t n_objects, Camera *camera, Options *options,
+                        const RenderParams *params, const RenderAov *aov, const DenoiseParams *dn)
+{
+  DenoiseParams d;
+  if (!dn)
+    denoise_params_default(&d);
+  render_records(framebuffer, objects, n_objects, 88, camera, options, params, aov, dn ? dn : &d);
+}
+
+void render_scene_denoised(uint8_t *framebuffer, SceneObject *objects, size_t n_objects, Camera *camera,
+                           Options *options, const RenderParams *params, const RenderAov *aov, const DenoiseParams *dn)
+{
+  DenoiseParams d;
+  if (!dn)
+    denoise_params_default(&d);
+  render_records(framebuffer, objects, n_objects, 96, camera, options, params, aov, dn ? dn : &d);
 }
