@@ -154,9 +154,10 @@ def keyed_jitter(seed, pixels, sample):
     return (c0 >> np.uint32(1)).astype(np.float64) / 2147483648.0, (c1 >> np.uint32(1)).astype(np.float64) / 2147483648.0
 
 
-def camera_rays(cam, seed, w, h, sample):
-    """the render's camera rays of one sample for every pixel, [n_px, 6] (oracle_camera_ray, vectorised)"""
-    pix = np.arange(w * h)
+def camera_rays(cam, seed, w, h, sample, pixels=None):
+    """the render's camera rays of one sample for every pixel (or the flat pixel indices `pixels`), [n, 6]
+    (oracle_camera_ray, vectorised)"""
+    pix = np.arange(w * h) if pixels is None else np.asarray(pixels, np.int64)
     j1, j2 = keyed_jitter(seed, pix, sample)
     u = ((pix % w) + j1) / (w - 1.0)
     v = ((pix // w) + j2) / (h - 1.0)

@@ -234,6 +234,34 @@ def path_log(scene, cam, width, height, samples, dielectric="stochastic", max_de
         cap = n
 
 
+def pixel_paths(scene, cam, width, height, pixels, samples, dielectric="stochastic", max_depth=5, seed=abi.SCENE_SEED,
+                sample_offset=0, threads=None):
+    """every vertex of every path of samples [sample_offset, sample_offset + samples) of the flat pixel indices
+    `pixels` only -> VERTEX_DTYPE [n]: the rows path_log gives for those pixels, in another order.  The paths are
+    walked forward one depth at a time with oracle_path_vertex from the keyed camera rays (tp 1, branch 1), so the
+    cost is that of the chosen pixels, not of the frame."""
+    from denoise_ref import camera_rays  # oracle_camera_ray of the keyed jitter, vectorised (pinned to the oracle)
+    pixels = np.asarray(pixels, np.int64).reshape(-1)
+    s = np.arange(sample_offset, sample_offset + samples, dtype=np.uint32)
+    rays = np.concatenate([camera_rays(cam, seed, width, height, int(k), pixels) for k in s]) if len(s) else np.zeros((0, 6))
+    pix = np.tile(pixels, len(s)).astype(np.uint32)
+    smp = np.repeat(s, len(pixels))
+    tp = np.ones((len(rays), 3))
+    branch = np.ones(len(rays), np.uint32)
+    rows = [np.zeros(0, VERTEX_DTYPE)]
+    depth = 0
+    while len(rays):
+        v = path_vertex(scene, rays, depth, branch, pix, smp, tp, dielectric=dielectric, max_depth=max_depth, seed=seed,
+                        threads=threads)
+        rows.append(v)
+        k_par, k_child = np.nonzero((np.arange(2)[None, :] < v["n_children"][:, None]) & (v["cut"] == 0))
+        rays, tp = v["child_ray"][k_par, k_child], v["child_tp"][k_par, k_child]
+        branch = v["child_branch"][k_par, k_child]
+        pix, smp = v["pixel"][k_par], v["sample"][k_par]
+        depth += 1
+    return np.concatenate(rows)
+
+
 def philox(ctr, key):
     ctr = np.ascontiguousarray(ctr, dtype=np.uint32).reshape(-1, 4)
     key = np.ascontiguousarray(key, dtype=np.uint32).reshape(-1, 2)

@@ -151,6 +151,20 @@ def contribution_bound(pid, n_slots, mag, weighted, count):
     return U * (w + np.maximum(n - 1, 0)[:, None] * m) * (1 + 1e-6) + SLACK * m
 
 
+def render_bound(abi, log, flags, emission, slot, n_slots, planes):
+    """|rendered sum - sum of the oracle's contributions| per slot (pixel) and channel of a whole render, from the
+    slot's vertices in the oracle log -> [n_slots, 3]: a term of a vertex at depth d is a float product of a
+    throughput that went through d + 1 vertices of at most 6 roundings each (throughput_units) and a colour (2
+    roundings); the slot's n terms are added in float, first per plane, then the planes in order (n + planes
+    roundings of the magnitude)"""
+    mag, _, count = vertex_terms(abi, log, flags, emission)
+    k_term = 6 * (log["depth"] + 1) + 2
+    weighted = slot_sums(slot, n_slots, mag * k_term[:, None])
+    m = slot_sums(slot, n_slots, mag)
+    n = slot_sums(slot, n_slots, count)[:, None]
+    return U * (weighted + (n + planes) * m) * (1 + 1e-6) + SLACK * m
+
+
 # ---- the walk -------------------------------------------------------------------------------------------------
 
 def _bits(rays):
@@ -405,10 +419,8 @@ def test_probe_walk_lands_on_the_render(gpu_api, abi, ol, name, dielectric, max_
 @pytest.mark.parametrize("name,max_depth", [("c1", 5), ("c4", 8), ("c5", 64)])
 @pytest.mark.parametrize("dielectric", ["stochastic", "split"])
 def test_render_within_the_float_bound_of_the_oracle(gpu_api, abi, ol, name, max_depth, dielectric):
-    """|gpu - oracle| <= K_pixel 2^-24 per pixel and channel, K_pixel from the pixel's vertices in the oracle log:
-    a term of a vertex at depth d is a float product of a throughput that went through d + 1 vertices of at most 6
-    roundings each (throughput_units) and a colour (2 roundings); the pixel's n terms are added in float, first per
-    plane, then the planes in order (n + planes roundings of the magnitude)"""
+    """|gpu - oracle| <= K_pixel 2^-24 per pixel and channel, K_pixel from the pixel's vertices in the oracle log
+    (render_bound)"""
     if dielectric == "split":
         max_depth = min(max_depth, 5)
     W, H, spp, planes = 32, 18, 4, 2
@@ -417,13 +429,7 @@ def test_render_within_the_float_bound_of_the_oracle(gpu_api, abi, ol, name, max
         _, acc, _ = sc.render(wk.cam, wk.desc, want_accum=True)
     log = ol.path_log(wk.src, wk.cam, W, H, spp, dielectric=dielectric, max_depth=max_depth)
     want, _ = ol.render_sum(wk.src, wk.cam, W, H, spp, dielectric=dielectric, max_depth=max_depth)
-    mag, _, count = vertex_terms(abi, log, wk.flags, wk.emission)
-    pix = log["pixel"].astype(np.int64)
-    k_term = 6 * (log["depth"] + 1) + 2
-    weighted = slot_sums(pix, W * H, mag * k_term[:, None]).reshape(H, W, 3)
-    m = slot_sums(pix, W * H, mag).reshape(H, W, 3)
-    n = slot_sums(pix, W * H, count).reshape(H, W, 1)
-    bound = U * (weighted + (n + planes) * m) * (1 + 1e-6) + SLACK * m
+    bound = render_bound(abi, log, wk.flags, wk.emission, log["pixel"].astype(np.int64), W * H, planes).reshape(H, W, 3)
     err = np.abs(acc.astype(np.float64) - want)
     print(f"{name} {dielectric}: largest error / bound = {np.max(err / np.maximum(bound, 1e-300)):.3f}")
     bad = np.argwhere(err > bound)
