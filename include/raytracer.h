@@ -183,8 +183,10 @@ typedef struct
 /* integrator: the reference compiles trace_path in and cast_ray out (raytracer.c:207-211) */
 enum
 {
-  RT_INTEGRATOR_PATH = 0,   /* trace_path, raytracer.c:482-554 */
-  RT_INTEGRATOR_WHITTED = 1 /* cast_ray, raytracer.c:556-641 */
+  RT_INTEGRATOR_PATH = 0,    /* trace_path, raytracer.c:482-554 */
+  RT_INTEGRATOR_WHITTED = 1, /* cast_ray, raytracer.c:556-641 */
+  RT_INTEGRATOR_PATH_NEE = 2 /* trace_path's estimator with next-event estimation (RTB_INTEGRATOR_PATH_NEE of rtb200.h):
+                                the same image in expectation, less noise */
 };
 
 /* dielectric estimator */

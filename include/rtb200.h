@@ -73,6 +73,13 @@ extern "C" {
 
 #define RTB_INTEGRATOR_PATH 0
 #define RTB_INTEGRATOR_WHITTED 1
+/* trace_path's estimator with next-event estimation: at every diffuse vertex one shadow ray towards an emissive
+ * sphere, combined with the hemisphere ray by the balance heuristic (DESIGN.md section 4.7).  Same expectation as
+ * RTB_INTEGRATOR_PATH, less noise.  Wavefront kernel only (kernel 0 or 6), both dielectric estimators.  The path rays
+ * are RTB_INTEGRATOR_PATH's, one for one (rays, rays_intersected and paths are equal); light samples draw from their
+ * own Philox block.  Emissive spheres are sampled; emissive MESHES are not, they keep contributing through the
+ * hemisphere ray at full weight (unbiased, just not variance-reduced). */
+#define RTB_INTEGRATOR_PATH_NEE 2
 
 typedef struct rtb_scene rtb_scene; /* opaque: device-resident SoA geometry, materials, BVH */
 
@@ -92,7 +99,8 @@ typedef struct
                                    floating-point summation order); 0 = auto */
   int reserved2;                /* kernel 6 tuning: ray sorting mode (0 = off) */
   int integrator;               /* RTB_INTEGRATOR_PATH: trace_path (raytracer.c:482-554, the upstream default);
-                                   RTB_INTEGRATOR_WHITTED: cast_ray (raytracer.c:556-641), max_depth <= 15 */
+                                   RTB_INTEGRATOR_WHITTED: cast_ray (raytracer.c:556-641), max_depth <= 15;
+                                   RTB_INTEGRATOR_PATH_NEE: trace_path with next-event estimation (kernel 0 or 6) */
   int profile;                  /* with `counters`: 1 = also count BVH node visits and time the wavefront kernels
                                    with CUDA events (trace_ms, shade_ms); 0 = rays, primitive tests and paths only */
 } rtb_render_desc;
@@ -110,6 +118,8 @@ typedef struct
   float trace_ms;                     /* wavefront kernels: CUDA-event time summed over the k_wf_trace launches */
   float shade_ms;                     /* wavefront kernels: same for k_wf_generate + k_wf_shade */
   unsigned long long trace_launches;  /* number of k_wf_trace launches */
+  unsigned long long shadow_rays;     /* RTB_INTEGRATOR_PATH_NEE: shadow rays traced (never counted in `rays`); else 0 */
+  unsigned long long shadow_hits;     /* of those, the ones whose nearest hit was their light */
 } rtb_counters;
 
 typedef struct

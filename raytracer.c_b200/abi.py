@@ -114,7 +114,8 @@ class RtbCounters(C.Structure):
                 ("prim_tests", C.c_ulonglong), ("node_visits", C.c_ulonglong),
                 ("paths", C.c_ulonglong), ("launches", C.c_ulonglong),
                 ("gpu_ms", C.c_float), ("build_ms", C.c_float),
-                ("trace_ms", C.c_float), ("shade_ms", C.c_float), ("trace_launches", C.c_ulonglong)]
+                ("trace_ms", C.c_float), ("shade_ms", C.c_float), ("trace_launches", C.c_ulonglong),
+                ("shadow_rays", C.c_ulonglong), ("shadow_hits", C.c_ulonglong)]
 
 
 class RtbSceneInfo(C.Structure):

@@ -353,6 +353,12 @@ def render(objects, camera, width, height, samples):
 
 # ---- the C ABI ----------------------------------------------------------------------------
 
+# rtb_render_desc.integrator (rtb200.h)
+INTEGRATOR_PATH = 0      # trace_path, the reference's estimator
+INTEGRATOR_WHITTED = 1   # cast_ray
+INTEGRATOR_PATH_NEE = 2  # trace_path with next-event estimation: same image in expectation, less noise (kernel 0 or 6)
+
+
 def make_desc(width, height, sample_begin, sample_end, max_depth=5, seed=abi.SCENE_SEED, kernel=0, tune=0, planes=0, tune2=0, integrator=0, profile=1,
               dielectric=0):
     d = abi.RtbRenderDesc()

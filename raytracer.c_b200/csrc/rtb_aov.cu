@@ -133,6 +133,12 @@ extern "C" int rtb_render_aov(rtb_scene *scene, const double *camera12, const rt
   int rc = rtb_check_desc(desc);
   if (rc != RTB_OK)
     return rc;
+  if (desc->integrator == RTB_INTEGRATOR_PATH_NEE)
+  {
+    /* integrator only selects the checker's M here; an NEE render's features are RTB_INTEGRATOR_PATH's */
+    rtb_set_error("rtb_render_aov: integrator RTB_INTEGRATOR_PATH or RTB_INTEGRATOR_WHITTED");
+    return RTB_EINVAL;
+  }
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
   RTB_CUDA(cudaSetDevice(scene->device));
 

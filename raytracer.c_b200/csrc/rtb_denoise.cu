@@ -301,8 +301,12 @@ extern "C" int rtb_render_denoised_aov(rtb_scene *scene, const double *camera12,
   RTB_CUDA(pool.alloc(reinterpret_cast<void **>(&d_out), sizeof(float) * 3 * n_px));
   RTB_CUDA(pool.alloc(reinterpret_cast<void **>(&d_fb), 3 * n_px));
   rc = rtb_render_accum(scene, camera12, desc, d_accum, nullptr, counters);
+  /* the features of a next-event-estimation render are the first hits of trace_path's own camera samples */
+  rtb_render_desc feat = *desc;
+  if (feat.integrator == RTB_INTEGRATOR_PATH_NEE)
+    feat.integrator = RTB_INTEGRATOR_PATH;
   if (rc == RTB_OK)
-    rc = rtb_render_aov(scene, camera12, desc, d_albedo, d_normal, d_depth, d_hits, d_object, nullptr, nullptr);
+    rc = rtb_render_aov(scene, camera12, &feat, d_albedo, d_normal, d_depth, d_hits, d_object, nullptr, nullptr);
   if (rc == RTB_OK)
     rc = rtb_denoise(&d, desc->width, desc->height, total_samples, d_accum, d_albedo, d_normal, d_depth, d_hits,
                      d_object, d_out, scene->device, nullptr);

@@ -121,6 +121,11 @@ struct rtb_scene
   cudaEvent_t wf_fork = nullptr, wf_joins[RTB_WF_MAX_GROUPS] = {};
   size_t wf_bytes = 0;
   unsigned long long *d_counters = nullptr;
+  /* RTB_INTEGRATOR_PATH_NEE: the light list (NeeLight[max(nee_lights, 1)], then int light_of[n_objects]), built on the
+   * scene's first NEE render (rtb_wavefront.cu) */
+  void *d_nee = nullptr;
+  int nee_lights = 0;
+  bool nee_built = false;
   rtb_scene_info info{};
   rtb_scene_tree_info tree{}; /* what rtb_scene_tree reports besides the arrays */
   std::vector<std::pair<void *, size_t>> owned; /* every device buffer of the scene arrays, with its size */

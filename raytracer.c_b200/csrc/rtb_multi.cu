@@ -128,7 +128,7 @@ struct RankCtx
   ncclComm_t nccl = nullptr;
   float *d_accum = nullptr;          /* [H*W*3] this rank's sum */
   uint8_t *d_fb = nullptr;           /* [H*W*3] rank 0 only */
-  unsigned long long *d_ctr = nullptr; /* 8 counters for the whole-job reduction */
+  unsigned long long *d_ctr = nullptr; /* 8 counters and 4 times (10 words) for the whole-job reduction */
   size_t accum_elems = 0;
 };
 
@@ -293,7 +293,7 @@ static int ensure_buffers(RankCtx &R, size_t elems)
     R.accum_elems = elems;
   }
   if (!R.d_ctr)
-    RTB_CUDA(cudaMalloc(reinterpret_cast<void **>(&R.d_ctr), sizeof(unsigned long long) * 8));
+    RTB_CUDA(cudaMalloc(reinterpret_cast<void **>(&R.d_ctr), sizeof(unsigned long long) * 10));
   return RTB_OK;
 }
 
@@ -338,18 +338,18 @@ static int rank_render_reduce(RankCtx &R, int n_ranks, rtb_scene *scene, const d
   {
     /* whole-job counters: sums over ranks (times: the slowest rank) */
     unsigned long long h[8] = { mine.rays, mine.rays_intersected, mine.prim_tests, mine.node_visits, mine.paths,
-                                mine.launches + (R.rank == 0 ? 1ull : 0ull), 0ull, 0ull };
+                                mine.launches + (R.rank == 0 ? 1ull : 0ull), mine.shadow_rays, mine.shadow_hits };
     float t[4] = { mine.gpu_ms, mine.trace_ms, mine.shade_ms, mine.build_ms };
     if (n_ranks > 1)
     {
-      float *d_t = reinterpret_cast<float *>(R.d_ctr + 6);
-      RTB_CUDA(cudaMemcpyAsync(R.d_ctr, h, sizeof(unsigned long long) * 6, cudaMemcpyHostToDevice, 0));
+      float *d_t = reinterpret_cast<float *>(R.d_ctr + 8);
+      RTB_CUDA(cudaMemcpyAsync(R.d_ctr, h, sizeof(unsigned long long) * 8, cudaMemcpyHostToDevice, 0));
       RTB_CUDA(cudaMemcpyAsync(d_t, t, sizeof(t), cudaMemcpyHostToDevice, 0));
       RTB_NCCL(nccl_api().GroupStart());
-      RTB_NCCL(nccl_api().AllReduce(R.d_ctr, R.d_ctr, 6, ncclUint64, ncclSum, R.nccl, 0));
+      RTB_NCCL(nccl_api().AllReduce(R.d_ctr, R.d_ctr, 8, ncclUint64, ncclSum, R.nccl, 0));
       RTB_NCCL(nccl_api().AllReduce(d_t, d_t, 4, ncclFloat32, ncclMax, R.nccl, 0));
       RTB_NCCL(nccl_api().GroupEnd());
-      RTB_CUDA(cudaMemcpyAsync(h, R.d_ctr, sizeof(unsigned long long) * 6, cudaMemcpyDeviceToHost, 0));
+      RTB_CUDA(cudaMemcpyAsync(h, R.d_ctr, sizeof(unsigned long long) * 8, cudaMemcpyDeviceToHost, 0));
       RTB_CUDA(cudaMemcpyAsync(t, d_t, sizeof(t), cudaMemcpyDeviceToHost, 0));
       RTB_CUDA(cudaStreamSynchronize(0));
     }
@@ -365,6 +365,8 @@ static int rank_render_reduce(RankCtx &R, int n_ranks, rtb_scene *scene, const d
     counters->shade_ms = t[2];
     counters->build_ms = t[3];
     counters->trace_launches = mine.trace_launches;
+    counters->shadow_rays = h[6];
+    counters->shadow_hits = h[7];
   }
   return RTB_OK;
 }

@@ -598,9 +598,15 @@ int rtb_check_desc(const rtb_render_desc *d)
     rtb_set_error("rtb_render_desc.kernel: 0 auto, 1..5 megakernel variants, 6 wavefront");
     return RTB_EINVAL;
   }
-  if (d->integrator != RTB_INTEGRATOR_PATH && d->integrator != RTB_INTEGRATOR_WHITTED)
+  if (d->integrator != RTB_INTEGRATOR_PATH && d->integrator != RTB_INTEGRATOR_WHITTED &&
+      d->integrator != RTB_INTEGRATOR_PATH_NEE)
   {
-    rtb_set_error("rtb_render_desc.integrator: RTB_INTEGRATOR_PATH or RTB_INTEGRATOR_WHITTED");
+    rtb_set_error("rtb_render_desc.integrator: RTB_INTEGRATOR_PATH, RTB_INTEGRATOR_WHITTED or RTB_INTEGRATOR_PATH_NEE");
+    return RTB_EINVAL;
+  }
+  if (d->integrator == RTB_INTEGRATOR_PATH_NEE && d->kernel != 0 && d->kernel != 6)
+  {
+    rtb_set_error("RTB_INTEGRATOR_PATH_NEE: wavefront path tracer only (kernel 0 or 6)");
     return RTB_EINVAL;
   }
   if (d->dielectric_mode != RTB_DIELECTRIC_STOCHASTIC && d->dielectric_mode != RTB_DIELECTRIC_SPLIT)
@@ -609,7 +615,7 @@ int rtb_check_desc(const rtb_render_desc *d)
     return RTB_EINVAL;
   }
   if (d->dielectric_mode == RTB_DIELECTRIC_SPLIT &&
-      (d->max_depth > 16 || (d->kernel != 0 && d->kernel != 6) || d->integrator != RTB_INTEGRATOR_PATH))
+      (d->max_depth > 16 || (d->kernel != 0 && d->kernel != 6) || d->integrator == RTB_INTEGRATOR_WHITTED))
   {
     /* 2^(depth+1) rays per path: the reference's estimator is tractable for shallow paths only (its MAX_DEPTH is 5) */
     rtb_set_error("RTB_DIELECTRIC_SPLIT: wavefront path tracer only (kernel 0 or 6), max_depth <= 16");
@@ -725,6 +731,8 @@ extern "C" int rtb_render_accum(rtb_scene *scene, const double *camera12, const 
       want_threads = std::min<long long>(wave_paths, path_cap[dev].load());
     if (desc->dielectric_mode == RTB_DIELECTRIC_SPLIT) /* the queues hold up to 64 entries per path slot */
       want_threads >>= std::min(desc->max_depth + 1, 6);
+    if (desc->integrator == RTB_INTEGRATOR_PATH_NEE) /* the shadow queue: 84 more bytes per queue entry (wf_render) */
+      want_threads = want_threads * 192 / (192 + 84);
     want_threads = std::max<long long>(want_threads, (long long)n_px);
   }
   int chunk = 0;
@@ -852,6 +860,8 @@ extern "C" int rtb_render_accum(rtb_scene *scene, const double *camera12, const 
     counters->trace_ms = phase_ms[0];
     counters->shade_ms = phase_ms[1];
     counters->trace_launches = (unsigned long long)phase_ms[2];
+    counters->shadow_rays = h[5];
+    counters->shadow_hits = h[6];
   }
   return RTB_OK;
 }

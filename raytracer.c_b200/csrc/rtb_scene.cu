@@ -1854,6 +1854,7 @@ extern "C" void rtb_scene_destroy(rtb_scene *scene)
     if (scene->wf_joins[g]) cudaEventDestroy(scene->wf_joins[g]);
   }
   if (scene->wf_fork) cudaEventDestroy(scene->wf_fork);
+  if (scene->d_nee) cudaFree(scene->d_nee);
   if (scene->d_scratch)
     rtb_cache_park(scene->device, scene->d_scratch, scene->scratch_bytes);
   delete scene;

@@ -826,6 +826,159 @@ __global__ void __launch_bounds__(128, WF_SHADE_BLOCKS) k_wf_shade(const __grid_
   wf_add_counters(A.counters, lane, pc.rays, pc.rays_hit, exact, 0ull, 0ull);
 }
 
+/* the shadow rays of the NEE shade kernel: a queue (light index in `branch`) and its length */
+struct WfShadowOut
+{
+  WfQueue q;
+  unsigned *count;
+  NeeView nv;
+};
+
+/* RTB_INTEGRATOR_PATH_NEE: k_wf_shade with next-event estimation (kept apart so that k_wf_shade itself is unchanged):
+ * the emission reached from a diffuse vertex gets its MIS weight, and the shadow ray of every diffuse vertex that is
+ * not depth-cut goes to so.q with the oversized-list part of its nearest hit seeded */
+template <bool SPLIT>
+__global__ void __launch_bounds__(128, WF_SHADE_BLOCKS) k_wf_shade_nee(const __grid_constant__ RenderArgs A, int wave, int depth,
+                                                      WfQueue qin, const unsigned *__restrict__ n_in, WfQueue qout,
+                                                      unsigned *n_out, float4 *__restrict__ planes, unsigned *keys_out,
+                                                      int sort_mode, unsigned *overflow, const __grid_constant__ WfShadowOut so)
+{
+  const int lane = threadIdx.x & 31;
+  const unsigned n = min(*n_in, qin.cap);
+  const unsigned gwarp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+  const unsigned n_warps = (gridDim.x * blockDim.x) >> 5;
+  const unsigned n_px = (unsigned)(A.width * A.height);
+  PathCounters pc = { 0u, 0u };
+  unsigned exact = 0, shadow_rays = 0;
+
+  for (unsigned base = gwarp * 32u; base < n; base += n_warps * 32u)
+  {
+    const unsigned i = base + (unsigned)lane;
+    PathState st;
+    st.o = d3_make(0, 0, 0);
+    st.d = d3_make(0, 0, 1);
+    st.tr = st.tg = st.tb = 0.0f;
+    st.depth = depth;
+    st.alive = false;
+    st.branch = 1u;
+    PathState second;
+    second.alive = false;
+    unsigned pid = 0;
+    HitRec seed, seed2, seed_s;
+    seed.t = DBL_MAX; seed.gid = 0x7FFFFFFF; seed.slot = 0;
+    seed2 = seed;
+    seed_s = seed;
+    NeeIO io;
+    io.from_diffuse = false;
+    io.diffuse_out = false;
+    io.shadow = false;
+    if (i < n)
+    {
+      const uint4 p = __ldcs(qin.path + i);
+      const double2 a = __ldcs(qin.o_xy + i), b = __ldcs(qin.oz_dx + i), c = __ldcs(qin.d_yz + i);
+      const HitRec best = unpack_hit(__ldcs(qin.hit + i));
+      /* bit 31 of the path slot id: the ray left a diffuse vertex (slot ids stay below 2^31) */
+      io.from_diffuse = (p.x >> 31) != 0u;
+      pid = p.x & 0x7FFFFFFFu;
+      st.o = d3_make(a.x, a.y, b.x);
+      st.d = d3_make(b.y, c.x, c.y);
+      st.tr = __uint_as_float(p.y); st.tg = __uint_as_float(p.z); st.tb = __uint_as_float(p.w);
+      st.alive = true;
+      const unsigned plane = pid / n_px;
+      const unsigned pixel = pid - plane * n_px;
+      const unsigned sample = (unsigned)(A.s_begin + (int)plane * A.chunk + wave);
+      pc.rays++;
+      pc.rays_hit++;
+      if (SPLIT)
+      {
+        st.branch = __ldcs(qin.branch + i);
+        float r = 0.0f, g = 0.0f, b2 = 0.0f;
+        path_shade<true, true>(A, st, best, pixel, sample, r, g, b2, pc, nullptr, &second, &so.nv, &io);
+        float *acc = reinterpret_cast<float *>(planes + pid);
+        if (r != 0.0f) atomicAdd(acc + 0, r);
+        if (g != 0.0f) atomicAdd(acc + 1, g);
+        if (b2 != 0.0f) atomicAdd(acc + 2, b2);
+        if (second.alive)
+          ray_seed_hit(A.sv, second.o, second.d, seed2, exact);
+      }
+      else
+      {
+        float4 acc = __ldcs(planes + pid);
+        const float4 before = acc;
+        path_shade<false, true>(A, st, best, pixel, sample, acc.x, acc.y, acc.z, pc, nullptr, nullptr, &so.nv, &io);
+        if (__float_as_uint(acc.x) != __float_as_uint(before.x) || __float_as_uint(acc.y) != __float_as_uint(before.y) ||
+            __float_as_uint(acc.z) != __float_as_uint(before.z))
+          __stcs(planes + pid, acc);
+      }
+      if (st.alive)
+        ray_seed_hit(A.sv, st.o, st.d, seed, exact);
+      if (io.shadow)
+      {
+        /* the shadow ray starts where the continuation starts: the vertex */
+        ray_seed_hit(A.sv, st.o, io.sd, seed_s, exact);
+        shadow_rays++;
+      }
+    }
+    const unsigned pid_out = io.diffuse_out ? (pid | 0x80000000u) : pid;
+    wf_enqueue(qout, n_out, st.alive, lane, st.o, st.d, pid_out, st.tr, st.tg, st.tb, seed, keys_out,
+               (keys_out && st.alive) ? ray_sort_key(A.sv, st.o, st.d, sort_mode) : 0u, st.branch, SPLIT ? overflow : nullptr);
+    if (SPLIT)
+      wf_enqueue(qout, n_out, second.alive, lane, second.o, second.d, pid, second.tr, second.tg, second.tb, seed2, nullptr, 0u,
+                 second.branch, overflow);
+    wf_enqueue(so.q, so.count, io.shadow, lane, st.o, io.sd, pid, io.pr, io.pg, io.pb, seed_s, nullptr, 0u,
+               (unsigned)io.light, nullptr);
+  }
+  wf_add_counters(A.counters, lane, pc.rays, pc.rays_hit, exact, 0ull, 0ull);
+  for (int off = 16; off > 0; off >>= 1)
+    shadow_rays += __shfl_xor_sync(WF_FULL, shadow_rays, off);
+  if (lane == 0 && shadow_rays)
+    atomicAdd(&A.counters[5], (unsigned long long)shadow_rays);
+}
+
+/* RTB_INTEGRATOR_PATH_NEE: a traced shadow ray contributes its payload times the light's emission when its nearest hit
+ * is its light.  Stochastic estimator: a path slot has at most one shadow ray per bounce, so its accumulator is still
+ * read-modify-written by one thread at a time, in vertex order (bit-reproducible sums); SPLIT: atomics. */
+template <bool SPLIT>
+__global__ void __launch_bounds__(128) k_wf_shadow_resolve(const __grid_constant__ SceneView sv, NeeView nv, WfQueue q,
+                                                           const unsigned *__restrict__ n_ptr, float4 *__restrict__ planes,
+                                                           unsigned long long *counters)
+{
+  const int lane = threadIdx.x & 31;
+  const unsigned n = min(*n_ptr, q.cap);
+  unsigned hits = 0;
+  for (unsigned i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x)
+  {
+    const HitRec best = unpack_hit(__ldcs(q.hit + i));
+    if (best.t >= 1e300)
+      continue;
+    const float4 *rec = best.slot >= 0 ? sv.prims + 3 * best.slot : sv.big + 3 * (~best.slot);
+    const int obj = (int)(__float_as_uint(__ldg(rec + 2).z) & 0x7FFFFFFFu);
+    const NeeLight &L = nv.lights[__ldcs(q.branch + i)];
+    if (obj != L.obj)
+      continue;
+    hits++;
+    const uint4 p = __ldcs(q.path + i);
+    const float cr = __uint_as_float(p.y) * L.er, cg = __uint_as_float(p.z) * L.eg, cb = __uint_as_float(p.w) * L.eb;
+    if (SPLIT)
+    {
+      float *acc = reinterpret_cast<float *>(planes + p.x);
+      if (cr != 0.0f) atomicAdd(acc + 0, cr);
+      if (cg != 0.0f) atomicAdd(acc + 1, cg);
+      if (cb != 0.0f) atomicAdd(acc + 2, cb);
+    }
+    else
+    {
+      float4 acc = planes[p.x];
+      acc.x += cr; acc.y += cg; acc.z += cb;
+      planes[p.x] = acc;
+    }
+  }
+  for (int off = 16; off > 0; off >>= 1)
+    hits += __shfl_xor_sync(WF_FULL, hits, off);
+  if (lane == 0 && hits)
+    atomicAdd(&counters[6], (unsigned long long)hits);
+}
+
 /* out[pixel][c] = sum over planes, in plane order (deterministic; same order as k_sum_planes) */
 __global__ void k_wf_sum_planes(const float4 *__restrict__ planes, int n_planes, unsigned n_px, float *__restrict__ out)
 {
@@ -966,11 +1119,13 @@ struct WfGroup
   unsigned *counts, *fetch;
   int planes, gen_blocks;
   bool has_last;
+  WfQueue sq;                /* RTB_INTEGRATOR_PATH_NEE: the group's slice of the shadow queue */
+  unsigned *scounts, *sfetch; /* its lengths and trace fetch cursors, per bounce */
 };
 
 /* the groups of wf_render: queues q[] hold `cap` entries; group g's counters start at ctr_base + g * ctr_one */
 static void wf_groups(const RenderArgs &A, int n_groups, const WfQueue q[2], size_t cap, char *ctr_base, size_t ctr_one,
-                      int n_bounces, WfGroup *G)
+                      int n_bounces, WfGroup *G, const WfQueue *shadow = nullptr)
 {
   const size_t n_px = (size_t)A.width * A.height;
   for (int g = 0; g < n_groups; g++)
@@ -992,6 +1147,18 @@ static void wf_groups(const RenderArgs &A, int n_groups, const WfQueue q[2], siz
     }
     R.counts = reinterpret_cast<unsigned *>(ctr_base + (size_t)g * ctr_one);
     R.fetch = R.counts + (n_bounces + 2);
+    R.sq = WfQueue{};
+    R.scounts = R.sfetch = nullptr;
+    if (shadow)
+    {
+      /* after the counts, the fetch cursors and the overflow flag */
+      R.sq = *shadow;
+      R.sq.o_xy += first_slot; R.sq.oz_dx += first_slot; R.sq.d_yz += first_slot;
+      R.sq.path += first_slot; R.sq.hit += first_slot; R.sq.branch += first_slot;
+      R.sq.cap = R.q[0].cap;
+      R.scounts = R.counts + 2 * (n_bounces + 2) + 1;
+      R.sfetch = R.scounts + (n_bounces + 2);
+    }
     R.gen_blocks = (int)(((long long)A.n_tiles * R.planes * 32 + 255) / 256);
   }
 }
@@ -1001,6 +1168,108 @@ static int wf_valid_planes(const WfGroup &R, const RenderArgs &A, int wave)
 {
   const int last_len = (A.s_end - A.s_begin) - (A.splits - 1) * A.chunk;
   return (R.has_last && wave >= last_len) ? R.planes - 1 : R.planes;
+}
+
+/* ---- light list of RTB_INTEGRATOR_PATH_NEE ------------------------------------------------------------------------ */
+
+struct NeeFound /* an emissive sphere found in the primitive records */
+{
+  double cx, cy, cz, r;
+  int obj, pad;
+};
+
+/* every sphere record (BVH primitives and oversized list) whose object emits -> out[], count in *n */
+__global__ void k_nee_collect(const __grid_constant__ SceneView sv, NeeFound *out, unsigned *n)
+{
+  const unsigned i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= (unsigned)(sv.n_prims + sv.n_big))
+    return;
+  const float4 *rec = i < (unsigned)sv.n_prims ? sv.prims + 3 * (size_t)i : sv.big + 3 * (size_t)(i - sv.n_prims);
+  const unsigned bits = __float_as_uint(rec[2].z);
+  if ((bits & RTB_PRIM_SPHERE_BIT) == 0u)
+    return;
+  const int obj = (int)(bits & 0x7FFFFFFFu);
+  const float4 m1 = sv.mats[2 * obj + 1];
+  if (m1.x == 0.0f && m1.y == 0.0f && m1.z == 0.0f)
+    return;
+  const float4 a = rec[0], b = rec[1];
+  NeeFound f;
+  f.cx = rec_double(a.x, a.y);
+  f.cy = rec_double(a.z, a.w);
+  f.cz = rec_double(b.x, b.y);
+  f.r = rec_double(b.z, b.w);
+  f.obj = obj;
+  f.pad = 0;
+  out[atomicAdd(n, 1u)] = f;
+}
+
+/* the scene's light list, built on its first NEE render and kept with the scene (scene creation and every other render
+ * are untouched by it) */
+static int nee_lights(rtb_scene *scene, cudaStream_t stream, NeeView &nv)
+{
+  if (!scene->nee_built)
+  {
+    const SceneView &sv = scene->view;
+    const size_t n_rec = (size_t)sv.n_prims + (size_t)sv.n_big;
+    std::vector<NeeFound> found;
+    if (n_rec > 0)
+    {
+      Dev<NeeFound> d_found;
+      Dev<unsigned> d_n;
+      RTB_CUDA(cudaMalloc(&d_found.p, sizeof(NeeFound) * std::min<size_t>(n_rec, (size_t)sv.n_objects + 1)));
+      RTB_CUDA(cudaMalloc(&d_n.p, sizeof(unsigned)));
+      RTB_CUDA(cudaMemsetAsync(d_n.p, 0, sizeof(unsigned), stream));
+      k_nee_collect<<<(unsigned)((n_rec + 255) / 256), 256, 0, stream>>>(sv, d_found.p, d_n.p);
+      RTB_CUDA(cudaGetLastError());
+      unsigned n = 0;
+      RTB_CUDA(cudaMemcpyAsync(&n, d_n.p, sizeof(unsigned), cudaMemcpyDeviceToHost, stream));
+      RTB_CUDA(cudaStreamSynchronize(stream));
+      found.resize(n);
+      if (n)
+        RTB_CUDA(cudaMemcpy(found.data(), d_found.p, sizeof(NeeFound) * n, cudaMemcpyDeviceToHost));
+    }
+    /* object order: the order of the selection CDF, which the oracle builds the same way */
+    std::sort(found.begin(), found.end(), [](const NeeFound &x, const NeeFound &y) { return x.obj < y.obj; });
+    std::vector<float4> mats(2 * (size_t)sv.n_objects);
+    if (sv.n_objects > 0)
+      RTB_CUDA(cudaMemcpy(mats.data(), sv.mats, sizeof(float4) * mats.size(), cudaMemcpyDeviceToHost));
+    std::vector<NeeLight> lights(found.size());
+    double total = 0.0;
+    for (size_t k = 0; k < found.size(); k++)
+    {
+      const float4 e = mats[2 * (size_t)found[k].obj + 1];
+      NeeLight &L = lights[k];
+      L.cx = found[k].cx; L.cy = found[k].cy; L.cz = found[k].cz; L.r = found[k].r;
+      L.er = e.x; L.eg = e.y; L.eb = e.z;
+      L.obj = found[k].obj;
+      const double w = ((double)fabsf(e.x) + (double)fabsf(e.y) + (double)fabsf(e.z)) * L.r * L.r;
+      total += w;
+      L.cdf = total; /* running sum; normalised below */
+    }
+    double prev = 0.0;
+    for (size_t k = 0; k < lights.size(); k++)
+    {
+      lights[k].cdf = lights[k].cdf / total;
+      lights[k].P = lights[k].cdf - prev;
+      prev = lights[k].cdf;
+    }
+    std::vector<int> light_of((size_t)std::max(sv.n_objects, 1), -1);
+    for (size_t k = 0; k < lights.size(); k++)
+      light_of[(size_t)lights[k].obj] = (int)k;
+    const size_t bytes = sizeof(NeeLight) * std::max<size_t>(lights.size(), 1) + sizeof(int) * light_of.size();
+    RTB_CUDA(cudaMalloc(&scene->d_nee, bytes));
+    if (!lights.empty())
+      RTB_CUDA(cudaMemcpy(scene->d_nee, lights.data(), sizeof(NeeLight) * lights.size(), cudaMemcpyHostToDevice));
+    RTB_CUDA(cudaMemcpy(static_cast<char *>(scene->d_nee) + sizeof(NeeLight) * std::max<size_t>(lights.size(), 1),
+                        light_of.data(), sizeof(int) * light_of.size(), cudaMemcpyHostToDevice));
+    scene->nee_lights = (int)lights.size();
+    scene->nee_built = true;
+  }
+  nv.lights = static_cast<const NeeLight *>(scene->d_nee);
+  nv.light_of = reinterpret_cast<const int *>(static_cast<const char *>(scene->d_nee) +
+                                              sizeof(NeeLight) * std::max(scene->nee_lights, 1));
+  nv.n_lights = scene->nee_lights;
+  return RTB_OK;
 }
 
 int wf_render(rtb_scene *scene, RenderArgs &A, const rtb_render_desc *desc, float *d_accum, cudaStream_t stream,
@@ -1032,6 +1301,14 @@ int wf_render(rtb_scene *scene, RenderArgs &A, const rtb_render_desc *desc, floa
   if (tune_rc != RTB_OK)
     return tune_rc;
   const int sort_mode = split ? 0 : (desc->reserved2 & 0xFF);
+  const bool nee = desc->integrator == RTB_INTEGRATOR_PATH_NEE;
+  NeeView nv = { nullptr, nullptr, 0 };
+  if (nee)
+  {
+    const int nee_rc = nee_lights(scene, stream, nv);
+    if (nee_rc != RTB_OK)
+      return nee_rc;
+  }
   const int sort_from = 1;                                           /* primary rays are coherent already */
   const int sort_until = (desc->reserved2 >> 8) & 0xFF ? (desc->reserved2 >> 8) & 0xFF : 255;
 
@@ -1039,7 +1316,8 @@ int wf_render(rtb_scene *scene, RenderArgs &A, const rtb_render_desc *desc, floa
   const size_t arr = align_up(cap * 16, 256);
   const size_t arr_planes = align_up(slots * 16, 256);
   const size_t arr4 = align_up(cap * 4, 256);
-  const size_t ctr_one = align_up(sizeof(unsigned) * (2 * (size_t)(n_bounces + 2) + 1), 256);
+  /* per group: queue lengths, fetch cursors, the overflow flag; NEE: the same two arrays for the shadow queue */
+  const size_t ctr_one = align_up(sizeof(unsigned) * ((nee ? 4 : 2) * (size_t)(n_bounces + 2) + 1), 256);
   const size_t ctr_bytes = WF_MAX_GROUPS * ctr_one; /* per plane group (stream) */
   size_t sort_tmp_bytes = 0;
   if (sort_mode)
@@ -1052,7 +1330,8 @@ int wf_render(rtb_scene *scene, RenderArgs &A, const rtb_render_desc *desc, floa
   cudaDeviceGetAttribute(&sm_count, cudaDevAttrMultiProcessorCount, scene->device);
   const bool pool = tune.pool;
   const size_t pool_bytes = wf_pool_stack_bytes(tune, sm_count);
-  const size_t need = arr * 10 + arr_planes + ctr_bytes + (sort_mode ? arr4 * 4 + sort_tmp_bytes : 0) + (split ? arr4 * 2 : 0) + pool_bytes;
+  const size_t need = arr * 10 + arr_planes + ctr_bytes + (sort_mode ? arr4 * 4 + sort_tmp_bytes : 0) + (split ? arr4 * 2 : 0) +
+                      pool_bytes + (nee ? arr * 5 + arr4 : 0);
   if (scene->wf_bytes < need)
   {
     if (scene->d_wf)
@@ -1110,6 +1389,17 @@ int wf_render(rtb_scene *scene, RenderArgs &A, const rtb_render_desc *desc, floa
     pool_stacks = reinterpret_cast<int2 *>(p);
     p += pool_bytes;
   }
+  WfQueue sq{}; /* NEE: shadow rays, the light index in `branch` */
+  if (nee)
+  {
+    sq.o_xy = reinterpret_cast<double2 *>(p); p += arr;
+    sq.oz_dx = reinterpret_cast<double2 *>(p); p += arr;
+    sq.d_yz = reinterpret_cast<double2 *>(p); p += arr;
+    sq.path = reinterpret_cast<uint4 *>(p); p += arr;
+    sq.hit = reinterpret_cast<uint4 *>(p); p += arr;
+    sq.branch = reinterpret_cast<unsigned *>(p); p += arr4;
+    sq.cap = (unsigned)cap;
+  }
   unsigned *keys = nullptr, *keys_sorted = nullptr, *iota = nullptr, *perm = nullptr;
   void *sort_tmp = nullptr;
   if (sort_mode)
@@ -1163,7 +1453,7 @@ int wf_render(rtb_scene *scene, RenderArgs &A, const rtb_render_desc *desc, floa
         RTB_CUDA(cudaEventCreateWithFlags(&scene->wf_fork, cudaEventDisableTiming));
     }
   WfGroup G[WF_MAX_GROUPS];
-  wf_groups(A, n_groups, q, cap, ctr_base, ctr_one, n_bounces, G);
+  wf_groups(A, n_groups, q, cap, ctr_base, ctr_one, n_bounces, G, nee ? &sq : nullptr);
   for (int g = 0; g < n_groups; g++)
     G[g].stream = g == 0 ? stream : scene->wf_streams[g];
   if (n_groups > 1)
@@ -1178,6 +1468,8 @@ int wf_render(rtb_scene *scene, RenderArgs &A, const rtb_render_desc *desc, floa
     {
       WfGroup &R = G[g];
       RTB_CUDA(cudaMemsetAsync(R.counts, 0, sizeof(unsigned) * 2 * (size_t)(n_bounces + 2), R.stream));
+      if (nee)
+        RTB_CUDA(cudaMemsetAsync(R.scounts, 0, sizeof(unsigned) * 2 * (size_t)(n_bounces + 2), R.stream));
       k_wf_generate<<<R.gen_blocks, 256, 0, R.stream>>>(R.A, wave, wf_valid_planes(R, A, wave), R.q[0], &R.counts[0]);
       launches++;
     }
@@ -1196,7 +1488,27 @@ int wf_render(rtb_scene *scene, RenderArgs &A, const rtb_render_desc *desc, floa
         mark();
         if (sort_out) /* slots beyond the queue's end keep the largest key and sort to the back */
           RTB_CUDA(cudaMemsetAsync(keys, 0xFF, slots * 4, st));
-        if (split)
+        if (nee)
+        {
+          /* shade (and emit one shadow ray per diffuse vertex), trace the shadow rays with the same trace kernel,
+           * add the ones that reach their light */
+          const WfShadowOut so = { R.sq, &R.scounts[b], nv };
+          if (split)
+            k_wf_shade_nee<true><<<shade_blocks, 128, 0, st>>>(R.A, wave, b, qi, &cnt[b], qo, &cnt[b + 1], planes, nullptr, 0,
+                                                               overflow, so);
+          else
+            k_wf_shade_nee<false><<<shade_blocks, 128, 0, st>>>(R.A, wave, b, qi, &cnt[b], qo, &cnt[b + 1], planes,
+                                                                sort_out ? keys : nullptr, sort_mode, nullptr, so);
+          mark();
+          wf_launch_trace(tune, stats, sm_count, st, A.sv, R.sq, &R.scounts[b], &R.sfetch[b], A.counters, pool_stacks, nullptr);
+          mark();
+          if (split)
+            k_wf_shadow_resolve<true><<<shade_blocks, 128, 0, st>>>(A.sv, nv, R.sq, &R.scounts[b], planes, A.counters);
+          else
+            k_wf_shadow_resolve<false><<<shade_blocks, 128, 0, st>>>(A.sv, nv, R.sq, &R.scounts[b], planes, A.counters);
+          launches += 2;
+        }
+        else if (split)
           k_wf_shade<true><<<shade_blocks, 128, 0, st>>>(R.A, wave, b, qi, &cnt[b], qo, &cnt[b + 1], planes, nullptr, 0, overflow);
         else
           k_wf_shade<false><<<shade_blocks, 128, 0, st>>>(R.A, wave, b, qi, &cnt[b], qo, &cnt[b + 1], planes,

@@ -9,7 +9,8 @@
  *   -S <seed>                Philox key (default 1666943821, main.c:182)
  *   -g <device>              CUDA device ordinal
  *   -c default|spheres:N|mesh:GRID|obj:FILE
- *   -i path|whitted          integrator: trace_path (upstream default) or cast_ray (raytracer.c:207-211)
+ *   -i path|whitted|nee      integrator: trace_path (upstream default), cast_ray (raytracer.c:207-211), or trace_path
+ *                            with next-event estimation (same image in expectation, less noise)
  *   -G <gpus>                render on GPUs 0..n-1 of the box (samples sharded, one ncclReduce; default $RTB_NUM_GPUS or 1)
  *   -D stochastic|split      dielectric estimator: one child per vertex (default) or the reference's two-way split
  *   -m <sx,sy,sz,ry,tx,ty,tz> with obj:FILE -- place the mesh like the reference's driver would: scale, rotation about
@@ -76,7 +77,11 @@ static bool parse_cli(int argc, char **argv, Cli *cli)
     case 'S': cli->seed = strtoull(val, NULL, 10); break;
     case 'g': cli->device = atoi(val); break;
     case 'c': cli->scene = val; break;
-    case 'i': cli->integrator = (strcmp(val, "whitted") == 0) ? RT_INTEGRATOR_WHITTED : RT_INTEGRATOR_PATH; break;
+    case 'i':
+      cli->integrator = (strcmp(val, "whitted") == 0) ? RT_INTEGRATOR_WHITTED
+                        : (strcmp(val, "nee") == 0)   ? RT_INTEGRATOR_PATH_NEE
+                                                      : RT_INTEGRATOR_PATH;
+      break;
     case 'G': cli->gpus = atoi(val); break;
     case 'D': cli->dielectric = (strcmp(val, "split") == 0) ? RT_DIELECTRIC_SPLIT : RT_DIELECTRIC_STOCHASTIC; break;
     case 'm': cli->placement = val; break;

@@ -224,7 +224,9 @@ static void fill_desc(rtb_render_desc *desc, const Options *options, const Rende
   desc->max_depth = p->max_depth;
   desc->dielectric_mode = p->dielectric_mode == RT_DIELECTRIC_SPLIT ? RTB_DIELECTRIC_SPLIT : RTB_DIELECTRIC_STOCHASTIC;
   desc->seed = p->seed;
-  desc->integrator = p->integrator == RT_INTEGRATOR_WHITTED ? RTB_INTEGRATOR_WHITTED : RTB_INTEGRATOR_PATH;
+  desc->integrator = p->integrator == RT_INTEGRATOR_WHITTED    ? RTB_INTEGRATOR_WHITTED
+                     : p->integrator == RT_INTEGRATOR_PATH_NEE ? RTB_INTEGRATOR_PATH_NEE
+                                                               : RTB_INTEGRATOR_PATH;
 }
 
 /* One comm per process and GPU count, made on first use (NCCL communicator set-up costs ~0.1-1 s) and
@@ -282,8 +284,12 @@ static int render_on_scene(rtb_scene *scene, const double *cam, const rtb_render
   else
   {
     rc = rtb_render_mean(scene, cam, desc, divisor, framebuffer, accum_out, counters);
+    /* the features of a next-event-estimation render are the first hits of trace_path's own camera samples */
+    rtb_render_desc feat = *desc;
+    if (feat.integrator == RTB_INTEGRATOR_PATH_NEE)
+      feat.integrator = RTB_INTEGRATOR_PATH;
     if (rc == RTB_OK && aov)
-      rc = rtb_render_aov_host(scene, cam, desc, aov->albedo, aov->normal, aov->depth, hits, aov->object, NULL);
+      rc = rtb_render_aov_host(scene, cam, &feat, aov->albedo, aov->normal, aov->depth, hits, aov->object, NULL);
   }
   if (rc == RTB_OK && aov)
   {
